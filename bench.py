@@ -44,7 +44,14 @@ def parse():
     ap.add_argument("--no-bam-leg", action="store_true", help="skip the leg that starts from a BAM resident on the device (idl_bam_open + idl_bam_submit; N=1 only: it writes the workload as a BAM first)")
     ap.add_argument("--e2e-batches", type=int, default=2, help="batches per step in the end-to-end leg (measured: 2 -> 41.6 ms per step, 3 -> 42.7, 4 -> 42.7: smaller batches leave the persistent kernels too few tasks per warp)")
     ap.add_argument("--verify", type=int, default=1, help="strong mode: compare the merged VCF with the oracle's once after timing")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after timing, write what the timed path computed in its last step (rank 0) as DIR/<name>.npy, "
+                    "float32/float64, at most 64 MB in all.  Weak mode: the result tables of the end-to-end leg (idl_submit / idl_wait, whose results "
+                    "reach the caller), not of the resident leg behind `value`, which copies back counters only; they are copied after that leg's "
+                    "timed window closes.  Strong mode and --impl reference: the merged VCF text")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 def scaling_mode(args):
@@ -171,6 +178,125 @@ def dedup_text(text):
     return "".join(l + "\n" for l in out)
 
 
+DUMP_BYTES = 64 << 20                           # --dump-outputs writes at most this much
+DUMP_SHARE = (DUMP_BYTES - (1 << 16)) // 6      # per table: six tables and a few small files
+NO_EVENTS = 0xFFFFFFFF                          # IDL_NO_EVENTS
+
+
+def dump_table(out, name, n, width, itemsize, gather, share=None):
+    """out[name] = gather(rows) for all n rows of a table, or for a fixed, seeded sample of them when the table would take more than
+    `share` bytes (DUMP_SHARE by default); the sampled row numbers go to out[name + "_rows"]"""
+    share = DUMP_SHARE if share is None else share
+    rows = np.arange(n)
+    if n * width * itemsize > share:
+        rows = np.unique(np.random.default_rng(0).integers(0, n, share // (width * itemsize + 8)))
+        out[name + "_rows"] = rows.astype(np.float64)
+    out[name] = gather(rows)
+
+
+def dump_text(text):
+    out = {}
+    b = np.frombuffer(text, dtype=np.uint8)
+    dump_table(out, "vcf", len(b), 1, 4, lambda rows: b[rows].astype(np.float32), share=DUMP_BYTES - (1 << 16))   # the only table
+    return out
+
+
+def _ragged(offsets, lengths, pos):
+    """positions `pos` in the concatenation of the blocks [offsets[i], offsets[i] + lengths[i]) -> indices into the array holding the blocks"""
+    ends = np.cumsum(lengths)
+    i = np.searchsorted(ends, pos, side="right")
+    return offsets[i] + pos - (ends[i] - lengths[i])
+
+
+def result_tables(r):
+    """host copies of the tables of one ticket (idl_results), taken before its release"""
+    from indelope_b200 import abi
+
+    def table(ptr, n, t):
+        return np.ctypeslib.as_array(C.cast(ptr, C.POINTER(t)), (n,)).copy() if n else np.zeros(0, np.dtype(t))
+    return {"reg": table(r.region, r.n_regions, abi.RegionResult), "ctg": table(r.contig, r.n_contigs, abi.ContigResult),
+            "aln": table(r.aln, r.n_alns, abi.AlnResult), "ev": table(r.event, r.n_events, abi.EventResult),
+            "cig": table(r.cigar, r.n_cigar_ops, C.c_uint32), "seq": table(r.contig_seq, r.n_contig_bases, C.c_uint8)}
+
+
+# fields that index another table of the same ticket
+LINKS = {("reg", "contig_begin"): "ctg", ("ctg", "seq_off"): "seq", ("ctg", "region"): "reg", ("ctg", "aln"): "aln", ("aln", "region"): "reg",
+         ("aln", "contig"): "ctg", ("aln", "cigar_off"): "cig", ("aln", "event_begin"): "ev", ("ev", "aln"): "aln"}
+
+
+def merge_tables(parts):
+    """the tables of a step's batches, in batch order, as one set of int64 columns: indices are moved past the rows of the batches
+    before (-1 and IDL_NO_EVENTS stay); a uint64 k-mer code keeps its 64 bits"""
+    m, at = {}, dict.fromkeys(("reg", "ctg", "aln", "ev", "cig", "seq"), 0)
+    for p in parts:
+        for t in ("reg", "ctg", "aln", "ev"):
+            for f in p[t].dtype.names:
+                v = p[t][f].astype(np.int64)
+                if (t, f) in LINKS:
+                    v = np.where((v < 0) | (v == NO_EVENTS), v, v + at[LINKS[t, f]])
+                m.setdefault(t, {}).setdefault(f, []).append(v)
+        for t in ("cig", "seq"):
+            m.setdefault(t, []).append(p[t])
+        for t in at:
+            at[t] += len(p[t])
+    return {t: {f: np.concatenate(v) for f, v in c.items()} if isinstance(c, dict) else np.concatenate(c) for t, c in m.items()}
+
+
+def _cols(t, names, rows):
+    return np.stack([t[f][rows] for f in names], axis=1).astype(np.float64).reshape(len(rows), len(names))
+
+
+def dump_results(parts):
+    """the result tables of a step's tickets (result_tables, in batch order) in the order a caller reads them: the regions, the contigs of
+    each region, the alignment of each contig that has one, the CIGAR ops and the event records of each alignment, the bases of each
+    contig.  The device hands out contig, alignment, CIGAR, event and base slots in completion order, so slot offsets are left out and
+    references between tables are indices in that order: two runs, or two builds, compare row for row.  int32/uint32 fields are exact
+    in float64, a uint64 k-mer code is split into two 32-bit halves, bases (ASCII) go to float32."""
+    from indelope_b200 import abi
+    m = merge_tables(parts)
+    reg, ctg, aln, ev, cig, seq = (m[k] for k in ("reg", "ctg", "aln", "ev", "cig", "seq"))
+
+    n_ctg = np.maximum(reg["n_contigs"], 0)
+    order = _ragged(reg["contig_begin"], n_ctg, np.arange(n_ctg.sum()))
+    con = {f: v[order] for f, v in ctg.items()}
+    has = con["aln"] >= 0
+    con["aln_index"] = np.where(has, np.cumsum(has) - 1, -1)
+    al = {f: v[con["aln"][has]] for f, v in aln.items()}
+    canon_ctg = np.full(len(ctg["start"]), -1, dtype=np.int64)
+    canon_ctg[order] = np.arange(len(order))
+    al["contig_index"] = canon_ctg[al["contig"]]
+    canon_aln = np.full(len(aln["region"]), -1, dtype=np.int64)
+    canon_aln[con["aln"][has]] = np.arange(int(has.sum()))
+    n_cig = np.where(al["status"] & abi.RS_CIGAR_OVERFLOW, 0, np.maximum(al["n_cigar"], 0))  # an overflowed CIGAR was not written
+    n_ev = np.where(al["event_begin"] == NO_EVENTS, 0, np.maximum(al["n_events"], 0))
+
+    out = {"counts": np.array([len(reg["status"]), len(ctg["start"]), len(aln["region"]), len(ev["aln"]), len(cig), len(seq)], dtype=np.float64)}
+    f = ["status", "n_contigs_pre", "n_contigs"]
+    dump_table(out, "regions", len(reg["status"]), len(f), 8, lambda rows, f=f: _cols(reg, f, rows))
+    f = ["start", "nreads", "len", "region", "aln_index"]
+    dump_table(out, "contigs", len(order), len(f), 8, lambda rows, f=f: _cols(con, f, rows))
+    f = "region ref_len max zdropped max_q max_t mqe mqe_t mte mte_q score n_cigar n_cigar_trunc n_events status contig_index".split()
+    dump_table(out, "alignments", int(has.sum()), len(f), 8, lambda rows, f=f: _cols(al, f, rows))
+    dump_table(out, "cigar", int(n_cig.sum()), 1, 8, lambda rows: cig[_ragged(al["cigar_off"], n_cig, rows)].astype(np.float64)[:, None])
+    f = [n for n, _ in abi.EventResult._fields_ if n not in ("aln", "ref_code", "alt_code")]
+
+    def events(rows):   # the alignment's index, the fields, the two k-mer codes as (high, low) halves
+        e = {k: v[_ragged(al["event_begin"], n_ev, rows)] for k, v in ev.items()}
+        e["aln_index"] = canon_aln[e["aln"]]
+        for k in ("ref_code", "alt_code"):
+            e[k + "_hi"], e[k + "_lo"] = (e[k] >> 32) & 0xFFFFFFFF, e[k] & 0xFFFFFFFF
+        return _cols(e, ["aln_index"] + f + ["ref_code_hi", "ref_code_lo", "alt_code_hi", "alt_code_lo"], np.arange(len(rows)))
+    dump_table(out, "events", int(n_ev.sum()), len(f) + 5, 8, events)
+    dump_table(out, "contig_bases", int(con["len"].sum()), 1, 4, lambda rows: seq[_ragged(con["seq_off"], con["len"], rows)].astype(np.float32))
+    return out
+
+
+def write_dump(path, out):
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main_reference(args, rank, world):
     if rank != 0:
         return
@@ -182,9 +308,11 @@ def main_reference(args, rank, world):
         run_oracle(rois, min(sample, 2000), cores)
     t0 = time.time(); regions = reads = 0
     for _ in range(args.steps):
-        n, nr, cnt, use_ref, _ = run_oracle(rois, sample, cores)
+        n, nr, cnt, use_ref, vcf = run_oracle(rois, sample, cores)
         regions += n; reads += nr
     dt = time.time() - t0
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, dump_text(vcf.encode()))
     val = regions / dt
     line = {
         "impl": "reference", "metric": "regions_per_s", "value": val, "unit": "regions/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -250,7 +378,7 @@ def main():
                 r.n_events * C.sizeof(abi.EventResult) + r.n_cigar_ops * 4 + r.n_contig_bases)
 
     sampler = ClockSampler(local)
-    extra = {}
+    extra, dumped = {}, {}
     if mode == "weak":
         # ---- pinned batches: one big batch for the device-resident leg, `e2e_batches` slices for the end-to-end legs
         big, big_bytes = alloc_pack(0, n_regions)
@@ -279,32 +407,44 @@ def main():
         # batches as the reference-facing API intends (idl_submit / idl_wait with tickets, `n_streams` batches in flight): the pipeline
         # runs on across step boundaries and is drained once, inside the timed region, before the closing barrier.  repack=True also
         # re-packs every batch from the ASCII reads on the host cores (idlh_pack: quality trim, 2-bit packing, records) each step.
-        def e2e_steps(k, repack):
+        def e2e_steps(k, repack, held=None):
             inflight, d2h, nl, kern = [], 0, 0, 0.0
 
             def retire():
                 nonlocal d2h, nl, kern
-                t = inflight.pop(0); r = ctx.wait(t).contents; d2h += result_bytes(r); nl += r.kernel_launches
-                kern += sum(getattr(r, s) for s in STAGES); ctx.release(t)
-            for _ in range(k):
+                t, last = inflight.pop(0); r = ctx.wait(t).contents; d2h += result_bytes(r); nl += r.kernel_launches
+                kern += sum(getattr(r, s) for s in STAGES)
+                if last:   # --dump-outputs: the last step's tickets stay unreleased, in batch order, until the timed window has closed
+                    held.append((t, r))
+                else:
+                    ctx.release(t)
+            for s in range(k):
                 for (b, _), (lo, hi) in zip(slices, spans):
                     if len(inflight) >= P.n_streams:
                         retire()
                     if repack:
                         rois.pack(lo, hi, P, b)
-                    inflight.append(ctx.submit(b))
+                    inflight.append((ctx.submit(b), held is not None and s == k - 1))
             while inflight:
                 retire()
             return d2h, nl, kern
 
-        def timed_e2e(repack):
+        def timed_e2e(repack, held=None):
             e2e_steps(args.warmup, repack)
             barrier()
             t0 = time.perf_counter()
-            d2h, nl, kern = e2e_steps(args.steps, repack)
+            d2h, nl, kern = e2e_steps(args.steps, repack, held)
             barrier()
             return time.perf_counter() - t0, d2h // max(1, args.steps), nl, kern
-        e2e_s, d2h_bytes, nl, e2e_kern_ms = timed_e2e(False)
+        if args.dump_outputs and len(slices) > P.n_streams:
+            # a held ticket keeps its lane: the last step's batches must all be in flight at once
+            raise SystemExit("--dump-outputs needs --e2e-batches <= %d (the library's streams)" % P.n_streams)
+        held = [] if args.dump_outputs else None
+        e2e_s, d2h_bytes, nl, e2e_kern_ms = timed_e2e(False, held)
+        if args.dump_outputs:
+            dumped = dump_results([result_tables(r) for _, r in held])
+            for t, _ in held:
+                ctx.release(t)
         launches += nl
         pk_s, _, nl, pk_kern_ms = timed_e2e(True)
         launches += nl
@@ -464,6 +604,8 @@ def main():
         extra["host_cascade_ms_per_step"] = 1000.0 * sum(a[3] for a in acc) / args.steps
         extra["merge_ms_per_step"] = 1000.0 * sum(a[4] for a in acc) / args.steps
         merged, mine_raw = acc[-1][5], acc[-1][6]
+        if rank == 0 and args.dump_outputs:
+            dumped = dump_text(merged)
     sampler.stop_flag = True; sampler.join(timeout=2)
 
     # max over ranks
@@ -573,6 +715,8 @@ def main():
                                     "ksw2_gcups": None if use_ref else (cnt["cells_a"] + cnt["cells_b"]) / cnt["seconds"] / 1e9,
                                     "sample": "first %d regions of the same workload, single thread (the reference is single-threaded on this path); CPU oracle%s" % (
                                         n, " calling the reference's own ksw2_extz2_sse.c compiled unmodified (oracle/_ref)" if use_ref else " with its own lane-exact ksw2")}
+        if args.dump_outputs:
+            write_dump(args.dump_outputs, dumped)
         print(json.dumps(line), file=OUT, flush=True)
     for b, _ in slices + ([(big, 0)] if mode == "weak" else []):
         ctx.batch_free(b)

@@ -3,6 +3,9 @@
 KATs: src/ksw2/ksw2.nim:166-239 (suite "ksw2 suite") and SURVEY.md appendix F (values obtained by running the
 reference C here). Fuzz: lane model == compiled reference on every ksw_extz_t field and the full CIGAR.
 """
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
@@ -103,3 +106,34 @@ def test_lane_model_equals_compiled_reference_fuzz():
         f1, c1, _ = orc.ksw2(q, t, gapo=go, gape=1, w=w, zdrop=z, impl="ref")
         f2, c2, _ = orc.ksw2(q, t, gapo=go, gape=1, w=w, zdrop=z, impl="lane")
         assert f1 == f2 and c1 == c2, (it, len(q), len(t), go, w, z, f1, f2, orc.cigar_str(c1), orc.cigar_str(c2))
+
+
+LANE_FUZZ = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ksw2_lane_fuzz.npz")
+
+
+def lane_fuzz_pairs():
+    """the 6 000 pairs of test_lane_model_equals_compiled_reference_fuzz"""
+    rng = np.random.default_rng(20171101)
+    return [random_pair(rng) for _ in range(6000)]
+
+
+def pairs_digest(pairs):
+    """SHA-256 over every pair's parameters and sequences: the inputs the recorded results belong to"""
+    h = hashlib.sha256()
+    for q, t, go, w, z in pairs:
+        h.update(np.array([len(q), len(t), go, w, z], dtype=np.int64).tobytes() + q.tobytes() + t.tobytes())
+    return h.hexdigest()
+
+
+def test_lane_model_reproduces_its_recorded_fuzz_results():
+    """Regression vectors, not the reference's output: tests/golden/ksw2_lane_fuzz.npz holds what the lane model (oracle/ksw2_lane.c)
+    computes on the pairs of the fuzz above, recorded with ksw2_lane.c as it has been since that fuzz was written.  Any change to the
+    lane model's fields or CIGARs fails here even where the compiled reference is not built; where it is built, the fuzz above
+    compares the lane model with the reference itself."""
+    pairs = lane_fuzz_pairs()
+    g = np.load(LANE_FUZZ)
+    assert str(g["made_with"]) == "lane" and str(g["inputs_sha256"]) == pairs_digest(pairs), "the fuzz pairs are not the recorded ones"
+    off = np.concatenate([[0], np.cumsum(np.maximum(g["fields"][:, orc.EZ_FIELDS.index("n_cigar")], 0))])
+    for it, (q, t, go, w, z) in enumerate(pairs):
+        f, c, _ = orc.ksw2(q, t, gapo=go, gape=1, w=w, zdrop=z, impl="lane")
+        assert [f[k] for k in orc.EZ_FIELDS] == g["fields"][it].tolist() and list(c) == g["cigar"][off[it]:off[it + 1]].tolist(), (it, f, orc.cigar_str(c))
