@@ -190,7 +190,7 @@ typedef struct idl_aln_result {
 #define IDL_EV_LOW_CPLX  2   /* :266 */
 #define IDL_EV_BUG_SAME  3   /* :268-275 */
 #define IDL_EV_SHORT    10   /* :234 */
-#define IDL_EV_WINDOW   11   /* reference window shorter than K (the reference would raise) */
+#define IDL_EV_WINDOW   11   /* reference window or contig shorter than K (the reference would raise) */
 #define IDL_EV_DP_ERROR 12   /* the alignment hit a capacity limit (idl_aln_result.status) */
 #define IDL_NO_EVENTS 0xffffffffu /* idl_aln_result.event_begin when no event records were written */
 

@@ -595,12 +595,15 @@ void callsemble(const Roi &r, const Fai &fai, const std::string &chrom, const or
 				offset = std::min<int64_t>(qloc.start, ctg.len() - qloc.stop - 1);
 				qstart = std::max<int64_t>(qloc.start - width, 0);
 				if (qstart + K > ctg.len()) qstart = ctg.len() - K;
+				// a contig shorter than K (min_ctg_len < K): the reference would raise here as well; no k-mers are reported
+				if (qstart < 0) { ref_kmer.clear(); reject = 11; break; }
 				alt_kmer = ctg.seq.substr(qstart, K);
 				if (alt_kmer == ref_kmer) {
 					qstart = std::max<int64_t>(qloc.start - 3, 0);
 					if (qstart + K > ctg.len()) {
 						int64_t qend = std::min<int64_t>(qloc.stop + 4, ctg.len());
 						qstart = qend - K;
+						if (qstart < 0) { ref_kmer.clear(); alt_kmer.clear(); reject = 11; break; }
 						alt_kmer = ctg.seq.substr(qstart, K);
 					} else alt_kmer = ctg.seq.substr(qstart, K);
 				}

@@ -73,21 +73,211 @@ def rois_from_reads(reads, chrom_seq, roi_start=None, roi_stop=None, chrom_name=
     return host.Rois(arrays=arrays), arrays
 
 
-def merge_rois(list_of_arrays):
-    """concatenate several one-chromosome region sets that share the same chromosome into one"""
+def merge_rois(list_of_arrays, chroms=None, chrom_names=None, chrom_seqs=None):
+    """concatenate several one-chromosome region sets into one.  Without `chroms` they share the first set's chromosome; with it,
+    set k lies on chromosome chroms[k] of chrom_names / chrom_seqs"""
     out = {k: [] for k in ("start", "stop", "mapq", "flag", "len", "seq_off", "bases", "quals", "roi_chrom", "roi_start", "roi_stop", "roi_read_begin",
                            "roi_n_reads", "read_idx")}
     nread = nbase = nidx = 0
-    for a in list_of_arrays:
-        for k in ("start", "stop", "mapq", "flag", "len", "bases", "quals", "roi_chrom", "roi_start", "roi_stop", "roi_n_reads"):
+    for j, a in enumerate(list_of_arrays):
+        for k in ("start", "stop", "mapq", "flag", "len", "bases", "quals", "roi_start", "roi_stop", "roi_n_reads"):
             out[k].append(a[k])
+        out["roi_chrom"].append(a["roi_chrom"] if chroms is None else np.full(len(a["roi_chrom"]), chroms[j], np.int32))
         out["seq_off"].append(a["seq_off"] + nbase)
         out["roi_read_begin"].append(a["roi_read_begin"] + nidx)
         out["read_idx"].append(a["read_idx"] + nread)
         nread += len(a["start"]); nbase += len(a["bases"]); nidx += len(a["read_idx"])
     m = {k: np.concatenate(v) for k, v in out.items()}
-    m["chrom_names"] = list_of_arrays[0]["chrom_names"]; m["chrom_seqs"] = list_of_arrays[0]["chrom_seqs"]
+    if chroms is None:
+        m["chrom_names"] = list_of_arrays[0]["chrom_names"]; m["chrom_seqs"] = list_of_arrays[0]["chrom_seqs"]
+    else:
+        m["chrom_names"] = list(chrom_names)
+        m["chrom_seqs"] = [np.frombuffer(s.encode(), dtype=np.uint8) if isinstance(s, str) else s for s in chrom_seqs]
     return m
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# Directed regions at chromosome ends: reads of a haplotype (reference + edits, with soft-clipped bases in front of the chromosome
+# start or past its end), each with its CIGAR, so that one set of reads makes both the Rois arrays and a BAM file
+# ---------------------------------------------------------------------------------------------------------------
+def random_seq(rng, n, alphabet="ACGT"):
+    return "".join(alphabet[i] for i in rng.integers(0, len(alphabet), n))
+
+
+def haplotype(ref, edits=(), lead="", tail=""):
+    """per-base list of (base, reference position or None, kind in M/I/S).  edits: (pos, "I", seq) inserts seq before ref[pos];
+    (pos, "D", n) deletes ref[pos:pos + n].  lead / tail: bases before position 0 / after the chromosome's end (soft clips)"""
+    ed = {p: (k, a) for p, k, a in edits}
+    out = [(c, None, "S") for c in lead]
+    i = 0
+    while i < len(ref):
+        k, a = ed.get(i, (None, None))
+        if k == "D":
+            i += a
+            continue
+        if k == "I":
+            out += [(c, None, "I") for c in a]
+        out.append((ref[i], i, "M"))
+        i += 1
+    return out + [(c, None, "S") for c in tail]
+
+
+def hap_read(hp, at, n, qual=None, mapq=60, flag=0):
+    """the read of bases [at, at + n) of a haplotype: dict(start, stop, seq, qual, mapq, flag, cigar) as rois_from_reads and
+    bam_record take them; insertions at either end of the read become soft clips"""
+    seg = hp[at:at + n]
+    m = [i for i, (_, p, _) in enumerate(seg) if p is not None]
+    assert m, "a read needs an aligned base"
+    cig, prev = [], None
+    for i, (_, p, k) in enumerate(seg):
+        if k == "I" and (i < m[0] or i > m[-1]):
+            k = "S"
+        if p is not None and prev is not None and p > prev + 1:
+            cig.append(["D", p - prev - 1])
+        if cig and cig[-1][0] == k:
+            cig[-1][1] += 1
+        else:
+            cig.append([k, 1])
+        if p is not None:
+            prev = p
+    seq = "".join(b for b, _, _ in seg)
+    return dict(start=seg[m[0]][1], stop=prev + 1, seq=seq, qual=[30] * len(seq) if qual is None else list(qual), mapq=mapq, flag=flag,
+                cigar=[(k, ln) for k, ln in cig])
+
+
+def _lowq(n, lead=0, trail=0):
+    return [4] * lead + [30] * (n - lead - trail) + [6] * trail
+
+
+def edge_fixtures(seed=2026):
+    """Three chromosomes whose regions sit at their ends.  Returns dict(names, seqs, reads: one list per chromosome sorted by start,
+    regions: (chromosome, start, stop) in pool order).  In pool order the region at the end of chrA is followed by the region at the
+    start of chrB.  Every event's position is chosen so that a path that exists only at an edge is taken:
+      chrA start  reads from position 0 (some with low-quality leading bases, some soft-clipped in front of the chromosome),
+                  an insertion 12 and a deletion 30 bases from the start
+      chrA middle homopolymer, {A,C}-only and ACG-repeat flanks (rejects of equal / low-complexity k-mers)
+      chrA end    a tandem-repeat expansion (AL fallback) 80 bases before the end and 5 extra bases in the 14-base homopolymer that
+                  ends the chromosome (equal k-mers, then the qend branch); reads end exactly at the end
+      chrB start  a homopolymer run at position 0 with 5 extra bases
+      chrB middle contigs that start 2 bases before a homopolymer with 5 extra bases (equal k-mers on both tries); 26-base reads
+                  with an insertion: a contig shorter than K
+      chrB end    contigs that start 20 bases before the end: 8 matching bases, a 5-base insertion, 12 matching bases, then bases
+                  past the end -- a reference window shorter than K
+      chrC        120 bp, shorter than one read, reads soft-clipped at both ends"""
+    rng = np.random.default_rng(seed)
+    names, seqs, reads, regions = ["chrA", "chrB", "chrC"], [], [[], [], []], []
+    RL = 150
+
+    # ---- chrA: 2600 bp
+    a = list(random_seq(rng, 2600))
+    a[1100:1145] = "A" * 45                                         # homopolymer
+    a[1300:1380] = random_seq(rng, 80, "AC")                        # only A and C: every k-mer has < 3 distinct bases
+    a[1600:1660] = "ACG" * 20                                       # 3-base repeat
+    a[2520:2560] = "ACGTT" * 8                                      # tandem repeat 80..40 bases before the end
+    a[2586:2600] = "A" * 14                                         # homopolymer that ends the chromosome
+    A = "".join(a)
+    seqs.append(A)
+    ref0 = haplotype(A)
+    alt0 = haplotype(A, [(12, "I", "GTTCA"), (30, "D", 6)])
+    clip0 = haplotype(A, [(12, "I", "GTTCA"), (30, "D", 6)], lead="TGCAT")
+    for k, at in enumerate([0, 0, 0, 1, 2, 4, 6, 9]):
+        reads[0].append(hap_read(alt0, at, RL, qual=_lowq(RL, lead=6 if k % 3 == 1 else 0)))
+    for at in (0, 0, 3, 5, 8, 11):
+        reads[0].append(hap_read(ref0, at, RL, qual=_lowq(RL, lead=5 if at == 3 else 0)))
+    for k in range(4):
+        reads[0].append(hap_read(clip0, 0, RL, mapq=60 if k else 35))
+    regions.append((0, 0, 40))
+    # middle: equal / low-complexity k-mers
+    mid = haplotype(A, [(1110, "I", "AAAAA"), (1200, "D", 3), (1330, "D", 6), (1615, "I", "ACGACG")])
+    for at in range(980, 1500, 12):
+        reads[0].append(hap_read(mid if (at // 12) % 3 else ref0, at, RL))
+    regions.append((0, 1100, 1380))
+    for at in range(1500, 1640, 10):
+        reads[0].append(hap_read(mid if (at // 10) % 3 else ref0, at, RL))
+    regions.append((0, 1600, 1640))
+    # end: a tandem-repeat expansion (AL fallback) and 5 extra bases in the 14-base homopolymer that ends the chromosome: both k-mers
+    # equal at first, the second try reaches past the contig's end and takes the qend branch; every read ends at or before the end
+    endA = haplotype(A, [(2520, "I", "ACGTT"), (2586, "I", "AAAAA")])
+    for k, back in enumerate([150, 150, 150, 150, 153, 157, 160, 164, 168]):
+        reads[0].append(hap_read(endA, len(endA) - back, RL, qual=_lowq(RL, trail=4 if k == 5 else 0)))
+    for back in (150, 150, 152, 156, 161, 166):
+        reads[0].append(hap_read(ref0, 2600 - back, RL))
+    regions.append((0, 2520, 2600))
+
+    # ---- chrB: 2000 bp, a homopolymer at position 0 and contigs starting 20 bases before the end
+    b = list(random_seq(rng, 2000))
+    b[0:45] = "A" * 45
+    b[998:1040] = "GC" + "A" * 40                                   # contigs start 2 bases before a homopolymer: equal k-mers twice
+    B = "".join(b)
+    seqs.append(B)
+    altB = haplotype(B, [(0, "I", "AAAAA")])
+    refB = haplotype(B)
+    for at in (0, 0, 0, 2, 4, 7):
+        reads[1].append(hap_read(altB, at, RL))
+    for at in (0, 0, 3, 6):
+        reads[1].append(hap_read(refB, at, RL))
+    regions.append((1, 0, 45))
+    altB2 = haplotype(B, [(1000, "I", "AAAAA")])
+    for _ in range(5):
+        reads[1].append(hap_read(altB2, 998, RL))
+    for at in (990, 994, 1001, 1004):
+        reads[1].append(hap_read(refB, at, RL))
+    regions.append((1, 995, 1045))
+    short = haplotype(B, [(1510, "I", "TCA")])                    # 26-base reads: a contig shorter than K (it aligns under -c 26)
+    for _ in range(6):
+        reads[1].append(hap_read(short, 1500, 26))
+    regions.append((1, 1505, 1515))
+    tailB = random_seq(rng, 140)
+    shortwin = haplotype(B, [(1988, "I", "CTTAG")], tail=tailB)
+    at = len(shortwin) - len(tailB) - 25                       # 8 + 5 + 12 bases before the end
+    for _ in range(6):
+        reads[1].append(hap_read(shortwin, at, RL))
+    refBe = haplotype(B, tail=tailB)
+    for back in (150, 147, 143, 140):
+        reads[1].append(hap_read(refBe, len(refBe) - len(tailB) - back, RL))
+    regions.append((1, 1970, 2000))
+
+    # ---- chrC: 120 bp, shorter than one read
+    C_ = random_seq(rng, 120)
+    seqs.append(C_)
+    lead, trail = random_seq(rng, 20), random_seq(rng, 20)
+    altC = haplotype(C_, [(60, "D", 6)], lead=lead, tail=trail)
+    refC = haplotype(C_, lead=lead, tail=trail)
+    for k in range(6):
+        reads[2].append(hap_read(altC, k % 3, 150 - 6 - (k % 3) * 2))
+    for k in range(4):
+        reads[2].append(hap_read(refC, k % 2, 150 - (k % 2)))
+    regions.append((2, 0, 120))
+    for r in reads:
+        r.sort(key=lambda x: x["start"])
+    return dict(names=names, seqs=seqs, reads=reads, regions=regions)
+
+
+def edge_rois(fx, extra=None):
+    """the fixtures as one Rois: a region holds the reads of its chromosome that overlap it (src/indelope.nim:449-452).  extra: optional
+    (name, sequence, arrays of a one-chromosome region set) appended as a fourth chromosome"""
+    sets, chroms = [], []
+    for c, lo, hi in fx["regions"]:
+        rr = [r for r in fx["reads"][c] if not (r["start"] > hi) and not (r["stop"] < lo)]
+        sets.append(rois_from_reads(rr, fx["seqs"][c], roi_start=lo, roi_stop=hi)[1]); chroms.append(c)
+    names, seqs = list(fx["names"]), list(fx["seqs"])
+    if extra is not None:
+        sets.append(extra[2]); chroms.append(len(names)); names.append(extra[0]); seqs.append(extra[1])
+    arrays = merge_rois(sets, chroms, names, seqs)
+    return host.Rois(arrays=arrays), arrays
+
+
+def edge_files(fx, directory):
+    """the fixtures as <directory>/edges.fa and <directory>/edges.bam (records with S operations, BGZF)"""
+    fa, bam = os.path.join(str(directory), "edges.fa"), os.path.join(str(directory), "edges.bam")
+    with open(fa, "w") as f:
+        for n, s in zip(fx["names"], fx["seqs"]):
+            f.write(">%s\n%s\n" % (n, "\n".join(s[i:i + 60] for i in range(0, len(s), 60))))
+    recs = [bam_record(c, r["start"], r["cigar"], r["seq"], qual=r["qual"], mapq=r["mapq"], flag=r["flag"], name=b"e%d_%d" % (c, k))
+            for c, rr in enumerate(fx["reads"]) for k, r in enumerate(rr)]
+    with open(bam, "wb") as f:
+        f.write(bgzf_compress(bam_bytes([(n, len(s)) for n, s in zip(fx["names"], fx["seqs"])], recs)))
+    return fa, bam
 
 
 def out_dir():

@@ -13,12 +13,12 @@ from oracle import pyoracle as orc
 pytestmark = pytest.mark.gpu
 
 
-def run_both(rois, arrays, min_reads=5, min_ctg_len=73, min_event_len=5, level=31, tag="x", **kw):
+def run_both(rois, arrays, min_reads=5, min_ctg_len=73, min_event_len=5, level=31, tag="x", max_reads=400_000, **kw):
     from indelope_b200 import api
     caller = api.Caller(0, min_reads=min_reads, min_ctg_len=min_ctg_len, min_event_len=min_event_len, out_flags=abi.OUT_SUPPORT, **kw)
     try:
         tm = []
-        vcf, dump = caller.call(rois, dump_level=level, timings=tm)
+        vcf, dump = caller.call(rois, dump_level=level, timings=tm, max_reads=max_reads)
     finally:
         caller.close()
     # the oracle runs the reference's own compiled ksw2_extz2_sse.c when oracle/_ref was built (it travels to the GPU box)
