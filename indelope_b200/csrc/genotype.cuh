@@ -2,7 +2,7 @@
 //
 //   sort_*        bucket sort of alignment tasks by estimated anti-diagonals, longest first: the 32/G alignments that
 //                 share a warp run in lockstep, so they should have similar lengths
-//   align_kernel  call-site A of kernel 2 (contig -> reference window, bw=50 z=400, :213-221) followed, in the same
+//   align4_kernel call-site A of kernel 2 (contig -> reference window, bw=50 z=400, :213-221) followed, in the same
 //                 group, by the glue: truncated CIGAR (src/ksw2/ksw2.nim:22-33), target/query event locations
 //                 (:71-91), ref/alt 27-mer selection and rejects (src/indelope.nim:229-281), get_min_flank (:118-132)
 //   kmer_kernel   kernel 3: ref/alt canonical 27-mer counting over the reads of the region (:283-311), one CTA per
@@ -13,25 +13,12 @@
 #include "common.cuh"
 #include "ksw2.cuh"
 #include "ksw2_rows.cuh"
-#include "ksw2_band.cuh"
 
 #define DP_WARPS 8
 #define DP_THREADS (DP_WARPS * 32)
 #define KMER_THREADS 128
 #define DP_G 8          // threads per alignment
 #define DP_NG (32 / DP_G)
-#ifndef KSW_A_CTAS
-#define KSW_A_CTAS 3 /* resident CTAs per SM of the banded call-site */
-#endif
-#ifndef KSW_BAND_G
-#define KSW_BAND_G 8 /* threads per alignment of the register-ring variant of the banded call-site (4 or 8) */
-#endif
-#ifndef KSW_BAND_WARPS
-#define KSW_BAND_WARPS 8 /* warps per CTA of the register-ring variant: 2 CTAs x 8 warps = 4 warps per scheduler at up to 128 registers */
-#endif
-#ifndef KSW_BAND_CTAS
-#define KSW_BAND_CTAS 2
-#endif
 #ifndef KSW_UNB_WARPS
 #define KSW_UNB_WARPS 5 /* warps per CTA of the unbanded al_kernel.  Measured on the chr1 workload (ms): 8 warps x 2 CTAs at 124 registers
                            22.0, 8 x 3 at 80 24.7, 10 x 2 at 95 21.8, 6 x 3 at 96 21.2, 7 x 3 at 80 21.8, 5 x 4 at 94 21.0, 2 x 10 at 94 21.0:
@@ -162,21 +149,20 @@ __device__ __forceinline__ int distinct_k(const uint8_t *a, int K)
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// call-site A + glue: one group of DP_G threads per alignment, DP_NG alignments per warp
+// call-site A + glue: one group of G threads per alignment, 32 / G alignments per warp
 // ---------------------------------------------------------------------------------------------------------------
-// BAND: the register-ring variant (ksw2_band.cuh), G threads per alignment; otherwise the column-owned shared-memory variant, 8 threads
-template <int G, bool BAND>
+template <int G>
 __device__ __forceinline__ void align_body(const GenoArgs &g, unsigned char *smem_raw)
 {
-	constexpr int GG = G, NGG = 32 / G;
-	const int lane = lane_id(), gl = lane & (GG - 1), grp = lane / GG;
-	const unsigned gmask = (GG == 32 ? 0xffffffffu : ((1u << GG) - 1u)) << (lane & ~(GG - 1));
+	constexpr int NG = 32 / G;
+	const int lane = lane_id(), gl = lane & (G - 1), grp = lane / G;
+	const unsigned gmask = ((1u << G) - 1u) << (lane & ~(G - 1));
 	const idl_params &P = g.P;
 	const int K = IDL_KMER, width = (K + 1) / 2 - 1; // :218
 	const unsigned n_alns = g.cnt->n_alns < g.cap_alns ? g.cnt->n_alns : g.cap_alns;
 	for (;;) {
 		unsigned base = 0;
-		if (lane == 0) base = atomicAdd(&g.cnt->aln_next, (unsigned)NGG);
+		if (lane == 0) base = atomicAdd(&g.cnt->aln_next, (unsigned)NG);
 		base = __shfl_sync(FULL_MASK, base, 0);
 		if (base >= n_alns) break;
 		const bool valid = base + grp < n_alns;
@@ -189,8 +175,7 @@ __device__ __forceinline__ void align_body(const GenoArgs &g, unsigned char *sme
 		KswQuery kq; kq.codes = qq; kq.seq2 = nullptr; kq.seqn = nullptr; kq.base = 0;
 		const KswMem M = dp_mem<G>(g, smem_raw, cr.len, tlen, (int)(blockDim.x >> 5));
 		KswOut o;
-		if constexpr (BAND) ksw2_band<G, true>(valid, cr.len, kq, tlen, tq, g.kpA, M, o); // the whole warp: 32 / G alignments in lockstep
-		else ksw2_group<G>(valid, cr.len, kq, tlen, tq, g.kpA, M, o);
+		ksw2_group<G>(valid, cr.len, kq, tlen, tq, g.kpA, M, o);
 		if (valid) {
 			const uint32_t *cg = M.cig;
 			const int n = o.n_cigar;
@@ -199,17 +184,17 @@ __device__ __forceinline__ void align_body(const GenoArgs &g, unsigned char *sme
 				ntr = ksw_trunc_count(cg, n, o.max_q);
 				for (int k = 0; k < ntr; ++k) nev += (cg[n - 1 - k] & 0xf) != 0;
 			}
-			ntr = __shfl_sync(gmask, ntr, 0, GG); nev = __shfl_sync(gmask, nev, 0, GG);
+			ntr = __shfl_sync(gmask, ntr, 0, G); nev = __shfl_sync(gmask, nev, 0, G);
 			unsigned coff = 0, eoff = 0;
 			const bool want_events = (P.stages & IDL_STAGE_GENOTYPE) && nev >= 1 && nev <= P.max_events; // :229
 			if (gl == 0) {
 				coff = atomicAdd(&g.cnt->n_cigar_ops, (unsigned)n);
 				if (want_events) eoff = atomicAdd(&g.cnt->n_events, (unsigned)nev);
 			}
-			coff = __shfl_sync(gmask, coff, 0, GG); eoff = __shfl_sync(gmask, eoff, 0, GG);
+			coff = __shfl_sync(gmask, coff, 0, G); eoff = __shfl_sync(gmask, eoff, 0, G);
 			unsigned st = dp_status_bits(o.status);
 			if (coff + (unsigned)n > g.cap_cigar) { st |= IDL_RS_CIGAR_OVERFLOW; if (gl == 0) atomicOr(&g.cnt->overflow, 8u); }
-			else for (int k = gl; k < n; k += GG) g.cigar[coff + k] = cg[n - 1 - k]; // forward order
+			else for (int k = gl; k < n; k += G) g.cigar[coff + k] = cg[n - 1 - k]; // forward order
 			bool ev_ok = want_events;
 			if (ev_ok && eoff + (unsigned)nev > g.cap_events) { ev_ok = false; if (gl == 0) atomicOr(&g.cnt->overflow, 16u); }
 			if (gl == 0) {
@@ -289,29 +274,19 @@ __device__ __forceinline__ void align_body(const GenoArgs &g, unsigned char *sme
 		__syncwarp();
 	}
 }
-
-__global__ void __launch_bounds__(DP_THREADS, KSW_A_CTAS) align_kernel(GenoArgs g) // any band width: the shared-memory rings
-{
-	extern __shared__ __align__(16) unsigned char smem_raw[];
-	align_body<8, false>(g, smem_raw);
-}
 #ifndef KSW_A4_WARPS
 #define KSW_A4_WARPS 4
 #endif
 #ifndef KSW_A4_CTAS
 #define KSW_A4_CTAS 4
 #endif
-// the same shared-memory rings with FOUR threads per alignment, eight alignments per warp in lockstep: the per-diagonal control code (band,
-// exact-score bookkeeping, z-drop, block entry) is issued once for twice as many alignments and the words of a diagonal fill the rounds
+// the shared-memory rings with FOUR threads per alignment, eight alignments per warp in lockstep: the per-diagonal control code (band,
+// exact-score bookkeeping, z-drop, block entry) is issued once for eight alignments and the words of a diagonal fill the rounds
+// (eight threads per alignment measured 12.9 against 10.1 ms on chr1, DESIGN.md 4.2)
 __global__ void __launch_bounds__(32 * KSW_A4_WARPS, KSW_A4_CTAS) align4_kernel(GenoArgs g)
 {
 	extern __shared__ __align__(16) unsigned char smem_raw[];
-	align_body<4, false>(g, smem_raw);
-}
-__global__ void __launch_bounds__(32 * KSW_BAND_WARPS, KSW_BAND_CTAS) align_band_kernel(GenoArgs g) // rounded bands of up to 96 lanes (w <= 79): the ring in registers
-{
-	extern __shared__ __align__(16) unsigned char smem_raw[];
-	align_body<KSW_BAND_G, true>(g, smem_raw);
+	align_body<4>(g, smem_raw);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -26,18 +26,7 @@ struct KswOut {
 	long long cells;  // exact in-band cells over executed diagonals
 };
 
-#ifndef KSW_PSTORE_MODE
-#define KSW_PSTORE_MODE 1 /* streaming stores: the backtrack matrix is written once and read back once, in part */
-#endif
-#if KSW_PSTORE_MODE == 1
-#define KSW_PSTORE(p, v) __stcs((p), (v))
-#elif KSW_PSTORE_MODE == 2
-#define KSW_PSTORE(p, v) __stwt((p), (v))
-#elif KSW_PSTORE_MODE == 3
-#define KSW_PSTORE(p, v) __stcg((p), (v))
-#else
-#define KSW_PSTORE(p, v) (*(p) = (v))
-#endif
+#define KSW_PSTORE(p, v) __stcs((p), (v)) /* streaming stores: the backtrack matrix is written once and read back once, in part */
 #define KSW_BTILE_BYTES 1152 /* backtrack tile: 32 rows of nine aligned words */
 #define KSW_BTILE_ROW 36
 #define KSW_QR_PAD 32     /* zero bytes in front of the reversed query: lanes left of the exact band index it below 0 */
@@ -238,9 +227,6 @@ __device__ __forceinline__ void ksw_core_word(const KswParams &P, bool fast_ok, 
 // not merge requests to a sector that is in flight, so every word cost a sector at the L2 and, the lines being long evicted, in DRAM:
 // al_kernel read 31.7 GB back for the 20.4 GB it wrote.)  lo / hi bound the byte offsets that may be touched (the workspace of this
 // alignment incl. its padding); a row whose entry bytes lie outside is never read by the walk (its state is forced there).
-#ifndef KSW_TILE_LD
-#define KSW_TILE_LD 1
-#endif
 // one word of the backtrack matrix into the shared-memory tile: an asynchronous copy (LDGSTS), so that the 33 words a thread moves per
 // tile are all in flight at once without holding 33 registers -- one DRAM round trip per tile, not one per batch of loads -- and with
 // the L2 prefetch size capped at 64 bytes: a plain ld.global pulled 128 bytes around every word it missed, four sectors per row of
@@ -248,13 +234,7 @@ __device__ __forceinline__ void ksw_core_word(const KswParams &P, bool fast_ok, 
 __device__ __forceinline__ void ksw_tile_cp(uint32_t *dst, const uint32_t *src)
 {
 	const uint32_t d = (uint32_t)__cvta_generic_to_shared(dst);
-#if KSW_TILE_LD == 1
 	asm volatile("cp.async.ca.shared.global.L2::64B [%0], [%1], 4;" :: "r"(d), "l"(src) : "memory");
-#elif KSW_TILE_LD == 2
-	asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" :: "r"(d), "l"(src) : "memory");
-#else
-	uint32_t v; asm volatile("ld.global.L1::no_allocate.L2::64B.u32 %0, [%1];" : "=r"(v) : "l"(src)); *dst = v;
-#endif
 }
 __device__ __forceinline__ void ksw_tile_wait() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 template <int G = 8, class F>

@@ -59,13 +59,11 @@ template <bool FRONT, bool WILD>
 __device__ __forceinline__ void ksw_rows_word(const KswParams &P, uint32_t m, uint32_t pc, uint32_t tw, uint32_t qv,
                                               uint32_t &x, uint32_t &v, uint32_t &u, uint32_t &y, uint32_t &gx, uint32_t &gy, uint32_t &dm2, uint32_t &chk, uint32_t *pdst)
 {
-	const uint32_t MAXSC = P.maxsc_4, Q4 = P.q_4;
+	const uint32_t Q4 = P.q_4;
 	const uint32_t ut = prmt(u, pc, 0x2106), yt = prmt(y, pc, 0x2107); // u, y of rows 4w-1 .. 4w+2 (previous diagonal)
 	uint32_t z0 = sel4(msb_to_mask4((tw ^ qv) + 0x7f7f7f7fu), P.misq_4, P.maxsc_4);
 	if (WILD) z0 = sel4(msb_to_mask4(((tw ^ 0x04040404u) + 0x7f7f7f7fu) & ((qv ^ 0x04040404u) + 0x7f7f7f7fu)), z0, P.qe2_4); // a code 4 on either side scores 0 (:219,226)
-#ifndef KSW_ROWS_NOCHK /* the proof after the fact that the carry-free form was exact: 0.51 of 19.3 ms */
-	chk |= x | v; chk |= ut | yt;
-#endif
+	chk |= x | v; chk |= ut | yt; // the proof after the fact that the carry-free form was exact: 0.51 of 19.3 ms
 	const uint32_t a = x + v, b = yt + ut;
 	uint32_t mk = ge4_pos(z0, a);                   // z >= a
 	uint32_t z = sel4(mk, z0, a);
@@ -73,12 +71,7 @@ __device__ __forceinline__ void ksw_rows_word(const KswParams &P, uint32_t m, ui
 	mk = ge4_pos(z, b);                             // z >= b
 	d = sel4(mk, d, 0x02020202u);
 	z = sel4(mk, z, b);
-#ifdef KSW_ROWS_WITH_MIN /* z = min(z, match + 2(q+e)) of :132: a no-op here.  z is H(t,j) - H(t-1,j-1) + 2(q+e) and a step along the main diagonal
-	   of an affine-gap DP gains at most the match score (Suzuki & Kasahara 2018, the bound ksw2's int8 lanes rest on); this variant computes real
-	   cells only (rows >= qlen are real cells of the query-extended problem, parked lanes are overwritten), so the clamp the reference needs
-	   for the stale lanes of its rounded band never binds.  0.64 of 19.3 ms; every parity test runs without it. */
-	z = sel4(msb_to_mask4(P.maxsc_h80 - z), z, MAXSC); // min(z, max score)
-#endif
+	// no z = min(z, match + 2(q+e)) of :132: on real cells a diagonal step gains at most the match score, so it never binds (DESIGN.md 4.2b)
 	const uint32_t zh = z | KSW_H80;
 	uint32_t un = (zh - v) ^ KSW_H80, vn = (zh - ut) ^ KSW_H80;
 	z -= Q4;
@@ -240,19 +233,7 @@ __device__ void ksw2_rows(bool valid, int qlen, const KswQuery query, int tlen, 
 				if (lo0 - 32 * s_hi < 3) pm = 1u << s_hi;          // the word of row r: lanes in front of t = 0
 				if (lo0 - 32 * s_lo > tlen - 1) pm |= 1u << s_lo;  // the word of row r - tlen: lanes past the target end
 			}
-			// KSW_ROWS_FULL_SECTORS: a slot is run by ALL EIGHT threads of the group as soon as one of them has a live word in it (thread 0 reaches the highest slot, thread
-			// 7 the lowest): the others' words are wholly in front of t = 0 or wholly past t = tlen-1 and stay parked behind an all-zero mask, in
-			// the same instruction stream (the word of row r / row r - tlen puts the slot on the masked path anyway).  Their backtrack words are
-			// never read, but the group then writes whole 32-byte sectors: a partly written sector is FETCHED from DRAM before it is written
-			// back (38 % of the sectors al_kernel wrote were, 7.8 GB of DRAM reads per launch that no load asked for).
-			// MEASURED: DRAM reads 20.4 -> 13.4 GB per launch, but 528 G instead of 440 G thread instructions and 20.3 instead of 19.1 ms: off by
-			// default.  (The uniform slot count `nsq` above already makes the tail of the last slot whole at no cost.)
-#ifdef KSW_ROWS_FULL_SECTORS
-			int g_hi = r >> 5, g_lo = (r - tlen + 1) >> 5;
-			g_hi = g_hi < nsq ? g_hi : nsq - 1; g_lo = g_lo > 0 ? g_lo : 0;
-			const unsigned gonm = (act && g_hi >= g_lo) ? (((2u << g_hi) - 1u) & ~((1u << g_lo) - 1u)) : 0u;
-			pm |= gonm & ~onm; onm = gonm;
-#endif
+			// only threads with a live word run a slot: whole sectors on the band's ramps cut DRAM fill reads but cost 1.2 ms (DESIGN.md 4.2c)
 			dg.onm = onm; dg.uon = __reduce_or_sync(FULL_MASK, onm); dg.upm = __reduce_or_sync(FULL_MASK, pm);
 		}
 		dg.lo0 = lo0; dg.tlen = tlen; dg.gl = gl; dg.srcl = srcl; dg.bconst = bconst; dg.taddr = taddr; dg.tsh = tsh; dg.prow = prow;
@@ -348,9 +329,6 @@ __device__ void ksw2_rows(bool valid, int qlen, const KswQuery query, int tlen, 
 	// barriers the four walkers drift apart and the warp runs them one after the other.  (The whole traceback is 3.2 of the
 	// 20.0 ms of al_kernel: tile prefetch 1.7, walkers 1.5.)
 	int i = run ? tlen - 1 : -1, j = run ? qlen - 1 : -1, n = 0, ovf = 0;
-#ifdef KSW_ROWS_NOTB /* timing / traffic experiments only: skip the traceback (results are wrong) */
-	i = j = -1;
-#endif
 	{
 		uint32_t *tile = (uint32_t*)M.xvuy;
 		uint32_t *cig = M.cig; const int cig_cap = M.cig_cap;

@@ -2,7 +2,7 @@
 //
 // One context per GPU.  A context owns `n_streams` lanes; each lane has its stream, device copies of one batch,
 // the result pools, the kernel workspaces and pinned host buffers for the results.  idl_submit issues, on the
-// lane's stream: cudaMemcpyAsync H2D of the pinned batch -> assemble_kernel -> align_kernel (DP + glue) ->
+// lane's stream: cudaMemcpyAsync H2D of the pinned batch -> assemble_kernel -> align4_kernel (DP + glue) ->
 // kmer_kernel -> al_kernel -> D2H of the counters; idl_wait then copies back exactly the used prefix of every
 // result pool.  All kernels are persistent (grid sized from the SM count) and pull work from device-side queues,
 // so the host never needs the intermediate counts.  No CPU fallback exists.
@@ -21,10 +21,6 @@
 static_assert(sizeof(idl_region) == 48 && sizeof(idl_read) == 24, "batch records are part of the ABI");
 static_assert(sizeof(idl_region_result) == 16 && sizeof(idl_contig_result) == 24 && sizeof(idl_aln_result) == 72 && sizeof(idl_event_result) == 128,
               "result records are part of the ABI");
-
-#ifndef IDL_ALIGN_G_DEFAULT
-#define IDL_ALIGN_G_DEFAULT 4 /* threads per alignment of the banded call-site: 4 (align4_kernel) measured 10.1 ms on chr1 against 12.9 with 8 */
-#endif
 
 namespace {
 
@@ -92,8 +88,6 @@ struct idl_ctx {
 	uint64_t next_ticket = 1;
 	int asm_ctas = 0, dp_ctas = 0, ns = 0, nw = 0;
 	int cig_cap = 2048;
-	int align_g = 8;        // IDL_ALIGN_G=4: four threads per alignment in the banded call-site (align4_kernel)
-	bool band_regs = false; // IDL_BAND_REGS=1: the banded call-site keeps its band ring in registers (ksw2_band.cuh) instead of shared memory (measured slower, kept for the parity tests)
 	char err[512] = {0};
 };
 
@@ -107,8 +101,6 @@ int fail(idl_ctx *c, cudaError_t e, const char *what)
 #define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(ctx, e_, #call); } while (0)
 
 size_t round_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
-int next_pow2(int x) { int p = 1; while (p < x) p <<= 1; return p; }
 
 // persistent kernel-2 grids: as many CTAs as fit on the device at this shared-memory size, at most ctx->dp_ctas (the workspaces are sized for that)
 int dp_grid(const idl_ctx *ctx, const void *kernel, size_t smem, int threads = 256)
@@ -195,9 +187,6 @@ int idl_create(int device, const idl_params *p, idl_ctx **out)
 	const char *ea = getenv("IDL_ASM_CTAS_PER_SM"), *ed = getenv("IDL_DP_CTAS_PER_SM");
 	ctx->asm_ctas = ctx->n_sm * (ea && atoi(ea) > 0 ? atoi(ea) : ASM_CTAS); // CTAs of each assembler launch (8 regions per CTA in the warp variant)
 	ctx->dp_ctas = ctx->n_sm * (ed && atoi(ed) > 0 ? atoi(ed) : 4); // upper bound; every launch asks the occupancy calculator
-	{ const char *eb = getenv("IDL_BAND_REGS"); ctx->band_regs = eb && *eb == '1'; }
-	{ const char *eg = getenv("IDL_ALIGN_G"); ctx->align_g = eg && atoi(eg) == 8 ? 8 : (eg && atoi(eg) == 4 ? 4 : IDL_ALIGN_G_DEFAULT); }
-	{ const char *el = getenv("IDL_L2_FETCH"); if (el && atoi(el) > 0) cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(el)); } // experiments: 32 / 64 / 128
 	ctx->lanes.resize((size_t)p->n_streams);
 	{
 		// IDL_OVERLAP_KERNELS=1: the kernels of a batch run on its lane's stream and may share the SMs with another batch's
@@ -214,8 +203,6 @@ int idl_create(int device, const idl_params *p, idl_ctx **out)
 		for (auto &ev : L.ev_d2h) if (cudaEventCreate(&ev) != cudaSuccess) { idl_destroy(ctx); return IDL_E_CUDA; }
 	}
 	// opt in to large dynamic shared memory for the DP kernels
-	cudaFuncSetAttribute(align_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-	cudaFuncSetAttribute(align_band_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
 	cudaFuncSetAttribute(align4_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
 	cudaFuncSetAttribute(al_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
 	cudaFuncSetAttribute(al_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
@@ -373,12 +360,8 @@ int launch_chain(idl_ctx *ctx, Lane &L, bool record_start = false)
 	const size_t rowsA = (size_t)ksw_rows_bound(P.max_contig_len, (int)max_ref, P.a_bw); // the anti-diagonals an alignment can execute before its band runs out
 	const size_t rowsB = (size_t)max_trim + std::max<size_t>(max_ref, 1536);
 	const size_t pitchB = std::max<size_t>(ksw_pitch(ncolB), P.b_bw < 0 ? 32 * (size_t)ksw_rows_w(max_trim) : 0); // the row-owned variant stores 32 W bytes per diagonal
-	// the banded call-site runs the register-ring variant whenever its band fits (w <= 79: indelope's 50 does), G threads per alignment
-	const bool bandA = ctx->band_regs && P.a_bw >= 0 && ksw_ncol(P.max_contig_len, (int)max_ref, P.a_bw) <= KSW_BAND_MAX_NCOL;
 	const size_t p_capA = round_up(rowsA * ksw_pitch(ncolA) + 2 * KSW_PMAT_PAD + 64, 256), p_capB = round_up(rowsB * pitchB + 2 * KSW_PMAT_PAD + 64, 256);
-	const bool a4 = !bandA && ctx->align_g == 4;
-	const size_t groups_a = bandA ? (size_t)ctx->n_sm * KSW_BAND_CTAS * KSW_BAND_WARPS * (32 / KSW_BAND_G) : a4 ? (size_t)ctx->n_sm * KSW_A4_CTAS * KSW_A4_WARPS * 8
-	                                                                                                            : (size_t)ctx->dp_ctas * DP_WARPS * DP_NG, groups_b = (size_t)ctx->dp_ctas * DP_WARPS * DP_NG;
+	const size_t groups_a = (size_t)ctx->n_sm * KSW_A4_CTAS * KSW_A4_WARPS * 8 /* align4_kernel: eight alignments per warp */, groups_b = (size_t)ctx->dp_ctas * DP_WARPS * DP_NG;
 	const size_t n_groups = std::max(groups_a, groups_b);
 	const int seq_spill_cap = (int)round_up(ksw_seq_bytes(std::max(P.max_contig_len, max_trim), std::max((int)max_ref, P.max_contig_len)) + 32, 16);
 	CK(L.pmat.ensure(std::max(groups_a * p_capA, groups_b * p_capB)));
@@ -442,27 +425,19 @@ int launch_chain(idl_ctx *ctx, Lane &L, bool record_start = false)
 	g.seq_spill = (uint8_t*)L.seq_spill.p; g.seq_spill_cap = seq_spill_cap;
 	const size_t smem_limit = 200 * 1024;
 	if (b->n_regions > 0 && (P.stages & IDL_STAGE_ALIGN)) {
-		g.ring_cols = bandA ? 0 : ksw_ring_cols(ncolA); // the register-ring variant keeps only the reversed query (later the backtrack tile) in shared memory
-		const char *es = getenv("IDL_SEQ_STAGE"); // contigs up to this many bases stage their reversed copy in shared memory, longer ones in the global spill area
-		// (four threads per alignment: 448 bases keep a group at 1.5 KB, four CTAs of 32 alignments per SM -- 16 warps; at 1024 bases three CTAs
+		g.ring_cols = ksw_ring_cols(ncolA);
+		// contigs up to 448 bases stage their reversed copy in shared memory, longer ones in the global spill area
+		// (448 bases keep a group at 1.5 KB, four CTAs of 32 alignments per SM -- 16 warps; at 1024 bases three CTAs
 		// fit and the kernel ran 12.4 instead of 10.1 ms.  Five CTAs at 256 bases gave nothing more.)
-		const int stage = es && atoi(es) >= 64 ? atoi(es) : (a4 ? 448 : 1024);
-		g.seq_cap = (int)round_up(ksw_seq_bytes(std::min(P.max_contig_len, stage), (int)max_ref), 16) + (bandA ? 32 : 0); // + KswBandEz
-		const size_t smem = (size_t)(bandA ? KSW_BAND_WARPS * (32 / KSW_BAND_G) : a4 ? KSW_A4_WARPS * 8 : DP_WARPS * DP_NG) * ksw_group_smem(g.ring_cols, g.seq_cap);
+		const int stage = 448;
+		g.seq_cap = (int)round_up(ksw_seq_bytes(std::min(P.max_contig_len, stage), (int)max_ref), 16);
+		const size_t smem = (size_t)KSW_A4_WARPS * 8 * ksw_group_smem(g.ring_cols, g.seq_cap);
 		if (smem > smem_limit) return IDL_E_CAPACITY;
 		sort_scan_kernel<<<1, 1024, 0, cs>>>(sA);
 		sort_scatter_kernel<<<ctx->n_sm * 4, 256, 0, cs>>>(sA, &a.cnt->n_alns, 1u, L.cap_alns);
-		if (bandA) {
-			int nb = 0;
-			if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, (const void*)align_band_kernel, 32 * KSW_BAND_WARPS, smem) != cudaSuccess || nb < 1) nb = 1;
-			align_band_kernel<<<ctx->n_sm * std::min(nb, KSW_BAND_CTAS), 32 * KSW_BAND_WARPS, smem, cs>>>(g);
-		}
-		else if (a4) {
-			int nb = 0;
-			if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, (const void*)align4_kernel, 32 * KSW_A4_WARPS, smem) != cudaSuccess || nb < 1) nb = 1;
-			align4_kernel<<<ctx->n_sm * std::min(nb, KSW_A4_CTAS), 32 * KSW_A4_WARPS, smem, cs>>>(g);
-		}
-		else align_kernel<<<dp_grid(ctx, (const void*)align_kernel, smem), DP_THREADS, smem, cs>>>(g);
+		int nb = 0;
+		if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, (const void*)align4_kernel, 32 * KSW_A4_WARPS, smem) != cudaSuccess || nb < 1) nb = 1;
+		align4_kernel<<<ctx->n_sm * std::min(nb, KSW_A4_CTAS), 32 * KSW_A4_WARPS, smem, cs>>>(g);
 		CK(cudaGetLastError()); L.launches += 3;
 	}
 	CK(cudaEventRecord(L.ev[EV_ALN], cs));
@@ -721,13 +696,12 @@ struct KswBatchArgs {
 	KswParams kp; idl_ez *out; uint32_t *cigar; unsigned long long *cigar_off; unsigned cigar_cap;
 	unsigned *next; unsigned *cig_used;
 	uint8_t *pmat; size_t p_cap; uint32_t *cig_scratch; int cig_cap; int ring_cols, seq_cap;
-	int no_rows; // IDL_KSW2_COLUMNS=1: keep unbanded alignments on the column-owned variant (tests compare the two)
+	int no_rows; // IDL_KSW2_COLUMNS=1: run every alignment on the column-owned ksw2_group<8> (tests compare it with the default variants)
 };
 
-// MODE 0: banded, shared-memory rings (any w >= 0); 1: unbanded (row-owned variant for reads of up to 160 bases, else the rings);
-// 2: banded, the ring in registers (rounded bands of up to 96 lanes), G threads per alignment
+// MODE 0: banded, shared-memory rings (any w >= 0), G threads per alignment; 1: unbanded (row-owned variant for reads of up to 160 bases, else the rings)
 template <int MODE, int G>
-__global__ void __launch_bounds__(MODE == 2 ? 32 * KSW_BAND_WARPS : (G == 4 ? 32 * KSW_A4_WARPS : DP_THREADS), MODE == 1 ? 2 : (MODE == 2 ? KSW_BAND_CTAS : (G == 4 ? KSW_A4_CTAS : 3))) ksw2_batch_kernel(KswBatchArgs a) // unbanded: 8 warps x 2 CTAs at 122 registers (uniform shapes: 774 GCUPS at 150x700 against 745 with al_kernel's 5 x 4)
+__global__ void __launch_bounds__(G == 4 ? 32 * KSW_A4_WARPS : DP_THREADS, MODE == 1 ? 2 : (G == 4 ? KSW_A4_CTAS : 3)) ksw2_batch_kernel(KswBatchArgs a) // unbanded: 8 warps x 2 CTAs at 122 registers (uniform shapes: 774 GCUPS at 150x700 against 745 with al_kernel's 5 x 4)
 {
 	extern __shared__ __align__(16) unsigned char smem_raw[];
 	constexpr int NG = 32 / G;
@@ -750,8 +724,7 @@ __global__ void __launch_bounds__(MODE == 2 ? 32 * KSW_BAND_WARPS : (G == 4 ? 32
 		KswQuery kq; kq.codes = a.query + (valid ? a.q_off[i] : 0); kq.seq2 = nullptr; kq.seqn = nullptr; kq.base = 0;
 		KswOut o;
 		const uint8_t *tq = a.target + (valid ? a.t_off[i] : 0);
-		if constexpr (MODE == 2) ksw2_band<G, true>(valid, qlen, kq, tlen, tq, a.kp, M, o);
-		else if constexpr (G == 4) ksw2_group<4, true, false>(valid, qlen, kq, tlen, tq, a.kp, M, o);
+		if constexpr (G == 4) ksw2_group<4, true, false>(valid, qlen, kq, tlen, tq, a.kp, M, o);
 		else {
 			const int rw = MODE == 1 && !a.no_rows ? ksw_rows_pick(valid, qlen, tlen, a.kp, M) : 0;
 			if (rw == 5) ksw2_rows<5, true>(valid, qlen, kq, tlen, tq, a.kp, M, o);
@@ -796,20 +769,15 @@ extern "C" int idl_ksw2_batch(idl_ctx *ctx, size_t n, const uint8_t *query, cons
 	KswBatchArgs a; memset(&a, 0, sizeof a);
 	a.n = (unsigned)n; a.kp = ksw_make_params(match, mismatch, gapo, gape, w, zdrop);
 	{ const char *e = getenv("IDL_KSW2_COLUMNS"); a.no_rows = e && *e == '1'; }
-	// IDL_BAND_REGS=1 and 0 <= w with a rounded band of up to 96 lanes: the register-ring variant of the banded call-site (tests compare the two)
-	const char *ebr = getenv("IDL_BAND_REGS");
-	const int mode = w < 0 ? 1 : (max_ncol <= KSW_BAND_MAX_NCOL && ebr && *ebr == '1' ? 2 : 0);
-	const char *eg4 = getenv("IDL_ALIGN_G");
-	const bool g4 = mode == 0 && (eg4 ? atoi(eg4) == 4 : ctx->align_g == 4); // the banded call-site with four threads per alignment
-	const int ng = mode == 2 ? 32 / KSW_BAND_G : (g4 ? 8 : DP_NG);
-	a.ring_cols = mode == 2 ? 0 : ksw_ring_cols(max_ncol);
+	const bool g4 = w >= 0 && !a.no_rows; // the banded call-site with four threads per alignment, as align4_kernel
+	const int ng = g4 ? 8 : DP_NG;
+	a.ring_cols = ksw_ring_cols(max_ncol);
 	a.p_cap = round_up(max_p + 2 * KSW_PMAT_PAD + 64, 256); a.cig_cap = max_q + max_t + 8; a.cigar_cap = (unsigned)cigar_cap;
-	a.seq_cap = (int)round_up(ksw_seq_bytes(max_q, max_t), 16) + (mode == 2 ? 32 : 0); // + KswBandEz
-	const int wpc = mode == 2 ? KSW_BAND_WARPS : (g4 ? KSW_A4_WARPS : DP_WARPS); // warps per CTA
+	a.seq_cap = (int)round_up(ksw_seq_bytes(max_q, max_t), 16);
+	const int wpc = g4 ? KSW_A4_WARPS : DP_WARPS; // warps per CTA
 	const size_t smem = (size_t)wpc * ng * ksw_group_smem(a.ring_cols, a.seq_cap);
 	if (smem > 200 * 1024) return IDL_E_CAPACITY;
-	const void *kfn = mode == 1 ? (const void*)ksw2_batch_kernel<1, 8> : mode == 2 ? (const void*)ksw2_batch_kernel<2, KSW_BAND_G> : g4 ? (const void*)ksw2_batch_kernel<0, 4>
-	                                                                                                                                  : (const void*)ksw2_batch_kernel<0, 8>;
+	const void *kfn = w < 0 ? (const void*)ksw2_batch_kernel<1, 8> : g4 ? (const void*)ksw2_batch_kernel<0, 4> : (const void*)ksw2_batch_kernel<0, 8>;
 	cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
 	const size_t per_cta = (size_t)wpc * ng;
 	const int ctas = (int)std::min<size_t>((n + per_cta - 1) / per_cta, (size_t)dp_grid(ctx, kfn, smem, 32 * wpc));
@@ -831,8 +799,7 @@ extern "C" int idl_ksw2_batch(idl_ctx *ctx, size_t n, const uint8_t *query, cons
 		a.next = (unsigned*)dmisc.p; a.cig_used = (unsigned*)dmisc.p + 1; a.pmat = (uint8_t*)dp.p; a.cig_scratch = (uint32_t*)dscr.p;
 		CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
 		CK(cudaEventRecord(e0, st));
-		if (mode == 1) ksw2_batch_kernel<1, 8><<<ctas, 32 * wpc, smem, st>>>(a);
-		else if (mode == 2) ksw2_batch_kernel<2, KSW_BAND_G><<<ctas, 32 * wpc, smem, st>>>(a);
+		if (w < 0) ksw2_batch_kernel<1, 8><<<ctas, 32 * wpc, smem, st>>>(a);
 		else if (g4) ksw2_batch_kernel<0, 4><<<ctas, 32 * wpc, smem, st>>>(a);
 		else ksw2_batch_kernel<0, 8><<<ctas, DP_THREADS, smem, st>>>(a);
 		CK(cudaGetLastError());

@@ -176,40 +176,12 @@ def test_unbanded_other_scoring_parameters(ctx, match, mismatch, gapo, gape):
     assert bad == [], bad[:3]
 
 
-def test_register_ring_equals_shared_memory_ring(ctx, monkeypatch):
-    """IDL_BAND_REGS=1 runs the banded call-site with the band ring in registers (ksw2_band.cuh) for rounded bands of up to 96
-    lanes instead of the shared-memory rings (ksw2.cuh, the default: it measured faster): same records and CIGARs, for several band
-    widths incl. the widest one the register ring serves (w = 79) and one it does not (w = 80: both runs take the rings)"""
-    rng = np.random.default_rng(29)
-    for w, z in [(50, 400), (79, 400), (80, 400), (1, 100), (17, -1), (33, 60)]:
-        qs, ts = [], []
-        for _ in range(250):
-            ql = int(rng.integers(1, 700)); base = rng.integers(0, 4, ql + 400).astype(np.uint8)
-            q = base[:ql].copy(); t = base[:max(1, ql + int(rng.integers(-60, 260)))].copy()
-            pos = int(rng.integers(0, max(1, ql - 1))); L = int(rng.integers(1, 90))
-            q = np.concatenate([q[:pos], rng.integers(0, 4, L).astype(np.uint8), q[pos:]]) if rng.random() < 0.5 else np.concatenate([q[:pos], q[min(len(q) - 1, pos + L):]])
-            m = rng.random(len(q)) < 0.02; q[m] = rng.integers(0, 5, int(m.sum()))
-            qs.append(q); ts.append(t)
-        a = ctx.ksw2_batch(qs, ts, gapo=4, gape=1, w=w, zdrop=z)
-        monkeypatch.setenv("IDL_BAND_REGS", "1")
-        b = ctx.ksw2_batch(qs, ts, gapo=4, gape=1, w=w, zdrop=z)
-        monkeypatch.delenv("IDL_BAND_REGS")
-        assert a[0] == b[0] and a[1] == b[1] and a[2] == b[2], (w, z)
-    # ... and against the oracle directly, production parameters
-    monkeypatch.setenv("IDL_BAND_REGS", "1")
-    pairs = []
-    for _ in range(600):
-        q, t, go, w, z = random_pair(rng)
-        if w >= 0:
-            pairs.append((q, t, 4, 50, 400))
-    assert check(ctx, pairs, "ref" if orc.have_ref() else "lane") == []
-
-
 def test_four_threads_per_alignment_equals_eight(ctx, monkeypatch):
-    """IDL_ALIGN_G=4 runs the banded call-site's shared-memory rings with four threads per alignment (eight alignments per warp in
-    lockstep) instead of eight: same records and CIGARs for several band widths, and the oracle on production parameters"""
+    """the banded call-site runs its shared-memory rings with four threads per alignment (eight alignments per warp in lockstep);
+    IDL_KSW2_COLUMNS=1 runs it on the eight-thread ring group that call-site B falls back to: same records and CIGARs for ten band
+    widths, and the oracle on production parameters"""
     rng = np.random.default_rng(31)
-    for w, z in [(50, 400), (100, 400), (7, 100), (33, -1), (200, 50)]:
+    for w, z in [(50, 400), (100, 400), (7, 100), (33, -1), (200, 50), (79, 400), (80, 400), (1, 100), (17, -1), (33, 60)]:
         qs, ts = [], []
         for _ in range(250):
             ql = int(rng.integers(1, 700)); base = rng.integers(0, 4, ql + 400).astype(np.uint8)
@@ -218,12 +190,11 @@ def test_four_threads_per_alignment_equals_eight(ctx, monkeypatch):
             q = np.concatenate([q[:pos], rng.integers(0, 4, L).astype(np.uint8), q[pos:]]) if rng.random() < 0.5 else np.concatenate([q[:pos], q[min(len(q) - 1, pos + L):]])
             m = rng.random(len(q)) < 0.02; q[m] = rng.integers(0, 5, int(m.sum()))
             qs.append(q); ts.append(t)
-        monkeypatch.setenv("IDL_ALIGN_G", "8")
         a = ctx.ksw2_batch(qs, ts, gapo=4, gape=1, w=w, zdrop=z)
-        monkeypatch.setenv("IDL_ALIGN_G", "4")
+        monkeypatch.setenv("IDL_KSW2_COLUMNS", "1")
         b = ctx.ksw2_batch(qs, ts, gapo=4, gape=1, w=w, zdrop=z)
+        monkeypatch.delenv("IDL_KSW2_COLUMNS")
         assert a[0] == b[0] and a[1] == b[1] and a[2] == b[2], (w, z)
-    monkeypatch.setenv("IDL_ALIGN_G", "4")
     pairs = []
     for _ in range(900):
         q, t, go, w, z = random_pair(rng)

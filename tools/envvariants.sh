@@ -7,7 +7,7 @@ for V in "$@"; do
 import json, sys
 try:
     d = json.load(open("gpurun_out/var.json")); k = d["kernel_ms"]
-    print("%-60s step %.2f ms  asm %.2f  align %.2f  al %.2f  kmer %.3f" % (sys.argv[1], d["ms_per_step"], k["assemble_kernel"], k["align_kernel"], k["al_kernel"], k["kmer_kernel"]))
+    print("%-60s step %.2f ms  asm %.2f  align %.2f  al %.2f  kmer %.3f" % (sys.argv[1], d["ms_per_step"], k["assemble_kernel"], k["align4_kernel"], k["al_kernel"], k["kmer_kernel"]))
 except Exception as e:
     print(sys.argv[1], "bench failed", e)
 PY

@@ -1,5 +1,5 @@
 #!/bin/bash
-# DRAM traffic of one kernel at the full default workload under environment settings (run under gpurun): tools/traffic_env.sh al_kernel "" "IDL_L2_FETCH=32"
+# DRAM traffic of one kernel at the full default workload under environment settings (run on the GPU machine): tools/traffic_env.sh al_kernel "" "IDL_DP_CTAS_PER_SM=3"
 K=$1; shift
 mkdir -p gpurun_out
 M=dram__bytes_read.sum,dram__bytes_write.sum,gpu__time_duration.sum,smsp__thread_inst_executed.sum,lts__t_sectors_srcunit_tex_op_read.sum,lts__t_sectors_srcunit_tex_op_write.sum

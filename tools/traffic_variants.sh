@@ -1,6 +1,6 @@
 #!/bin/bash
 # DRAM traffic / instruction counts of one kernel of the chain at the full default workload, for compile-time variants (run under gpurun):
-#   tools/traffic_variants.sh al_kernel "" "-DKSW_PSTORE_MODE=0" ...
+#   tools/traffic_variants.sh al_kernel "" "-DKSW_UNB_WARPS=8 -DKSW_UNB_CTAS=2" ...
 K=$1; shift
 mkdir -p gpurun_out
 M=dram__bytes_read.sum,dram__bytes_write.sum,gpu__time_duration.sum,smsp__thread_inst_executed.sum,lts__t_sectors_srcunit_tex_op_read.sum,lts__t_sectors_srcunit_tex_op_write.sum,lts__t_sectors_srcunit_tex_op_read_lookup_miss.sum,lts__t_sectors_srcunit_tex_op_write_lookup_miss.sum
