@@ -33,7 +33,8 @@ typedef enum {
 	IDL_E_CUDA = -2,        /* a CUDA call failed; idl_last_cuda_error() has the text */
 	IDL_E_ARG = -3,
 	IDL_E_NOMEM = -4,
-	IDL_E_CAPACITY = -5,    /* batch exceeds what idl_batch_alloc / idl_create sized */
+	IDL_E_CAPACITY = -5,    /* batch exceeds what idl_batch_alloc / idl_create sized, or its longest read / window needs more kernel-2
+	                           workspace or shared memory than one CTA may have (DESIGN.md 7) */
 	IDL_E_TICKET = -6,
 	IDL_E_BUSY = -7,
 	IDL_E_FORMAT = -8       /* idl_bam_open: not a BGZF / BAM file, corrupt member, unsorted records; the call's message has the detail */

@@ -88,6 +88,7 @@ struct idl_ctx {
 	uint64_t next_ticket = 1;
 	int asm_ctas = 0, dp_ctas = 0, ns = 0, nw = 0;
 	int cig_cap = 2048;
+	size_t ws_budget = 0; // bytes of kernel-2 workspace (backtrack matrices, CIGAR scratch, sequence spill) one lane may hold
 	char err[512] = {0};
 };
 
@@ -102,13 +103,39 @@ int fail(idl_ctx *c, cudaError_t e, const char *what)
 
 size_t round_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
-// persistent kernel-2 grids: as many CTAs as fit on the device at this shared-memory size, at most ctx->dp_ctas (the workspaces are sized for that)
+// persistent kernel-2 grids: as many CTAs as fit on the device at this shared-memory size, at most ctx->dp_ctas (launch_chain caps it further
+// to the CTAs whose workspaces it allocated)
 int dp_grid(const idl_ctx *ctx, const void *kernel, size_t smem, int threads = 256)
 {
 	int nb = 0;
 	if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, threads, smem) != cudaSuccess || nb < 1) nb = 1;
-	// the per-group workspaces are sized for dp_ctas CTAs of DP_WARPS warps
 	return std::min(ctx->dp_ctas * 256 / threads, ctx->n_sm * nb);
+}
+
+// Shared memory of one kernel-2 CTA at call-site A (align4_kernel) and B (al_kernel).  launch_chain launches with these sizes, and idl_create
+// refuses parameters whose worst case (the longest window any batch can have) does not fit DP_SMEM_LIMIT, so that no batch fails for it.
+constexpr size_t DP_SMEM_LIMIT = 200 * 1024;
+struct DpSmem { int ring_cols, seq_cap; size_t bytes; };
+DpSmem smem_site_a(const idl_params &P, int max_ref)
+{
+	// contigs up to 448 bases stage their reversed copy in shared memory, longer ones in the global spill area
+	// (448 bases keep a group at 1.5 KB, four CTAs of 32 alignments per SM -- 16 warps; at 1024 bases three CTAs
+	// fit and the kernel ran 12.4 instead of 10.1 ms.  Five CTAs at 256 bases gave nothing more.)
+	const int stage = 448;
+	DpSmem s;
+	s.ring_cols = ksw_ring_cols(ksw_ncol(P.max_contig_len, max_ref, P.a_bw));
+	s.seq_cap = (int)round_up(ksw_seq_bytes(std::min(P.max_contig_len, stage), max_ref), 16);
+	s.bytes = (size_t)KSW_A4_WARPS * 8 * ksw_group_smem(s.ring_cols, s.seq_cap);
+	return s;
+}
+DpSmem smem_site_b(const idl_params &P, int max_trim, int max_ref)
+{
+	DpSmem s;
+	// unbanded: room for the row-owned variant's target staging whatever the reads' length
+	s.ring_cols = std::max(ksw_ring_cols(ksw_ncol(max_trim, std::max(max_ref, P.max_contig_len), P.b_bw)), P.b_bw < 0 ? 256 : 0);
+	s.seq_cap = (int)round_up(ksw_seq_bytes(max_trim, max_ref), 16);
+	s.bytes = (size_t)(P.b_bw < 0 ? KSW_UNB_WARPS : DP_WARPS) * DP_NG * ksw_group_smem(s.ring_cols, s.seq_cap);
+	return s;
 }
 
 } // namespace
@@ -171,6 +198,9 @@ int idl_create(int device, const idl_params *p, idl_ctx **out)
 	if (p->max_contig_len < 64 || p->max_contig_len % 64 || p->max_contig_len > 32768 || p->max_reads_per_region < 1 || p->max_reads_per_region > 4000 ||
 	    p->max_read_len < 1 || p->max_read_len > 4096 || p->n_streams < 1 || p->n_streams > 8 || p->max_events < 1 || p->max_events > IDL_MAX_EVENTS)
 		return IDL_E_ARG;
+	// the query of call-site B (a trimmed read) is staged in shared memory: with the unbanded default that holds reads of up to 960 bases
+	// (DESIGN.md 7).  Longer max_read_len is refused here, so that a longer read drops its region (IDL_RS_READ_TOO_LONG) instead of its batch.
+	if (smem_site_a(*p, 1 << 20).bytes > DP_SMEM_LIMIT || smem_site_b(*p, p->max_read_len, 1 << 20).bytes > DP_SMEM_LIMIT) return IDL_E_ARG;
 	int n = 0;
 	if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) return IDL_E_NO_DEVICE;
 	if (device < 0 || device >= n) return IDL_E_ARG;
@@ -180,7 +210,15 @@ int idl_create(int device, const idl_params *p, idl_ctx **out)
 	cudaError_t e = cudaSetDevice(device);
 	if (e != cudaSuccess) { delete ctx; return IDL_E_CUDA; }
 	cudaDeviceProp prop;
-	if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) ctx->n_sm = prop.multiProcessorCount;
+	size_t total_mem = 0;
+	if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) { delete ctx; return IDL_E_CUDA; }
+	ctx->n_sm = prop.multiProcessorCount; total_mem = prop.totalGlobalMem;
+	{
+		// kernel-2 workspace per lane: a quarter of the device shared by the lanes, at most 16 GiB (DESIGN.md 7); IDL_WS_BUDGET_MB overrides it
+		const char *eb = getenv("IDL_WS_BUDGET_MB");
+		ctx->ws_budget = std::min<size_t>(16ull << 30, total_mem / (4 * (size_t)p->n_streams));
+		if (eb && atoll(eb) > 0) ctx->ws_budget = (size_t)atoll(eb) << 20;
+	}
 	ctx->ns = p->max_reads_per_region + 2;
 	ctx->nw = p->max_contig_len / 32 + 2;
 	// persistent grids: CTAs per SM (tunable for experiments through the environment)
@@ -343,10 +381,13 @@ int launch_chain(idl_ctx *ctx, Lane &L, bool record_start = false)
 	// workspaces
 	const size_t n_small = L.n_small;
 	const size_t n_big = b->n_regions - n_small;
-	const int big_ctas = (int)std::min<size_t>(n_big, (size_t)ctx->asm_ctas), small_ctas = (int)std::min<size_t>((n_small + 7) / 8, (size_t)ctx->asm_ctas);
-	// the assembler addresses its arenas with 32-bit element offsets
-	if ((size_t)big_ctas * ctx->ns * std::max<size_t>(3 * (size_t)ctx->nw, (size_t)P.max_contig_len) >= 0xffffffffULL ||
-	    (size_t)small_ctas * 8 * ASM_SMALL_NS * std::max<size_t>(3 * (size_t)ctx->nw, (size_t)P.max_contig_len) >= 0xffffffffULL) return IDL_E_CAPACITY;
+	// the assembler addresses its arenas with 32-bit element offsets: at large max_reads_per_region / max_contig_len fewer CTAs are
+	// launched (they pull regions from an atomic queue, so any grid computes the same); only an arena of one CTA that does not fit fails
+	const size_t per_big = (size_t)ctx->ns * std::max<size_t>(3 * (size_t)ctx->nw, (size_t)P.max_contig_len);
+	const size_t per_small = (size_t)8 * ASM_SMALL_NS * std::max<size_t>(3 * (size_t)ctx->nw, (size_t)P.max_contig_len);
+	if (per_big >= 0xffffffffULL || per_small >= 0xffffffffULL) return IDL_E_CAPACITY;
+	const int big_ctas = (int)std::min<size_t>({n_big, (size_t)ctx->asm_ctas, (size_t)0xfffffffeULL / per_big});
+	const int small_ctas = (int)std::min<size_t>({(n_small + 7) / 8, (size_t)ctx->asm_ctas, (size_t)0xfffffffeULL / per_small});
 	if (n_big) {
 		CK(L.planes.ensure((size_t)big_ctas * ctx->ns * 3 * ctx->nw * 4));
 		CK(L.sup.ensure((size_t)big_ctas * ctx->ns * P.max_contig_len * 2));
@@ -361,9 +402,16 @@ int launch_chain(idl_ctx *ctx, Lane &L, bool record_start = false)
 	const size_t rowsB = (size_t)max_trim + std::max<size_t>(max_ref, 1536);
 	const size_t pitchB = std::max<size_t>(ksw_pitch(ncolB), P.b_bw < 0 ? 32 * (size_t)ksw_rows_w(max_trim) : 0); // the row-owned variant stores 32 W bytes per diagonal
 	const size_t p_capA = round_up(rowsA * ksw_pitch(ncolA) + 2 * KSW_PMAT_PAD + 64, 256), p_capB = round_up(rowsB * pitchB + 2 * KSW_PMAT_PAD + 64, 256);
-	const size_t groups_a = (size_t)ctx->n_sm * KSW_A4_CTAS * KSW_A4_WARPS * 8 /* align4_kernel: eight alignments per warp */, groups_b = (size_t)ctx->dp_ctas * DP_WARPS * DP_NG;
-	const size_t n_groups = std::max(groups_a, groups_b);
 	const int seq_spill_cap = (int)round_up(ksw_seq_bytes(std::max(P.max_contig_len, max_trim), std::max((int)max_ref, P.max_contig_len)) + 32, 16);
+	// Every group of a kernel-2 grid owns a backtrack matrix, CIGAR scratch and a spill area, addressed by its index in the launched grid.
+	// Both grids are persistent and take their tasks from atomic counters, so fewer groups compute the same records: each grid is capped
+	// at the CTAs its tasks can keep busy and at the CTAs whose workspaces fit the lane's budget, and the workspaces are sized for that cap.
+	const size_t gpc_a = (size_t)KSW_A4_WARPS * 8 /* align4_kernel: eight alignments per warp */, warps_b = P.b_bw < 0 ? KSW_UNB_WARPS : DP_WARPS, gpc_b = warps_b * DP_NG;
+	const size_t ws_fixed = (size_t)ctx->cig_cap * 4 + (size_t)seq_spill_cap;
+	const size_t ctas_a = std::min<size_t>({(size_t)ctx->n_sm * KSW_A4_CTAS, ((size_t)L.cap_alns + gpc_a - 1) / gpc_a, ctx->ws_budget / (gpc_a * (p_capA + ws_fixed))});
+	const size_t ctas_b = std::min<size_t>({(size_t)ctx->dp_ctas * DP_WARPS / warps_b, (2 * (size_t)L.cap_items + gpc_b - 1) / gpc_b, ctx->ws_budget / (gpc_b * (p_capB + ws_fixed))});
+	if (ctas_a < 1 || ctas_b < 1) return IDL_E_CAPACITY; // the workspaces of one CTA exceed the budget: reads or windows too long for this device
+	const size_t groups_a = ctas_a * gpc_a, groups_b = ctas_b * gpc_b, n_groups = std::max(groups_a, groups_b);
 	CK(L.pmat.ensure(std::max(groups_a * p_capA, groups_b * p_capB)));
 	CK(L.cig_scratch.ensure(n_groups * (size_t)ctx->cig_cap * 4));
 	CK(L.seq_spill.ensure(n_groups * (size_t)seq_spill_cap));
@@ -423,21 +471,16 @@ int launch_chain(idl_ctx *ctx, Lane &L, bool record_start = false)
 	g.kpB = ksw_make_params(P.match, P.mismatch, P.b_gapo, P.b_gape, P.b_bw, P.b_zdrop);
 	g.pmat = (uint8_t*)L.pmat.p; g.p_cap = p_capA; g.cig_scratch = (uint32_t*)L.cig_scratch.p; g.cig_cap = ctx->cig_cap;
 	g.seq_spill = (uint8_t*)L.seq_spill.p; g.seq_spill_cap = seq_spill_cap;
-	const size_t smem_limit = 200 * 1024;
 	if (b->n_regions > 0 && (P.stages & IDL_STAGE_ALIGN)) {
-		g.ring_cols = ksw_ring_cols(ncolA);
-		// contigs up to 448 bases stage their reversed copy in shared memory, longer ones in the global spill area
-		// (448 bases keep a group at 1.5 KB, four CTAs of 32 alignments per SM -- 16 warps; at 1024 bases three CTAs
-		// fit and the kernel ran 12.4 instead of 10.1 ms.  Five CTAs at 256 bases gave nothing more.)
-		const int stage = 448;
-		g.seq_cap = (int)round_up(ksw_seq_bytes(std::min(P.max_contig_len, stage), (int)max_ref), 16);
-		const size_t smem = (size_t)KSW_A4_WARPS * 8 * ksw_group_smem(g.ring_cols, g.seq_cap);
-		if (smem > smem_limit) return IDL_E_CAPACITY;
+		const DpSmem sm = smem_site_a(P, (int)max_ref);
+		g.ring_cols = sm.ring_cols; g.seq_cap = sm.seq_cap;
+		const size_t smem = sm.bytes;
+		if (smem > DP_SMEM_LIMIT) return IDL_E_CAPACITY; // idl_create's check makes this unreachable
 		sort_scan_kernel<<<1, 1024, 0, cs>>>(sA);
 		sort_scatter_kernel<<<ctx->n_sm * 4, 256, 0, cs>>>(sA, &a.cnt->n_alns, 1u, L.cap_alns);
 		int nb = 0;
 		if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, (const void*)align4_kernel, 32 * KSW_A4_WARPS, smem) != cudaSuccess || nb < 1) nb = 1;
-		align4_kernel<<<ctx->n_sm * std::min(nb, KSW_A4_CTAS), 32 * KSW_A4_WARPS, smem, cs>>>(g);
+		align4_kernel<<<(int)std::min((size_t)ctx->n_sm * std::min(nb, KSW_A4_CTAS), ctas_a), 32 * KSW_A4_WARPS, smem, cs>>>(g);
 		CK(cudaGetLastError()); L.launches += 3;
 	}
 	CK(cudaEventRecord(L.ev[EV_ALN], cs));
@@ -446,16 +489,16 @@ int launch_chain(idl_ctx *ctx, Lane &L, bool record_start = false)
 		kmer_kernel<<<ctx->n_sm * 8, KMER_THREADS, 0, cs>>>(g);
 		CK(cudaGetLastError()); L.launches++;
 		CK(cudaEventRecord(L.ev[EV_KMER], cs));
-		g.ring_cols = std::max(ksw_ring_cols(ncolB), P.b_bw < 0 ? 256 : 0); // unbanded: room for the row-owned variant's target staging whatever the reads' length
-		g.seq_cap = (int)round_up(ksw_seq_bytes(max_trim, (int)max_ref), 16);
+		const DpSmem sm = smem_site_b(P, max_trim, (int)max_ref);
+		g.ring_cols = sm.ring_cols; g.seq_cap = sm.seq_cap;
 		const int al_warps = P.b_bw < 0 ? KSW_UNB_WARPS : DP_WARPS;
-		const size_t smem = (size_t)al_warps * DP_NG * ksw_group_smem(g.ring_cols, g.seq_cap);
-		if (smem > smem_limit) return IDL_E_CAPACITY;
+		const size_t smem = sm.bytes;
+		if (smem > DP_SMEM_LIMIT) return IDL_E_CAPACITY; // idl_create's check makes this unreachable
 		al_prep_kernel<<<ctx->n_sm * 8, 256, 0, cs>>>(g);
 		sort_scan_kernel<<<1, 1024, 0, cs>>>(sB);
 		sort_scatter_kernel<<<ctx->n_sm * 4, 256, 0, cs>>>(sB, &a.cnt->n_al_items, 2u, 2 * L.cap_items);
-		if (P.b_bw < 0) al_kernel<true><<<dp_grid(ctx, (const void*)al_kernel<true>, smem, 32 * al_warps), 32 * al_warps, smem, cs>>>(g); // unbanded (the reference's setting)
-		else al_kernel<false><<<dp_grid(ctx, (const void*)al_kernel<false>, smem), DP_THREADS, smem, cs>>>(g);
+		if (P.b_bw < 0) al_kernel<true><<<std::min(dp_grid(ctx, (const void*)al_kernel<true>, smem, 32 * al_warps), (int)ctas_b), 32 * al_warps, smem, cs>>>(g); // unbanded (the reference's setting)
+		else al_kernel<false><<<std::min(dp_grid(ctx, (const void*)al_kernel<false>, smem), (int)ctas_b), DP_THREADS, smem, cs>>>(g);
 		al_vote_kernel<<<ctx->n_sm * 4, 256, 0, cs>>>(g);
 		CK(cudaGetLastError()); L.launches += 5;
 	} else CK(cudaEventRecord(L.ev[EV_KMER], cs));

@@ -159,10 +159,17 @@ CP make_contig(const std::string &dna, int64_t start, uint32_t support = 1)
 	return o;
 }
 
+// the capacity limits the device enforces per region (dump bit 64): the longest contig reached at any point of assemble + combine
+// (a trimmed read or the product of a merge, against idl_params.max_contig_len) and the most voting sites of one merge (IDL_MAX_CORRECTIONS)
+struct Limits { int64_t max_len = 0, max_corr = 0; };
+thread_local Limits *g_limits = nullptr;
+
 // :156-222
 void insert_contig(Contig &t, Contig &q, const Match &m)
 {
 	if (!m.aligned()) return;
+	struct Track { Contig &t; ~Track() { if (g_limits) g_limits->max_len = std::max(g_limits->max_len, t.len()); } } track{t};
+	if (g_limits) g_limits->max_corr = std::max(g_limits->max_corr, (int64_t)m.corrections.size());
 	std::set<int64_t> dont_overwrite;
 	for (const Corr &c : m.corrections) {
 		if (c.qbest) { t.seq[c.toff] = q.seq[c.qoff]; t.sup[c.toff] = q.sup[c.qoff]; }
@@ -516,6 +523,7 @@ std::vector<CP> assemble(const Roi &r, int64_t *n_contigs, Counters *cn, int min
 		if (skippable(read)) continue;
 		int32_t tl; int32_t o = trim_read(read.qual, read.len, &tl);
 		std::string read_seq = tl > 0 ? read.seq.substr(o, tl) : std::string();
+		if (g_limits) g_limits->max_len = std::max(g_limits->max_len, (int64_t)read_seq.size());
 		CP qc = make_contig(read_seq, read.start + o);
 		list_insert(contigs, qc, (int64_t)(min_overlap_pct * (double)read_seq.size()), 0, allowable_mismatch, cn);
 	}
@@ -546,8 +554,12 @@ void callsemble(const Roi &r, const Fai &fai, const std::string &chrom, const or
 	Counters &cn = out.cn;
 	std::string &d = out.dump;
 	int64_t n_contigs = 0;
+	Limits lim;
+	g_limits = &lim;
 	std::vector<CP> contigs = assemble(r, &n_contigs, &cn);
+	g_limits = nullptr;
 	cn.contigs_pre += n_contigs; cn.contigs_post += (int64_t)contigs.size();
+	if (P.dump_level & 64) d += "L\t" + std::to_string(r.ordinal) + "\tmax_len=" + std::to_string(lim.max_len) + "\tmax_corr=" + std::to_string(lim.max_corr) + "\n";
 	if (P.dump_level & 1) {
 		d += "R\t" + std::to_string(r.ordinal) + "\tpre=" + std::to_string(n_contigs) + "\tn=" + std::to_string(contigs.size()) + "\n";
 		for (size_t ci = 0; ci < contigs.size(); ++ci) dump_contig(d, r.ordinal, ci, *contigs[ci], (P.dump_level & 2) != 0);

@@ -45,7 +45,7 @@ typedef struct {
 	int32_t min_ctg_len;    /* -c, :569 */
 	int32_t min_event_len;  /* -e, :570 */
 	int32_t use_ref_ksw2;   /* 1: run DPs through oracle/_ref/libksw2_ref.so (must be loaded first) */
-	int32_t dump_level;     /* bit0 R/C lines, bit1 supports in C lines, bit2 A lines, bit3 E lines, bit4 V lines, bit5 no dedup */
+	int32_t dump_level;     /* bit0 R/C lines, bit1 supports in C lines, bit2 A lines, bit3 E lines, bit4 V lines, bit5 no dedup, bit6 L lines (capacity limits per region; test only) */
 	int32_t n_threads;      /* regions are independent; >1 only parallelises across regions */
 } orc_params_t;
 

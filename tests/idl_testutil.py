@@ -384,3 +384,159 @@ def parse_bam(data):
                bases=np.concatenate(bases) if bases else np.zeros(0, np.uint8), quals=np.concatenate(quals) if quals else np.zeros(0, np.uint8),
                cigar=np.array(cigar, np.uint32))
     return text, refs, out, n_unplaced
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# Capacity limits: the oracle's per-region L lines (dump bit 64), region subsets, and directed regions built to sit exactly on a limit
+# ---------------------------------------------------------------------------------------------------------------
+DUMP_LIMITS = 64  # oracle only: "L <region> max_len=<longest contig of assemble + combine> max_corr=<most voting sites of one merge>"
+
+
+def limits(odump):
+    """{region ordinal: (longest contig, most voting sites)} from an oracle dump made with DUMP_LIMITS"""
+    out = {}
+    for l in odump.splitlines():
+        if l.startswith("L\t"):
+            f = l.split("\t")
+            out[int(f[1])] = (int(f[2].split("=")[1]), int(f[3].split("=")[1]))
+    return out
+
+
+def by_region(dump, types="RCAE"):
+    """{region ordinal: [lines]} of the per-region record types"""
+    out = {}
+    for l in dump.splitlines():
+        if l[:1] in types:
+            out.setdefault(int(l.split("\t")[1]), []).append(l)
+    return out
+
+
+def region_subset(arrays, keep):
+    """the same reads and chromosomes with only the regions whose index is in `keep` (in order)"""
+    keep = np.asarray(sorted(keep), np.int64)
+    out = dict(arrays)
+    for k in ("roi_chrom", "roi_start", "roi_stop", "roi_read_begin", "roi_n_reads"):
+        out[k] = np.asarray(arrays[k])[keep]
+    return out
+
+
+def redraw_mapq(arrays, seed=7):
+    """every read's MAPQ drawn again over 0-255, weighted toward the gates of the calling path (5/6, 9/10, 19/20) and toward 255"""
+    rng = np.random.default_rng(seed)
+    n = len(arrays["mapq"])
+    edges = np.array([5, 6, 9, 10, 19, 20, 255], np.uint8)
+    pick = rng.random(n)
+    m = rng.integers(0, 256, n).astype(np.uint8)
+    m = np.where(pick < 0.45, edges[rng.integers(0, len(edges), n)], m)
+    m = np.where((pick >= 0.45) & (pick < 0.6), np.uint8(255), m)
+    out = dict(arrays)
+    out["mapq"] = m
+    return out
+
+
+def tiled_region(ref, at, span, read_len, step, hap=None, mapq=60, last_len=None):
+    """reads of `read_len` bases every `step` bases from `at` (of `hap`, the reference by default), the last one `last_len` long, so that
+    they assemble into one contig of exactly `span` bases: each read overlaps the contig by read_len - step >= 0.88 of its length"""
+    src = ref if hap is None else hap
+    reads, s = [], at
+    while True:
+        n = at + span - s
+        if n <= (last_len or read_len) + step - 1:           # the last read: read_len .. read_len + step - 1 bases
+            reads.append(dict(start=s, seq=src[s:s + n], mapq=mapq))
+            break
+        reads.append(dict(start=s, seq=src[s:s + read_len], mapq=mapq))
+        s += step
+    assert reads[-1]["start"] + len(reads[-1]["seq"]) == at + span
+    return reads
+
+
+def cap_fixture(cap, seed=11):
+    """regions around max_contig_len = cap, in pool order: [0] reads tiling exactly cap bases (called), [1] exactly cap + 1 bases (the merge
+    check drops it), and when cap + 1 fits max_read_len, [2] five copies of one read of cap bases (called) and [3] of cap + 1 bases (the
+    read-trim check drops it); a region with a 12-base deletion at the end keeps the batch calling a variant"""
+    rng = np.random.default_rng(seed)
+    ref = random_seq(rng, 3 * cap + 12000)
+    sets, at = [], 1000
+    for span in (cap, cap + 1):
+        reads = tiled_region(ref, at, span, 100, 10)
+        sets.append(rois_from_reads(reads, ref, roi_start=at + 40, roi_stop=at + 60)[1]); at += span + 1000
+    if cap < 512:
+        for n in (cap, cap + 1):
+            reads = [dict(start=at, seq=ref[at:at + n]) for _ in range(5)]
+            sets.append(rois_from_reads(reads, ref, roi_start=at + 40, roi_stop=at + 60)[1]); at += n + 1000
+    hap = ref[:at + 100] + ref[at + 112:]
+    reads = [dict(start=at + i, seq=(hap if (i // 3) % 2 else ref)[at + i:at + i + 100]) for i in range(30, 72, 3)]
+    sets.append(rois_from_reads(reads, ref, roi_start=at + 90, roi_stop=at + 120)[1])
+    return merge_rois(sets)
+
+
+def length_fixture(lengths, seed=3, mapqs=None):
+    """one region per entry of `lengths` (a list of read lengths): reads of those lengths, alternately from the reference and from a haplotype
+    with a 12-base deletion in a tandem repeat, all overlapping the deletion; qualities 30, so every trimmed length equals the read's length.  mapqs: optional
+    per-region list of MAPQs (cycled over the reads)"""
+    rng = np.random.default_rng(seed)
+    sets, ref_parts, off = [], [], 0
+    for k, lens in enumerate(lengths):
+        L = max(lens)
+        seg = random_seq(rng, 2 * L + 400)
+        d = L + 200                                   # deletion of seg[d:d + 12]: two units of a 6-base tandem repeat (the AL fallback)
+        seg = seg[:d - 24] + "ACGTTG" * 10 + seg[d + 36:]
+        hap = seg[:d] + seg[d + 12:]
+        reads = []
+        for i, n in enumerate(lens):
+            lo, hi = max(0, d - n + 20), d - 20       # the read covers the deletion with >= 20 bases on each side
+            s = lo + (i * 7919) % max(1, hi - lo)
+            src = hap if i % 2 else seg
+            r = dict(start=off + s, seq=src[s:s + n])
+            if mapqs is not None:
+                r["mapq"] = int(mapqs[k][i % len(mapqs[k])])
+            reads.append(r)
+        reads.sort(key=lambda r: r["start"])
+        ref_parts.append(seg)
+        sets.append((reads, off + d - 10, off + d + 22))
+        off += len(seg)
+    ref = "".join(ref_parts)
+    return merge_rois([rois_from_reads(r, ref, roi_start=a, roi_stop=b)[1] for r, a, b in sets])
+
+
+def corr_fixture(sites=(128, 129), seed=13):
+    """one region per entry of `sites`: a 500-base read with three 100-base copies of its start (a contig of 4 reads whose last 400 bases
+    have support 1) and four copies of a 499-base read one base to the right that differs from it at `n` positions of those 400 bases.
+    The two contigs stay apart in assemble (a single read never votes) and merge in the first combine pass with exactly n voting sites,
+    every one allowed (support 4 against 1, both contigs of 4 reads)"""
+    rng = np.random.default_rng(seed)
+    sets, parts, off = [], [], 0
+    for n in sites:
+        seg = random_seq(rng, 1000)
+        a = seg[200:700]
+        b = list(seg[201:700])
+        for k in range(n):
+            p = 120 + 2 * k - 1                              # position 120 + 2k of the long read
+            b[p] = "ACGT"[("ACGT".index(b[p]) + 1 + k % 3) % 4]
+        b = "".join(b)
+        reads = [dict(start=off + 200, seq=a)] + [dict(start=off + 200, seq=a[:100]) for _ in range(3)] + \
+                [dict(start=off + 201, seq=b) for _ in range(4)]
+        sets.append((reads, off + 400, off + 420))
+        parts.append(seg); off += len(seg)
+    ref = "".join(parts)
+    return merge_rois([rois_from_reads(r, ref, roi_start=lo, roi_stop=hi)[1] for r, lo, hi in sets])
+
+
+def long_contig_fixture(spans=(6000, 4900), seed=17):
+    """one region per entry of `spans`: 250-base reads every 20 bases of a haplotype with a 12-base deletion in the middle, which assemble
+    into one contig of about `span` bases aligned to a window about as long (call-site A, band 50)"""
+    rng = np.random.default_rng(seed)
+    sets, parts, off = [], [], 0
+    for span in spans:
+        seg = random_seq(rng, span + 1000)
+        d = 500 + span // 2
+        hap = seg[:d] + seg[d + 12:]
+        reads = tiled_region(hap, 500, span, 250, 20)
+        for r in reads:
+            r["start"] += off
+            if r["start"] - off + len(r["seq"]) > d:
+                r["stop"] = r["start"] + len(r["seq"]) + (12 if r["start"] - off < d else 0)
+        sets.append((reads, off + d - 10, off + d + 22))
+        parts.append(seg); off += len(seg)
+    ref = "".join(parts)
+    return merge_rois([rois_from_reads(r, ref, roi_start=lo, roi_stop=hi)[1] for r, lo, hi in sets])
