@@ -296,6 +296,7 @@ typedef struct idl_sweep_out {
 	float ms_h2d, ms_kernels, ms_d2h;       /* CUDA events on the call's stream */
 	uint64_t algorithmic_bytes;   /* records + CIGARs once, one evidence byte per position written and read once, results */
 	uint64_t streamed_bytes;      /* what the passes really move through HBM (memsets, difference array twice, evidence + cuts twice ...) */
+	size_t n_edge[2];             /* idl_bam_sweep_window: selected runs left out because they touch zone_lo / zone_hi (0 otherwise) */
 } idl_sweep_out;
 
 int idl_sweep(int device, const idl_sweep_in *in, int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out);
@@ -351,6 +352,16 @@ void idl_bam_close(idl_bam *bam);
 /* gen_roi for one target on the resident records: the regions idl_sweep returns for the same records given as host arrays;
  * read_idx[] are indices into the BAM's kept records (0 .. n_records). */
 int idl_bam_sweep(idl_bam *bam, int32_t target, int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out);
+
+/* The same on a ZONE of positions [zone_lo, zone_hi] (0 <= zone_lo <= zone_hi <= chrom_len) and for the regions that overlap one of n_iv intervals
+ * [iv_beg[k], iv_end[k]) (0-based, half open, sorted and disjoint; n_iv = 0 selects nothing).  The position passes cover only the zone, so the cost
+ * follows the zone and the records, not the target's length.  A region is returned when it overlaps an interval and lies strictly inside the zone:
+ * roi_start > zone_lo unless zone_lo == 0, roi_end < zone_hi unless zone_hi == chrom_len.  Such a region equals the whole target's when the records
+ * are every record that touches the zone (DESIGN.md 4a: a slice of the file that starts at a linear-index offset and ends at a record boundary).
+ * Selected runs that touch an inner edge are left out and counted in out->n_edge[0] (zone_lo) and out->n_edge[1] (zone_hi): evidence beyond the
+ * zone may extend them, and the caller widens the zone and calls again.  With IDL_SWEEP_EVIDENCE the evidence bytes of the zone's positions. */
+int idl_bam_sweep_window(idl_bam *bam, int32_t target, int32_t zone_lo, int32_t zone_hi, size_t n_iv, const int32_t *iv_beg, const int32_t *iv_end,
+                         int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out);
 
 #define IDL_BAM_SEQ 1u      /* bases (ASCII, "=ACMGRSVTWYHKDBN") and qualities */
 #define IDL_BAM_CIGAR 2u    /* CIGAR operations */

@@ -134,6 +134,20 @@ idlh_dataset *idlh_load_targets(const char *fasta_path, const char *bam_path, ch
  * chain inside it as idl_bam_open_slice takes them; 0 ok, 1 the index lists no record for the target, -1 error */
 int idlh_bai_target_span(const char *bam_path, int32_t target, uint64_t *file_begin, uint64_t *file_end, uint64_t *first_record, uint64_t *end_member,
                          uint64_t *end_offset, char *err, size_t errlen);
+/* the records of one target from the first record of 16 kb window w0 (linear index) to the first record of window w1 + 1, or to the target's end
+ * (*to_end = 1): the run of members as idl_bam_open_slice takes it, and *zone_lo, the first position whose evidence, cuts and records are those of the
+ * whole file (0 at window 0 or at the target's first record, else (w0 << 14) + 1; DESIGN.md 4a).  0 ok, 1 the run holds no record, -1 error */
+int idlh_bai_region_run(const char *bam_path, int32_t target, int64_t w0, int64_t w1, uint64_t *file_begin, uint64_t *file_end, uint64_t *first_record,
+                        uint64_t *end_member, uint64_t *end_offset, int64_t *zone_lo, int32_t *to_end, char *err, size_t errlen);
+/* -r / -R of the command line: region strings chr[:beg[-end]] (1-based, inclusive, commas allowed in numbers) and a BED file (0-based, half open; '#',
+ * 'track', 'browser' and blank lines skipped, CRLF accepted, columns after the third ignored), validated against the targets of the BAM header, as
+ * sorted, merged half-open intervals per target.  Intervals are clipped to the target; intervals on a decoy target (hs37d5, GL*, which are never
+ * called, src/indelope.nim:41-42) are dropped with a note on stderr.  NULL with the reason in err (the BED line number included). */
+typedef struct idlh_regions idlh_regions;
+idlh_regions *idlh_regions_parse(int32_t n_ref, const char *const *ref_name, const int64_t *ref_len, int32_t n_region, const char *const *region, const char *bed_path,
+                                 char *err, size_t errlen);
+int64_t idlh_regions_get(const idlh_regions *r, int32_t target, int64_t *beg, int64_t *end, int64_t cap);   /* intervals of a target (up to cap copied); returns their number */
+void idlh_regions_free(idlh_regions *r);
 int idlh_dataset_set_targets(idlh_dataset *d, int32_t n_ref, const char *const *ref_name, const int64_t *ref_len, char *err, size_t errlen);
 idlh_rois *idlh_rois_from_arrays(const idlh_dataset *d, int64_t n_reads, const int32_t *start, const int32_t *stop, const int32_t *len, const uint8_t *mapq, const uint16_t *flag,
                                  const int64_t *seq_off, const uint8_t *bases, const uint8_t *quals, int64_t n_rois, const int32_t *roi_chrom, const int32_t *roi_start,

@@ -110,12 +110,17 @@ class Caller:
         self.ctx.close()
 
 
-def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4, max_reads=400_000, by_target=False, timings=None, **kw):
+def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4, max_reads=400_000, by_target=False, timings=None, regions=None, bed=None, **kw):
     """`indelope --gpu-decode [options] <fasta> <bam>` in process: the VCF (header + records) with everything in front of callsemble on the
     device as well -- BGZF inflate and record parse (idl_bam_open), gen_roi per target (idl_bam_sweep, src/indelope.nim:515-545,601-602), the
     batches built from the resident records (idl_bam_submit).  The host reads the two files and writes the VCF text.
     by_target: the file is not decoded as a whole but target by target, each from the run of BGZF members <bam>.bai points to
-    (idl_bam_open_slice) -- for files that do not fit in device memory; needs the index."""
+    (idl_bam_open_slice) -- for files that do not fit in device memory; needs the index.
+    regions (list of `chr[:beg[-end]]`, 1-based, inclusive) and / or bed (a BED file, 0-based, half open): `indelope -r ... -R ...` -- only the regions of
+    interest of the whole-file run that overlap them, from just the BGZF members that hold them (idl_bam_sweep_window; needs the index).  `timings` then
+    also receives one dict per target with slices, retries and bytes read and decoded.  ValueError for a bad region or BED line."""
+    if regions or bed:
+        by_target = True
     if by_target:
         st = host.Stream(fasta, bam)          # parses the BAM header and orders the FASTA's sequences after it; no record is read through it
         tg = st.targets()
@@ -130,50 +135,116 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
         ref.set_targets(whole.ref_names, whole.ref_len)
         names, seqs = ref.sequences()
         keep = (ref,)
+    selected = None
+    if regions or bed:
+        selected = host.parse_regions(names, ref_len, regions, bed)
+        if names:
+            host.bai_target_span(bam, 0)      # IOError without the index, before anything runs
     caller = Caller(device, min_reads=min_reads, min_ctg_len=min_ctg_len, min_event_len=min_event_len, **kw)
     writer = host.VcfWriter()
     empty = dict(start=[], stop=[], mapq=[], flag=[], len=[], seq_off=[], bases=[], quals=[])
     out = [host.Rois(arrays=dict(empty, roi_chrom=[], roi_start=[], roi_stop=[], roi_read_begin=[], roi_n_reads=[], read_idx=[], chrom_names=names, chrom_seqs=seqs)).header()]
-    n_regions_done = 0
+    done = [0]
+    sweep_args = dict(min_event_support=max(3, min_reads - 2), min_read_coverage=min_reads, max_read_coverage=600)
+
+    def slice_of(sp):
+        with open(bam, "rb") as f:
+            f.seek(sp["file_begin"]); run = f.read(sp["file_end"] - sp["file_begin"])
+        return cuda.Bam(run, device=device, slice=dict(ref_names=names, ref_len=ref_len, first_record=sp["first_record"], end_member=sp["end_member"],
+                                                       end_offset=sp["end_offset"])), len(run)
+
+    def call_swept(b, c, r, first=0):
+        """regions [first, n) of one sweep of b through idl_bam_submit, records appended to out"""
+        n = len(r["roi_start"]) - first
+        if n <= 0:
+            return
+        chrom = np.full(n, c, np.int32)
+        rs, re, nr = r["roi_start"][first:], r["roi_end"][first:], r["roi_n_reads"][first:]
+        idx = r["read_idx"][int(r["roi_read_begin"][first]):]
+        begin = np.concatenate([[0], np.cumsum(nr)]).astype(np.int64)
+        rois = host.Rois(arrays=dict(empty, roi_chrom=chrom, roi_start=rs, roi_stop=re, roi_read_begin=begin[:-1], roi_n_reads=nr, read_idx=idx, chrom_names=names, chrom_seqs=seqs))
+        b.set_reference(c, seqs[c])
+        inflight = []
+
+        def drain():
+            lo, t = inflight.pop(0)
+            res = caller.ctx.wait(t)
+            v, _ = writer.records(rois, lo, caller.params, res, 0)
+            if timings is not None:
+                timings.append({k: getattr(res.contents, k) for k in ("ms_assemble", "ms_align", "ms_genotype", "ms_al", "n_regions", "n_events")})
+            caller.ctx.release(t); out.append(v)
+        for lo, hi in plan_batches(rois, 0, n, max_reads=max_reads):
+            if len(inflight) >= caller.params.n_streams:
+                drain()
+            inflight.append((lo, caller.ctx.bam_submit(b, chrom[lo:hi], rs[lo:hi], re[lo:hi], nr[lo:hi], idx[begin[lo]:begin[hi]], ordinal_base=done[0] + lo)))
+        while inflight:
+            drain()
+        done[0] += n
+
+    def call_target_regions(c, ivs):
+        """the slices of one target's intervals, grown until no selected region touches an inner zone edge (indelope_main.cpp main_regions)"""
+        stats = dict(target=c, intervals=len(ivs), slices=0, retries=0, bytes_read=0, bytes_decoded=0, regions=0)
+        todo = []
+        for b0, e0 in ivs:
+            w0, w1 = ((b0 - 1) >> 14) if b0 > 0 else 0, ((e0 - 1) >> 14) + 1
+            if todo and w0 <= todo[-1][1]:
+                todo[-1] = [todo[-1][0], max(todo[-1][1], w1), todo[-1][2] + [(b0, e0)], None]
+            else:
+                todo.append([w0, w1, [(b0, e0)], None])
+        for s in todo:
+            s[3] = host.bai_region_run(bam, c, s[0], s[1])
+        last_end = -1
+        while todo:
+            w0, w1, iv, run = todo.pop(0)
+            while todo and not run["empty"] and not todo[0][3]["empty"] and todo[0][3]["file_begin"] <= run["file_end"]:
+                n = todo.pop(0); w1 = max(w1, n[1]); iv = iv + n[2]
+                run = host.bai_region_run(bam, c, w0, w1)
+            if run["empty"]:
+                if not run["to_end"]:
+                    stats["retries"] += 1
+                    todo.insert(0, [w0, w1 + 1, iv, host.bai_region_run(bam, c, w0, w1 + 1)])
+                continue
+            b, nbytes = slice_of(run)
+            try:
+                stats["slices"] += 1; stats["bytes_read"] += nbytes; stats["bytes_decoded"] += b.info["inflated_bytes"]
+                zone_hi = ref_len[c] if run["to_end"] else int(b.fetch([b.n_records - 1], what=0)["start"][0]) - 1
+                if zone_hi < run["zone_lo"] or zone_hi < iv[-1][1] - 1:
+                    stats["retries"] += 1
+                    todo.insert(0, [w0, w1 + 1, iv, host.bai_region_run(bam, c, w0, w1 + 1)])
+                    continue
+                r = b.sweep_window(c, run["zone_lo"], zone_hi, [x[0] for x in iv], [x[1] for x in iv], **sweep_args)
+                if r["n_edge"][0] or r["n_edge"][1]:
+                    stats["retries"] += 1
+                    w0, w1 = w0 - (1 if r["n_edge"][0] else 0), w1 + (1 if r["n_edge"][1] else 0)
+                    todo.insert(0, [w0, w1, iv, host.bai_region_run(bam, c, w0, w1)])
+                    continue
+                first = int(np.searchsorted(r["roi_start"], last_end, side="right"))   # regions an earlier slice (before this one grew left) called
+                call_swept(b, c, r, first)
+                stats["regions"] += len(r["roi_start"]) - first
+                if len(r["roi_start"]) > first:
+                    last_end = int(r["roi_end"][-1])
+            finally:
+                b.close()
+        if timings is not None:
+            timings.append(stats)
+
     try:
         for c, name in enumerate(names):
             if name == "hs37d5" or name.startswith("GL"):   # skippable targets, src/indelope.nim:41-42
+                continue
+            if selected is not None:
+                if selected[c]:
+                    call_target_regions(c, selected[c])
                 continue
             if by_target:
                 sp = host.bai_target_span(bam, c)
                 if sp is None:
                     continue
-                with open(bam, "rb") as f:
-                    f.seek(sp["file_begin"]); run = f.read(sp["file_end"] - sp["file_begin"])
-                b = cuda.Bam(run, device=device, slice=dict(ref_names=names, ref_len=ref_len, first_record=sp["first_record"], end_member=sp["end_member"],
-                                                            end_offset=sp["end_offset"]))
+                b, _ = slice_of(sp)
             else:
                 b = whole
             try:
-                r = b.sweep(c, min_event_support=max(3, min_reads - 2), min_read_coverage=min_reads, max_read_coverage=600)
-                n = len(r["roi_start"])
-                if n == 0:
-                    continue
-                chrom = np.full(n, c, np.int32); rs, re, nr, idx = r["roi_start"], r["roi_end"], r["roi_n_reads"], r["read_idx"]
-                begin = np.concatenate([[0], np.cumsum(nr)]).astype(np.int64)
-                rois = host.Rois(arrays=dict(empty, roi_chrom=chrom, roi_start=rs, roi_stop=re, roi_read_begin=begin[:-1], roi_n_reads=nr, read_idx=idx, chrom_names=names, chrom_seqs=seqs))
-                b.set_reference(c, seqs[c])
-                inflight = []
-
-                def drain():
-                    lo, t = inflight.pop(0)
-                    res = caller.ctx.wait(t)
-                    v, _ = writer.records(rois, lo, caller.params, res, 0)
-                    if timings is not None:
-                        timings.append({k: getattr(res.contents, k) for k in ("ms_assemble", "ms_align", "ms_genotype", "ms_al", "n_regions", "n_events")})
-                    caller.ctx.release(t); out.append(v)
-                for lo, hi in plan_batches(rois, 0, n, max_reads=max_reads):
-                    if len(inflight) >= caller.params.n_streams:
-                        drain()
-                    inflight.append((lo, caller.ctx.bam_submit(b, chrom[lo:hi], rs[lo:hi], re[lo:hi], nr[lo:hi], idx[begin[lo]:begin[hi]], ordinal_base=n_regions_done + lo)))
-                while inflight:
-                    drain()
-                n_regions_done += n
+                call_swept(b, c, b.sweep(c, **sweep_args))
             finally:
                 if by_target:
                     b.close()

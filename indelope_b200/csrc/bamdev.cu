@@ -826,11 +826,15 @@ done:
 #undef BFAIL
 }
 
-int idl_bam_sweep(idl_bam *b, int32_t target, int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out)
+// idl_bam_sweep (n_iv < 0: the whole target) and idl_bam_sweep_window
+static int bam_sweep(idl_bam *b, int32_t target, int64_t zone_lo, int64_t zone_hi, long long n_iv, const int32_t *iv_beg, const int32_t *iv_end,
+                     int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out)
 {
 	if (!b || !out || target < 0 || target >= b->info.n_ref) return IDL_E_ARG;
 	const size_t r0 = (size_t)b->ref_first[(size_t)target], r1 = (size_t)b->ref_first[(size_t)target + 1];
 	if (b->ref_len[(size_t)target] > INT_MAX) return IDL_E_CAPACITY;
+	if (n_iv < 0) zone_hi = b->ref_len[(size_t)target];
+	if (zone_lo < 0 || zone_hi < zone_lo || zone_hi > b->ref_len[(size_t)target]) return IDL_E_ARG;
 	if (r1 == r0 && !(flags & IDL_SWEEP_EVIDENCE)) {
 		// a target without records has no regions (a header with thousands of alt / decoy contigs): nothing to launch
 		idl_sweep_out *o = (idl_sweep_out*)calloc(1, sizeof *o);
@@ -844,10 +848,23 @@ int idl_bam_sweep(idl_bam *b, int32_t target, int32_t min_event_support, int32_t
 	in.chrom_len = (int32_t)b->ref_len[(size_t)target]; in.n_reads = r1 - r0;
 	in.start = b->R.pos + r0; in.stop = b->R.stop + r0; in.flag = b->R.flag + r0; in.cigar = b->d_cigar; in.cig_off = (const uint64_t*)(b->d_cig_off + r0);
 	if (cudaStreamSynchronize(b->st) != cudaSuccess) return IDL_E_CUDA;
-	const int rc = idl_sweep_impl(b->device, &in, true, 0, min_event_support, min_read_coverage, max_read_coverage, flags, out);
+	const int rc = idl_sweep_impl(b->device, &in, true, 0, (int32_t)zone_lo, (int32_t)zone_hi, n_iv, iv_beg, iv_end, min_event_support, min_read_coverage, max_read_coverage,
+	                              flags, out);
 	if (rc != IDL_OK) return rc;
 	for (size_t k = 0; k < (*out)->n_read_idx; ++k) (*out)->read_idx[k] += (int64_t)r0;
 	return IDL_OK;
+}
+
+int idl_bam_sweep(idl_bam *b, int32_t target, int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out)
+{
+	return bam_sweep(b, target, 0, 0, -1, nullptr, nullptr, min_event_support, min_read_coverage, max_read_coverage, flags, out);
+}
+
+int idl_bam_sweep_window(idl_bam *b, int32_t target, int32_t zone_lo, int32_t zone_hi, size_t n_iv, const int32_t *iv_beg, const int32_t *iv_end,
+                         int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out)
+{
+	if (n_iv >= (1ull << 31)) return IDL_E_CAPACITY;
+	return bam_sweep(b, target, zone_lo, zone_hi, (long long)n_iv, iv_beg, iv_end, min_event_support, min_read_coverage, max_read_coverage, flags, out);
 }
 
 void idl_bam_reads_free(idl_bam_reads *r)

@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <atomic>
 #include <map>
+#include <memory>
 #include <condition_variable>
 #include <deque>
 #include <mutex>
@@ -360,56 +361,63 @@ int idlh_write_bam(const idlh_dataset *d, const char *path, int level)
 
 /* reference FASTA + coordinate-sorted BAM -> dataset.  Records without a reference id are dropped (a per-target query never
  * returns them); everything else, flags included, is kept for the sweep's `skippable` test (src/indelope.nim:40-47). */
-/* Where the records of one target lie in the BAM file, from <bam>.bai (SAM spec 5.2): the smallest chunk begin and the largest chunk end of the target's
- * bins are the virtual offsets of its first record and of the byte behind its last one.  [*file_begin, *file_end) is the run of whole BGZF members that
- * holds them, *first_record the offset of the first record inside the inflated bytes of that run, (*end_member, *end_offset) the end as idl_bam_open_slice
- * takes it.  Returns 0, 1 when the index lists no record for the target, -1 on error. */
-int idlh_bai_target_span(const char *bam_path, int32_t target, uint64_t *file_begin, uint64_t *file_end, uint64_t *first_record, uint64_t *end_member,
-                         uint64_t *end_offset, char *err, size_t errlen)
+} // extern "C"
+
+namespace {
+
+// What the region front ends need of <bam>.bai (SAM spec 5.2), per target: the smallest chunk begin and the largest chunk end of its bins (the virtual
+// offsets of its first record and of the byte behind its last one) and its 16 kb linear index.  The index read last is kept (a header with thousands of
+// targets asks for them one after the other, a region list for one target after the other).
+struct BaiSummary { std::vector<std::pair<uint64_t, uint64_t>> span; std::vector<std::vector<uint64_t>> lin; };
+
+bool bai_summary(const char *bam_path, std::shared_ptr<const BaiSummary> &out, std::string &why)
 {
-	// the spans of every target of the index read last (a header with thousands of targets asks for them one after the other)
-	static std::mutex mu; static std::string cached_path; static std::vector<std::pair<uint64_t, uint64_t>> spans;
+	static std::mutex mu; static std::string cached_path; static long long cached_stamp = -1; static std::shared_ptr<const BaiSummary> cached;
 	std::lock_guard<std::mutex> lock(mu);
-	static long long cached_stamp = -1;
 	long long stamp = -1;
 	{ struct stat sb; if (stat((std::string(bam_path) + ".bai").c_str(), &sb) == 0) stamp = (long long)sb.st_mtime * 1000003LL + (long long)sb.st_size; }
 	if (cached_path != bam_path || stamp != cached_stamp) {
-		cached_stamp = stamp;
-		cached_path.clear(); spans.clear();
-		std::vector<uint8_t> bai; std::string why;
-		if (!read_file((std::string(bam_path) + ".bai").c_str(), bai, why)) { set_err(err, errlen, why + " (no index: write one with idlh_write_bam or samtools index)"); return -1; }
-		if (bai.size() < 8 || memcmp(bai.data(), "BAI\1", 4) != 0) { set_err(err, errlen, "not a BAI index"); return -1; }
+		cached_path.clear(); cached.reset();
+		std::vector<uint8_t> bai;
+		if (!read_file((std::string(bam_path) + ".bai").c_str(), bai, why)) { why += " (no index: write one with idlh_write_bam or samtools index)"; return false; }
+		if (bai.size() < 8 || memcmp(bai.data(), "BAI\1", 4) != 0) { why = "not a BAI index"; return false; }
 		size_t ia = 4;
 		auto rd32 = [&](uint32_t &x) -> bool { if (ia + 4 > bai.size()) return false; x = le32(bai.data() + ia); ia += 4; return true; };
 		auto rd64 = [&](uint64_t &x) -> bool { if (ia + 8 > bai.size()) return false; x = (uint64_t)le32(bai.data() + ia) | (uint64_t)le32(bai.data() + ia + 4) << 32; ia += 8; return true; };
 		uint32_t n_ref = 0;
-		if (!rd32(n_ref)) { set_err(err, errlen, "truncated index"); return -1; }
-		std::vector<std::pair<uint64_t, uint64_t>> sp;
+		BaiSummary S;
+		if (!rd32(n_ref)) { why = "truncated index"; return false; }
 		for (uint32_t r = 0; r < n_ref; ++r) {
 			uint64_t lo = ~0ULL, hi = 0;
 			uint32_t n_bin = 0;
-			if (!rd32(n_bin)) { set_err(err, errlen, "truncated index"); return -1; }
+			if (!rd32(n_bin)) { why = "truncated index"; return false; }
 			for (uint32_t b = 0; b < n_bin; ++b) {
 				uint32_t bin = 0, n_chunk = 0;
-				if (!rd32(bin) || !rd32(n_chunk)) { set_err(err, errlen, "truncated index"); return -1; }
+				if (!rd32(bin) || !rd32(n_chunk)) { why = "truncated index"; return false; }
 				for (uint32_t c = 0; c < n_chunk; ++c) {
 					uint64_t a = 0, z = 0;
-					if (!rd64(a) || !rd64(z)) { set_err(err, errlen, "truncated index"); return -1; }
+					if (!rd64(a) || !rd64(z)) { why = "truncated index"; return false; }
 					if (bin != 37450u) { lo = std::min(lo, a); hi = std::max(hi, z); }   // 37450: the metadata pseudo-bin of samtools
 				}
 			}
 			uint32_t n_intv = 0;
-			if (!rd32(n_intv) || ia + (size_t)n_intv * 8 > bai.size()) { set_err(err, errlen, "truncated index"); return -1; }
-			ia += (size_t)n_intv * 8;
-			sp.push_back({lo, hi});
+			if (!rd32(n_intv) || ia + (size_t)n_intv * 8 > bai.size()) { why = "truncated index"; return false; }
+			std::vector<uint64_t> lin(n_intv);
+			for (uint32_t w = 0; w < n_intv; ++w) rd64(lin[w]);
+			S.span.push_back({lo, hi}); S.lin.push_back(std::move(lin));
 		}
-		spans.swap(sp); cached_path = bam_path;
+		cached = std::make_shared<const BaiSummary>(std::move(S)); cached_path = bam_path; cached_stamp = stamp;
 	}
-	if (target < 0 || (size_t)target >= spans.size()) { set_err(err, errlen, "the index has no such target"); return -1; }
-	const uint64_t vmin = spans[(size_t)target].first, vmax = spans[(size_t)target].second;
-	if (vmin == ~0ULL || vmax <= vmin) return 1;
-	*file_begin = vmin >> 16; *first_record = vmin & 0xffff;
-	const uint64_t ce = vmax >> 16, ue = vmax & 0xffff;
+	out = cached;
+	return true;
+}
+
+// the run of whole BGZF members that holds the records at virtual offsets [vbeg, vend), as idl_bam_open_slice takes it
+int member_run(const char *bam_path, uint64_t vbeg, uint64_t vend, uint64_t *file_begin, uint64_t *file_end, uint64_t *first_record, uint64_t *end_member,
+               uint64_t *end_offset, char *err, size_t errlen)
+{
+	*file_begin = vbeg >> 16; *first_record = vbeg & 0xffff;
+	const uint64_t ce = vend >> 16, ue = vend & 0xffff;
 	*end_member = ce - *file_begin; *end_offset = ue;
 	if (ue == 0) { *file_end = ce; return 0; }
 	// the member the records end in is part of the run: its size is in its own header
@@ -422,6 +430,150 @@ int idlh_bai_target_span(const char *bam_path, int32_t target, uint64_t *file_be
 	*file_end = ce + (uint64_t)le16(h + 16) + 1;
 	return 0;
 }
+
+bool is_decoy(const std::string &name) { return name == "hs37d5" || name.compare(0, 2, "GL") == 0; }   // skippable targets, src/indelope.nim:41-42
+
+} // namespace
+
+extern "C" {
+
+/* Where the records of one target lie in the BAM file, from <bam>.bai (SAM spec 5.2): the smallest chunk begin and the largest chunk end of the target's
+ * bins are the virtual offsets of its first record and of the byte behind its last one.  [*file_begin, *file_end) is the run of whole BGZF members that
+ * holds them, *first_record the offset of the first record inside the inflated bytes of that run, (*end_member, *end_offset) the end as idl_bam_open_slice
+ * takes it.  Returns 0, 1 when the index lists no record for the target, -1 on error. */
+int idlh_bai_target_span(const char *bam_path, int32_t target, uint64_t *file_begin, uint64_t *file_end, uint64_t *first_record, uint64_t *end_member,
+                         uint64_t *end_offset, char *err, size_t errlen)
+{
+	std::shared_ptr<const BaiSummary> P; std::string why;
+	if (!bai_summary(bam_path, P, why)) { set_err(err, errlen, why); return -1; }
+	const BaiSummary &S = *P;
+	if (target < 0 || (size_t)target >= S.span.size()) { set_err(err, errlen, "the index has no such target"); return -1; }
+	const uint64_t vmin = S.span[(size_t)target].first, vmax = S.span[(size_t)target].second;
+	if (vmin == ~0ULL || vmax <= vmin) return 1;
+	return member_run(bam_path, vmin, vmax, file_begin, file_end, first_record, end_member, end_offset, err, errlen);
+}
+
+/* The records of one target from the first record of 16 kb window w0 to the first record of window w1 + 1 (or to the target's last record), by the linear
+ * index of <bam>.bai.  Every record in front of the run ends at or before position W0 = w0 << 14 (that is what the linear index records; an empty window
+ * holds an earlier offset, which only moves the run's start forward in the file), so the evidence, cuts and record lists of positions >= *zone_lo =
+ * W0 + 1 are those of the whole file -- 0 when w0 == 0 or the run starts at the target's first record (DESIGN.md 4a).  *to_end = 1 when the run ends
+ * behind the target's last record.  The run as idl_bam_open_slice takes it.  Returns 0, 1 when the run holds no record, -1 on error. */
+int idlh_bai_region_run(const char *bam_path, int32_t target, int64_t w0, int64_t w1, uint64_t *file_begin, uint64_t *file_end, uint64_t *first_record,
+                        uint64_t *end_member, uint64_t *end_offset, int64_t *zone_lo, int32_t *to_end, char *err, size_t errlen)
+{
+	std::shared_ptr<const BaiSummary> P; std::string why;
+	if (!bai_summary(bam_path, P, why)) { set_err(err, errlen, why); return -1; }
+	const BaiSummary &S = *P;
+	if (target < 0 || (size_t)target >= S.span.size()) { set_err(err, errlen, "the index has no such target"); return -1; }
+	if (w0 < 0 || w1 < w0) { set_err(err, errlen, "bad window range"); return -1; }
+	const uint64_t vmin = S.span[(size_t)target].first, vmax = S.span[(size_t)target].second;
+	const std::vector<uint64_t> &lin = S.lin[(size_t)target];
+	*zone_lo = 0; *to_end = 1;
+	if (vmin == ~0ULL || vmax <= vmin) return 1;
+	auto first_of = [&](int64_t w) -> uint64_t {   // the first record of window w; the target's end behind its last window
+		if ((uint64_t)w >= lin.size()) return vmax;
+		const uint64_t o = lin[(size_t)w];
+		return o < vmin ? vmin : (o > vmax ? vmax : o);   // 0: no record up to this window (htslib writes empty windows so)
+	};
+	const uint64_t vb = first_of(w0), ve = std::max(vb, first_of(w1 + 1));
+	*to_end = ve >= vmax;
+	*zone_lo = (w0 == 0 || vb == vmin) ? 0 : (w0 << 14) + 1;
+	if (ve <= vb) return 1;
+	return member_run(bam_path, vb, ve, file_begin, file_end, first_record, end_member, end_offset, err, errlen);
+}
+
+/* -r / -R: region strings (1-based, inclusive, as samtools takes them) and BED lines (0-based, half open) -> per target sorted, merged half-open intervals */
+struct idlh_regions { std::vector<std::vector<std::pair<int64_t, int64_t>>> iv; };
+
+idlh_regions *idlh_regions_parse(int32_t n_ref, const char *const *ref_name, const int64_t *ref_len, int32_t n_region, const char *const *region, const char *bed_path,
+                                 char *err, size_t errlen)
+{
+	auto R = std::unique_ptr<idlh_regions>(new idlh_regions());
+	R->iv.resize(n_ref > 0 ? (size_t)n_ref : 0);
+	std::map<std::string, int32_t> tid;
+	for (int32_t c = 0; c < n_ref; ++c) tid[ref_name[c]] = c;
+	std::vector<char> noted((size_t)std::max(n_ref, 0), 0);
+	auto add = [&](int32_t c, int64_t b, int64_t e) {
+		if (is_decoy(ref_name[c])) {
+			if (!noted[(size_t)c]) fprintf(stderr, "indelope: note: %s is a decoy target and is not called\n", ref_name[c]);
+			noted[(size_t)c] = 1;
+			return;
+		}
+		b = std::min(b, ref_len[c]); e = std::min(e, ref_len[c]);
+		if (b < e) R->iv[(size_t)c].push_back({b, e});
+	};
+	// a number with optional thousands commas; false if anything else is there
+	auto number = [](const std::string &t, int64_t &x) -> bool {
+		std::string d;
+		for (char ch : t) { if (ch == ',') continue; if (ch < '0' || ch > '9') return false; d += ch; }
+		if (d.empty() || d.size() > 15) return false;
+		x = std::stoll(d);
+		return true;
+	};
+	for (int32_t k = 0; k < n_region; ++k) {
+		const std::string r = region[k];
+		auto bad = [&](const std::string &why) -> idlh_regions* { set_err(err, errlen, "region '" + r + "': " + why); return nullptr; };
+		auto it = tid.find(r);   // a whole target, also one whose name contains ':'
+		if (it != tid.end()) { add(it->second, 0, ref_len[it->second]); continue; }
+		const size_t colon = r.rfind(':');
+		if (colon == std::string::npos) return bad("no such target in the BAM header");
+		const std::string name = r.substr(0, colon), rest = r.substr(colon + 1);
+		it = tid.find(name);
+		if (it == tid.end()) return bad("no such target in the BAM header");
+		const size_t dash = rest.find('-');
+		int64_t beg = 0, end = ref_len[it->second];
+		if (!number(rest.substr(0, dash), beg)) return bad("expected chr[:beg[-end]] with numbers");
+		if (dash != std::string::npos && dash + 1 < rest.size() && !number(rest.substr(dash + 1), end)) return bad("expected chr[:beg[-end]] with numbers");
+		if (beg < 1) return bad("beg must be >= 1 (1-based)");
+		if (end < beg) return bad("end must be >= beg");
+		add(it->second, beg - 1, end);
+	}
+	if (bed_path && *bed_path) {
+		std::vector<uint8_t> f; std::string why;
+		if (!read_file(bed_path, f, why)) { set_err(err, errlen, why); return nullptr; }
+		size_t at = 0; int64_t line_no = 0;
+		while (at < f.size()) {
+			size_t e = at;
+			while (e < f.size() && f[e] != '\n') ++e;
+			std::string line((const char*)f.data() + at, e - at);
+			at = e + 1; ++line_no;
+			while (!line.empty() && (line.back() == '\r' || line.back() == ' ' || line.back() == '\t')) line.pop_back();
+			if (line.empty() || line[0] == '#' || line.compare(0, 5, "track") == 0 || line.compare(0, 7, "browser") == 0) continue;
+			std::vector<std::string> col;
+			for (size_t p = 0; p <= line.size() && col.size() < 3; ) {
+				size_t q = line.find_first_of("\t ", p);
+				if (q == std::string::npos) q = line.size();
+				if (q > p) col.push_back(line.substr(p, q - p));
+				p = q + 1;
+			}
+			auto bad = [&](const std::string &w) -> idlh_regions* { set_err(err, errlen, std::string(bed_path) + " line " + std::to_string(line_no) + ": " + w); return nullptr; };
+			if (col.size() < 3) return bad("expected chrom, start and end");
+			const auto it = tid.find(col[0]);
+			if (it == tid.end()) return bad("target '" + col[0] + "' is not in the BAM header");
+			int64_t b = 0, en = 0;
+			if (col[1].find(',') != std::string::npos || col[2].find(',') != std::string::npos || !number(col[1], b) || !number(col[2], en)) return bad("start and end must be non-negative integers");
+			if (en < b) return bad("end is smaller than start");
+			add(it->second, b, en);
+		}
+	}
+	for (auto &v : R->iv) {   // sorted and merged: overlapping or touching intervals become one
+		std::sort(v.begin(), v.end());
+		std::vector<std::pair<int64_t, int64_t>> m;
+		for (const auto &x : v) { if (!m.empty() && x.first <= m.back().second) m.back().second = std::max(m.back().second, x.second); else m.push_back(x); }
+		v.swap(m);
+	}
+	return R.release();
+}
+
+int64_t idlh_regions_get(const idlh_regions *r, int32_t target, int64_t *beg, int64_t *end, int64_t cap)
+{
+	if (!r || target < 0 || (size_t)target >= r->iv.size()) return 0;
+	const auto &v = r->iv[(size_t)target];
+	for (size_t k = 0; k < v.size() && (int64_t)k < cap; ++k) { beg[k] = v[k].first; end[k] = v[k].second; }
+	return (int64_t)v.size();
+}
+
+void idlh_regions_free(idlh_regions *r) { delete r; }
 
 /* The FASTA's sequences ordered as the BAM header lists its targets, WITHOUT reading the BAM's records: only the first members of the file are read and
  * inflated, as far as the header reaches (what `open(b, path)` + `b.hdr.targets` give the reference's main, src/indelope.nim:595-601).  For the path that

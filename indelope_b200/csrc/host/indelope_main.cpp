@@ -40,6 +40,10 @@ static const char USAGE[] =
 	"  -d --device <INT>           CUDA device [default: 0]\n"
 	"  -g --gpu-decode             inflate and parse the BAM and find the regions of interest on the GPU as well (idl_bam_open,\n"
 	"                              idl_bam_sweep); the file is then read whole instead of streamed, --threads is not used\n"
+	"  -r --region <chr[:beg[-end]]>  call only the regions of interest that overlap this region (1-based, inclusive, as samtools; may be\n"
+	"                              repeated).  Only the BAM members that hold them are read, through <BAM>.bai; the regions found and called are\n"
+	"                              exactly those of the whole-file run that overlap the region\n"
+	"  -R --regions-file <BED>     the same for the intervals of a BED file (0-based, half open); -r and -R may be combined (their union)\n"
 	"  -h --help                   show help\n";
 
 struct Lane { idl_batch *batch = nullptr; size_t cap[4] = {0, 0, 0, 0}; };
@@ -216,6 +220,46 @@ static int main_gpu_decode(const std::string &fa, const std::string &bam_path, i
 	return status;
 }
 
+// regions [first, n_rois) of one sweep of a decoded slice (targets in header order, regions in gen_roi's order) through idl_bam_submit in batches, two in
+// flight, and their records on stdout; n_regions_before is the number of regions of the run emitted before these (the ordinals run on)
+static int call_swept(idl_ctx *ctx, idl_bam *bam, int32_t c, const idl_sweep_out *sw, size_t first, const idlh_dataset *ref, const idlh_roiset *all, const idl_params &P,
+                      idlh_vcf *writer, size_t n_regions_before)
+{
+	idl_sweep_out view = *sw, *so = &view;
+	view.n_rois -= first; view.roi_start += first; view.roi_end += first; view.roi_n_reads += first; view.read_idx += first < sw->n_rois ? sw->roi_read_begin[first] : 0;
+	int status = 0;
+	if (so->n_rois && idl_bam_set_reference(bam, c, all->chrom_seq[c], all->chrom_len[c]) != IDL_OK) status = die("idl_bam_set_reference", "could not place the reference on the device");
+	std::vector<int32_t> chrom(so->n_rois, c);
+	std::deque<Flight> inflight;
+	auto drain = [&]() -> bool {
+		const Flight fl = inflight.front(); inflight.pop_front();
+		const idl_results *res = nullptr;
+		const int w = idl_wait(ctx, fl.ticket, &res);
+		if (w != IDL_OK) { status = die("idl_wait", std::string(idl_strerror(w)) + " " + idl_last_cuda_error(ctx)); idlh_rois_free(fl.rois); return false; }
+		char *txt = idlh_vcf_records(writer, idlh_rois_view(fl.rois), 0, &P, res, 0, nullptr);
+		fputs(txt, stdout); idlh_free(txt);
+		idl_release(ctx, fl.ticket); idlh_rois_free(fl.rois);
+		return true;
+	};
+	size_t at_idx = 0;
+	for (size_t lo = 0; lo < so->n_rois && !status; ) {
+		size_t hi = lo; int64_t reads = 0;
+		while (hi < so->n_rois && (hi == lo || (reads + so->roi_n_reads[hi] <= 400000 && hi - lo < 20000))) reads += so->roi_n_reads[hi++];
+		idlh_rois *grp = idlh_rois_from_arrays(ref, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, (int64_t)(hi - lo), chrom.data() + lo,
+		                                       so->roi_start + lo, so->roi_end + lo, so->roi_n_reads + lo, so->read_idx + at_idx);
+		if (inflight.size() >= (size_t)(P.n_streams > 0 ? P.n_streams : 1) && !drain()) { idlh_rois_free(grp); break; }
+		uint64_t ticket = 0;
+		const int r = idl_bam_submit(ctx, bam, hi - lo, chrom.data() + lo, so->roi_start + lo, so->roi_end + lo, so->roi_n_reads + lo, so->read_idx + at_idx,
+		                             (uint32_t)(n_regions_before + lo), &ticket);
+		if (r != IDL_OK) { status = die("idl_bam_submit", std::string(idl_strerror(r)) + " " + idl_last_cuda_error(ctx)); idlh_rois_free(grp); break; }
+		inflight.push_back({grp, ticket});
+		at_idx += (size_t)reads; lo = hi;
+	}
+	while (!inflight.empty() && !status) if (!drain()) break;
+	while (!inflight.empty()) { idlh_rois_free(inflight.front().rois); inflight.pop_front(); }
+	return status;
+}
+
 // --gpu-decode for a file that does not fit in device memory as a whole (or with INDELOPE_BY_TARGET=1): target by target.  For every target the index
 // <bam>.bai says which run of BGZF members holds its records; that run is read, decoded on the device (idl_bam_open_slice), swept, called and dropped.
 // Regions keep gen_roi's order (targets in header order), so the dedup state carries over from target to target as in the reference's single loop.
@@ -291,34 +335,7 @@ static int main_gpu_by_target(const std::string &fa, const std::string &bam_path
 		if (r != IDL_OK) { status = die("idl_bam_sweep", idl_strerror(r)); idl_bam_close(bam); break; }
 		t_sweep += now_s() - t1; t1 = now_s();
 		++n_targets;
-		if (so->n_rois && idl_bam_set_reference(bam, c, all->chrom_seq[c], all->chrom_len[c]) != IDL_OK) status = die("idl_bam_set_reference", "could not place the reference on the device");
-		std::vector<int32_t> chrom(so->n_rois, c);
-		std::deque<Flight> inflight;
-		auto drain = [&]() -> bool {
-			const Flight fl = inflight.front(); inflight.pop_front();
-			const idl_results *res = nullptr;
-			const int w = idl_wait(ctx, fl.ticket, &res);
-			if (w != IDL_OK) { status = die("idl_wait", std::string(idl_strerror(w)) + " " + idl_last_cuda_error(ctx)); idlh_rois_free(fl.rois); return false; }
-			char *txt = idlh_vcf_records(writer, idlh_rois_view(fl.rois), 0, &P, res, 0, nullptr);
-			fputs(txt, stdout); idlh_free(txt);
-			idl_release(ctx, fl.ticket); idlh_rois_free(fl.rois);
-			return true;
-		};
-		size_t at_idx = 0;
-		for (size_t lo = 0; lo < so->n_rois && !status; ) {
-			size_t hi = lo; int64_t reads = 0;
-			while (hi < so->n_rois && (hi == lo || (reads + so->roi_n_reads[hi] <= 400000 && hi - lo < 20000))) reads += so->roi_n_reads[hi++];
-			idlh_rois *grp = idlh_rois_from_arrays(ref, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, (int64_t)(hi - lo), chrom.data() + lo,
-			                                       so->roi_start + lo, so->roi_end + lo, so->roi_n_reads + lo, so->read_idx + at_idx);
-			if (inflight.size() >= (size_t)(P.n_streams > 0 ? P.n_streams : 1) && !drain()) { idlh_rois_free(grp); break; }
-			uint64_t ticket = 0;
-			r = idl_bam_submit(ctx, bam, hi - lo, chrom.data() + lo, so->roi_start + lo, so->roi_end + lo, so->roi_n_reads + lo, so->read_idx + at_idx, (uint32_t)(n_regions + lo), &ticket);
-			if (r != IDL_OK) { status = die("idl_bam_submit", std::string(idl_strerror(r)) + " " + idl_last_cuda_error(ctx)); idlh_rois_free(grp); break; }
-			inflight.push_back({grp, ticket});
-			at_idx += (size_t)reads; lo = hi;
-		}
-		while (!inflight.empty() && !status) if (!drain()) break;
-		while (!inflight.empty()) { idlh_rois_free(inflight.front().rois); inflight.pop_front(); }
+		status = call_swept(ctx, bam, c, so, 0, ref, all, P, writer, n_regions);
 		n_regions += so->n_rois;
 		idl_sweep_free(so);
 		idl_bam_close(bam);
@@ -335,11 +352,167 @@ static int main_gpu_by_target(const std::string &fa, const std::string &bam_path
 	return status;
 }
 
+// -r / -R: only the regions of interest that overlap the given intervals, decoding only the BAM members that hold them.  Per target the intervals become
+// slices of the file: from the linear-index offset of the 16 kb window in front of an interval to that of the window behind it (idlh_bai_region_run);
+// slices whose member runs overlap or touch are merged and decoded once.  Each slice is decoded (idl_bam_open_slice) and swept over the zone of positions
+// whose evidence it determines exactly (idl_bam_sweep_window, DESIGN.md 4a); when a selected region touches an inner edge of the zone, or the zone does not
+// reach the last interval, the slice grows by one window on that side and is swept again.  A reader thread reads the next slice's members meanwhile.
+static int main_regions(const std::string &fa, const std::string &bam_path, const std::vector<std::string> &regions, const std::string &bed, int min_reads,
+                        int min_ctg_len, int min_event_len, int device)
+{
+	char err[512] = {0};
+	const bool timing = getenv("INDELOPE_TIMING") != nullptr;
+	const double t_begin = now_s();
+	idl_params P;
+	idl_default_params(&P);
+	P.min_reads = min_reads; P.min_ctg_len = min_ctg_len; P.min_event_len = min_event_len;
+	const int32_t min_ev = min_reads - 2 > 3 ? min_reads - 2 : 3;
+	idlh_dataset *ref = idlh_load_targets(fa.c_str(), bam_path.c_str(), err, sizeof err);
+	if (!ref) return die("input", err);
+	idlh_rois *seqs = idlh_rois_from_arrays(ref, 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr);
+	const idlh_roiset *all = idlh_rois_view(seqs);
+	std::vector<const char*> names((size_t)all->n_chroms); std::vector<int64_t> lens((size_t)all->n_chroms);
+	for (int32_t c = 0; c < all->n_chroms; ++c) { names[(size_t)c] = all->chrom_name[c]; lens[(size_t)c] = all->chrom_len[c]; }
+	std::vector<const char*> rv; for (const std::string &r : regions) rv.push_back(r.c_str());
+	idlh_regions *sel = idlh_regions_parse(all->n_chroms, names.data(), lens.data(), (int32_t)rv.size(), rv.data(), bed.empty() ? nullptr : bed.c_str(), err, sizeof err);
+	auto cleanup = [&]() { idlh_regions_free(sel); idlh_rois_free(seqs); idlh_dataset_free(ref); };
+	if (!sel) { cleanup(); return die("regions", err); }
+	{   // the index must be there before anything is printed
+		uint64_t v[5];
+		if (all->n_chroms > 0 && idlh_bai_target_span(bam_path.c_str(), 0, v, v + 1, v + 2, v + 3, v + 4, err, sizeof err) < 0) { cleanup(); return die("input", bam_path + ": " + err); }
+	}
+	idl_ctx *ctx = nullptr;
+	const int create_rc = idl_create(device, &P, &ctx);
+	if (create_rc != IDL_OK) { cleanup(); return die("libindelope_cuda", std::string(idl_strerror(create_rc)) + " (this program has no CPU path; it needs a CUDA device)"); }
+	{ char *h = idlh_vcf_header(all); fputs(h, stdout); idlh_free(h); }   // echo header % [b.contig_header, "sample"], :599
+	int status = 0;
+	idlh_vcf *writer = idlh_vcf_new();
+	size_t n_regions = 0, n_slices = 0, n_retries = 0, n_intervals = 0; uint64_t bytes_read = 0, bytes_decoded = 0;
+	double t_read = 0, t_open = 0, t_sweep = 0, t_call = 0;
+	// one slice: window range [w0, w1], its intervals, where its members lie
+	struct Slice { int64_t w0 = 0, w1 = 0; std::vector<int32_t> beg, end; uint64_t fb = 0, fe = 0, first = 0, em = 0, eo = 0; int64_t zone_lo = 0; int32_t to_end = 1; int rr = 1; };
+	struct Read { uint64_t fb = 0, fe = 0; std::vector<uint8_t> bytes; std::string error; };
+	auto locate = [&](int32_t c, Slice &S) -> bool {
+		S.rr = idlh_bai_region_run(bam_path.c_str(), c, S.w0, S.w1, &S.fb, &S.fe, &S.first, &S.em, &S.eo, &S.zone_lo, &S.to_end, err, sizeof err);
+		if (S.rr < 0) { status = die("input", bam_path + ": " + err); return false; }
+		return true;
+	};
+	auto load = [&](uint64_t fb, uint64_t fe, Read *R) {
+		R->fb = fb; R->fe = fe; R->error.clear(); R->bytes.resize((size_t)(fe - fb));
+		FILE *f = fopen(bam_path.c_str(), "rb");
+		if (!f) { R->error = "cannot open " + bam_path; return; }
+		if (fseek(f, (long)fb, SEEK_SET) != 0 || fread(R->bytes.data(), 1, R->bytes.size(), f) != R->bytes.size()) R->error = "cannot read " + bam_path;
+		fclose(f);
+	};
+	Read ahead; std::thread reader;
+	std::vector<int64_t> ib, ie;
+	for (int32_t c = 0; c < all->n_chroms && !status; ++c) {
+		const int64_t n_iv = idlh_regions_get(sel, c, nullptr, nullptr, 0);
+		if (n_iv == 0) continue;
+		ib.resize((size_t)n_iv); ie.resize((size_t)n_iv);
+		idlh_regions_get(sel, c, ib.data(), ie.data(), n_iv);
+		n_intervals += (size_t)n_iv;
+		int64_t last_end = -1;   // of the last region called on this target
+		// the first slice of every interval: the window holding the position in front of it to the window behind its last base
+		std::deque<Slice> todo;
+		for (int64_t k = 0; k < n_iv && !status; ++k) {
+			Slice S;
+			S.w0 = ib[(size_t)k] > 0 ? (ib[(size_t)k] - 1) >> 14 : 0; S.w1 = ((ie[(size_t)k] - 1) >> 14) + 1;
+			S.beg.push_back((int32_t)ib[(size_t)k]); S.end.push_back((int32_t)ie[(size_t)k]);
+			if (!todo.empty() && S.w0 <= todo.back().w1) {   // overlapping window ranges: one slice
+				Slice &B = todo.back(); B.w1 = std::max(B.w1, S.w1); B.beg.push_back(S.beg[0]); B.end.push_back(S.end[0]);
+			} else todo.push_back(S);
+		}
+		for (Slice &S : todo) if (!locate(c, S)) break;
+		while (!todo.empty() && !status) {
+			Slice S = todo.front(); todo.pop_front();
+			// slices whose member runs overlap or touch are decoded once
+			while (!todo.empty() && S.rr == 0 && todo.front().rr == 0 && todo.front().fb <= S.fe) {
+				const Slice &N = todo.front();
+				S.w1 = std::max(S.w1, N.w1); S.beg.insert(S.beg.end(), N.beg.begin(), N.beg.end()); S.end.insert(S.end.end(), N.end.begin(), N.end.end());
+				todo.pop_front();
+				if (!locate(c, S)) break;
+			}
+			if (status) break;
+			if (S.rr == 1) {   // no record in the run
+				if (S.to_end) continue;                      // ... up to the target's end: no region
+				++S.w1; ++n_retries;
+				if (locate(c, S)) todo.push_front(S);
+				continue;
+			}
+			double t1 = now_s();
+			if (reader.joinable()) reader.join();
+			Read R;
+			if (ahead.fb == S.fb && ahead.fe == S.fe && !ahead.bytes.empty()) R = std::move(ahead); else load(S.fb, S.fe, &R);
+			ahead = Read();
+			if (!todo.empty() && todo.front().rr == 0) reader = std::thread(load, todo.front().fb, todo.front().fe, &ahead);   // the next slice as it stands
+			t_read += now_s() - t1;
+			if (!R.error.empty()) { status = die("input", R.error); break; }
+			bytes_read += R.bytes.size();
+			t1 = now_s();
+			idl_bam_slice sl; memset(&sl, 0, sizeof sl);
+			sl.n_ref = all->n_chroms; sl.ref_name = names.data(); sl.ref_len = lens.data(); sl.first_record = S.first; sl.end_member = S.em; sl.end_offset = S.eo;
+			idl_bam *bam = nullptr; char berr[512] = {0};
+			const int orc = idl_bam_open_slice(device, R.bytes.data(), R.bytes.size(), &sl, &bam, berr, sizeof berr);
+			if (orc != IDL_OK) { status = die("input", bam_path + " (" + names[(size_t)c] + "): " + (berr[0] ? berr : idl_strerror(orc))); break; }
+			const idl_bam_info *info = idl_bam_get_info(bam);
+			bytes_decoded += info->inflated_bytes; ++n_slices;
+			t_open += now_s() - t1; t1 = now_s();
+			// the zone: positions below the start of the slice's last record are exact (every record left out on the right starts there or later)
+			int64_t zone_hi = lens[(size_t)c];
+			if (!S.to_end) {
+				const int64_t last = info->n_records - 1;
+				idl_bam_reads *rd = nullptr;
+				if (last < 0 || idl_bam_fetch(bam, 1, &last, 0, &rd) != IDL_OK) { status = die("idl_bam_fetch", "cannot read the slice's last record"); idl_bam_close(bam); break; }
+				zone_hi = (int64_t)rd->start[0] - 1;
+				idl_bam_reads_free(rd);
+			}
+			if (zone_hi < S.zone_lo || zone_hi < (int64_t)S.end.back() - 1) {   // the zone does not reach the last interval's last base yet
+				idl_bam_close(bam);
+				++S.w1; ++n_retries;
+				if (locate(c, S)) todo.push_front(S);
+				t_sweep += now_s() - t1;
+				continue;
+			}
+			idl_sweep_out *so = nullptr;
+			const int r = idl_bam_sweep_window(bam, c, (int32_t)S.zone_lo, (int32_t)zone_hi, S.beg.size(), S.beg.data(), S.end.data(), min_ev, min_reads, 600, 0, &so);
+			if (r != IDL_OK) { status = die("idl_bam_sweep_window", idl_strerror(r)); idl_bam_close(bam); break; }
+			t_sweep += now_s() - t1; t1 = now_s();
+			if (so->n_edge[0] || so->n_edge[1]) {   // a selected region reaches beyond the zone: grow the slice on that side
+				if (so->n_edge[0]) --S.w0;
+				if (so->n_edge[1]) ++S.w1;
+				++n_retries;
+				idl_sweep_free(so); idl_bam_close(bam);
+				if (locate(c, S)) todo.push_front(S);
+				continue;
+			}
+			// a slice grown to the left may share regions with the slice before it: those were called there
+			size_t first = 0;
+			while (first < so->n_rois && so->roi_start[first] <= last_end) ++first;
+			status = call_swept(ctx, bam, c, so, first, ref, all, P, writer, n_regions);
+			n_regions += so->n_rois - first;
+			if (so->n_rois > first) last_end = so->roi_end[so->n_rois - 1];
+			idl_sweep_free(so);
+			idl_bam_close(bam);
+			t_call += now_s() - t1;
+		}
+	}
+	if (reader.joinable()) reader.join();
+	if (timing)
+		fprintf(stderr, "indelope timing (regions): %zu intervals, %.1f MB read, %.1f MB decoded, slices %zu, retries %zu, regions %zu; waited %.3f s for reads, "
+		        "idl_bam_open_slice %.3f s, zone + idl_bam_sweep_window %.3f s, build + call + vcf %.3f s, total %.3f s\n", n_intervals, bytes_read / 1e6,
+		        bytes_decoded / 1e6, n_slices, n_retries, n_regions, t_read, t_open, t_sweep, t_call, now_s() - t_begin);
+	idlh_vcf_free(writer);
+	idl_destroy(ctx);
+	cleanup();
+	return status;
+}
+
 int main(int argc, char **argv)
 {
 	int min_reads = 3, min_ctg_len = 73, min_event_len = 4, threads = 1, device = 0;
 	bool gpu_sweep = false;
-	std::vector<std::string> pos;
+	std::vector<std::string> pos, regions; std::string bed;
 	for (int i = 1; i < argc; ++i) {
 		const std::string a = argv[i];
 		auto int_opt = [&](const char *s, const char *l, int &dst) -> int { // 0 no match, 1 consumed, -1 error
@@ -355,6 +528,17 @@ int main(int argc, char **argv)
 		if (a == "-h" || a == "--help") { fputs(USAGE, stdout); return 0; }
 		if (a == "--version") { puts("indelope 0.0.1"); return 0; }
 		if (a == "-g" || a == "--gpu-decode" || a == "--gpu-sweep") { gpu_sweep = true; continue; }
+		auto str_opt = [&](const char *s, const char *l, std::string &dst) -> int { // 0 no match, 1 consumed, -1 error
+			if (a == s || a == l) { if (i + 1 >= argc) return -1; dst = argv[++i]; }
+			else if (a.rfind(std::string(l) + "=", 0) == 0) dst = a.substr(strlen(l) + 1);
+			else if (a.size() > 2 && a.compare(0, 2, s) == 0 && a[1] != '-') dst = a.substr(2);
+			else return 0;
+			return dst.empty() ? -1 : 1;
+		};
+		std::string one;
+		int sr;
+		if ((sr = str_opt("-r", "--region", one))) { if (sr < 0) { fputs(USAGE, stderr); return 1; } regions.push_back(one); continue; }
+		if ((sr = str_opt("-R", "--regions-file", bed))) { if (sr < 0) { fputs(USAGE, stderr); return 1; } continue; }
 		int rc;
 		if ((rc = int_opt("-m", "--min-reads", min_reads)) || (rc = int_opt("-c", "--min-contig-len", min_ctg_len)) ||
 		    (rc = int_opt("-e", "--min-event-len", min_event_len)) || (rc = int_opt("-t", "--threads", threads)) || (rc = int_opt("-d", "--device", device))) {
@@ -369,6 +553,7 @@ int main(int argc, char **argv)
 	char err[512] = {0};
 	const bool timing = getenv("INDELOPE_TIMING") != nullptr;
 	const double t_begin = now_s(); double t_sweep = 0, t_pack = 0, t_wait = 0, t_vcf = 0, t0;
+	if (!regions.empty() || !bed.empty()) return main_regions(pos[0], pos[1], regions, bed, min_reads, min_ctg_len, min_event_len, device);   // with or without -g
 	if (gpu_sweep) {
 		// the whole file on the device when it fits (the file and ~5x its size: inflated stream + record arrays), else target by target through the index
 		bool by_target = getenv("INDELOPE_BY_TARGET") != nullptr;

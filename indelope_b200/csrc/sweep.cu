@@ -36,9 +36,11 @@ constexpr int SW_TILE = SW_THREADS * SW_ITEMS;     // elements per CTA
 __device__ __forceinline__ bool sw_skippable(uint16_t f) { return (f & 0x400) || (f & 0x200) || (f & 0x4) || (f & 0x800) || (f & 0x100); } // :40-47
 
 // (A) one thread per record: event intervals into the difference array (event_locations :430-442; every op but M is an event, the
-// ones that do not consume the reference are one base wide), stop of a non-skippable record for the prefix maximum
+// ones that do not consume the reference are one base wide), stop of a non-skippable record for the prefix maximum.  The position arrays cover the
+// zone [zone_lo, zone_hi] only (index = position - zone_lo): a record that starts before the zone or ends behind it is clipped to it before it
+// addresses `diff` -- the usual case for a zone cut out of a target, not an edge case
 __global__ void sw_mark_kernel(size_t n, const int32_t *start, const int32_t *stop, const uint16_t *flag, const uint32_t *cigar, const unsigned long long *cig_off,
-                               int32_t tlen, int *diff, int32_t *stopv)
+                               int32_t zone_lo, int32_t zone_hi, int *diff, int32_t *stopv)
 {
 	const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if (i >= n) return;
@@ -51,8 +53,11 @@ __global__ void sw_mark_kernel(size_t n, const int32_t *start, const int32_t *st
 		const bool cons = op == 0 || op == 2 || op == 3 || op == 7 || op == 8;
 		if (op != 0) {
 			const long long es = s + off; long long ee = cons ? es + len : es + 1;
-			if (ee > (long long)tlen + 1) ee = (long long)tlen + 1;   // evidence has tlen + 1 entries (:522)
-			if (es >= 0 && es < ee) { atomicAdd(diff + es, 1); atomicAdd(diff + ee, -1); }
+			if (ee > (long long)zone_hi + 1) ee = (long long)zone_hi + 1;   // evidence has tlen + 1 entries (:522); the zone ends at zone_hi <= tlen
+			if (es >= 0) {
+				const long long a = es > zone_lo ? es : zone_lo;
+				if (a < ee) { atomicAdd(diff + (a - zone_lo), 1); atomicAdd(diff + (ee - zone_lo), -1); }
+			}
 		}
 		if (cons) off += len;
 	}
@@ -136,8 +141,9 @@ template <bool MAX> __global__ void __launch_bounds__(SW_SCAN_THREADS) sw_scan_t
 }
 
 // (B) apply pass of the prefix maximum over the records: pm[i] = max(stopv[0..i]) and the cuts: a record whose start lies beyond every
-// non-skippable stop before it opens a new chunk (:529), runs of evidence are cut at its start
-__global__ void __launch_bounds__(SW_THREADS) sw_prefmax_apply_kernel(const int32_t *stopv, const int32_t *start, size_t n, const int *totals, int32_t *pm, uint8_t *cut, int32_t tlen)
+// non-skippable stop before it opens a new chunk (:529), runs of evidence are cut at its start (cuts outside the zone are not stored)
+__global__ void __launch_bounds__(SW_THREADS) sw_prefmax_apply_kernel(const int32_t *stopv, const int32_t *start, size_t n, const int *totals, int32_t *pm, uint8_t *cut,
+                                                                      int32_t zone_lo, int32_t zone_hi)
 {
 	__shared__ int sh[SW_THREADS / 32];
 	const size_t base = (size_t)blockIdx.x * SW_TILE + (size_t)threadIdx.x * SW_ITEMS;
@@ -150,7 +156,7 @@ __global__ void __launch_bounds__(SW_THREADS) sw_prefmax_apply_kernel(const int3
 	for (int k = 0; k < SW_ITEMS; ++k) {
 		if (base + k < n) {
 			const int32_t s = start[base + k];
-			if (s > run && s >= 0 && s <= tlen) cut[s] = 1;
+			if (s > run && s >= zone_lo && s <= zone_hi) cut[s - zone_lo] = 1;
 			run = max(run, v[k]);
 			pm[base + k] = run;
 		}
@@ -229,15 +235,34 @@ __global__ void __launch_bounds__(SW_THREADS) sw_runs_kernel(const uint8_t *ev, 
 // (E) one warp per run: the records that overlap it (overlaps :449-452), in order.  Candidates: from the first record whose prefix
 // maximum of stops reaches roi_start (nothing before it can overlap) to the first record that starts beyond roi_end (:485).
 // WRITE = false: count; a run is a region iff min_reads <= count <= max_reads (:486).  WRITE = true: the lists of the regions.
+// Runs are positions relative to zone_lo.  With a selection (sel.n_iv >= 0) only runs that overlap one of the sorted, disjoint intervals
+// [iv_beg, iv_end) are regions, and a selected run that touches an edge of the zone that is not the target's (rs == edge_lo, re == edge_hi) is
+// not one either: it is counted in n_edge[0] / n_edge[1], because evidence beyond the zone may extend it.
+struct SwSelect { int n_iv; const int32_t *iv_beg, *iv_end; int32_t edge_lo, edge_hi; unsigned long long *n_edge; };
 template <bool WRITE>
-__global__ void __launch_bounds__(SW_THREADS) sw_reads_kernel(const int32_t *run_start, const int32_t *run_end, int n_runs, const int32_t *start, const int32_t *stopv,
+__global__ void __launch_bounds__(SW_THREADS) sw_reads_kernel(const int32_t *run_start, const int32_t *run_end, int n_runs, int32_t zone_lo, SwSelect sel,
+                                                              const int32_t *start, const int32_t *stopv,
                                                               const int32_t *pm, size_t n_reads, int min_reads, int max_reads, int *count, const int *slot,
                                                               const int *read_off, int32_t *roi_start, int32_t *roi_end, long long *roi_read_begin,
                                                               int32_t *roi_n_reads, long long *read_idx)
 {
 	const int warp = (int)(((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
 	if (warp >= n_runs) return;
-	const int32_t rs = run_start[warp], re = run_end[warp];
+	const int32_t rs = run_start[warp] + zone_lo, re = run_end[warp] + zone_lo;
+	if (!WRITE && sel.n_iv >= 0) {
+		int a = 0, b = sel.n_iv;                                     // the last interval with iv_beg <= re
+		while (a < b) { const int mid = (a + b) >> 1; if (sel.iv_beg[mid] <= re) a = mid + 1; else b = mid; }
+		const bool picked = a > 0 && sel.iv_end[a - 1] > rs;
+		const bool lo_edge = rs == sel.edge_lo, hi_edge = re == sel.edge_hi;
+		if (!picked || lo_edge || hi_edge) {
+			if (lane == 0) {
+				count[warp] = 0;
+				if (picked && lo_edge) atomicAdd(sel.n_edge, 1ull);
+				if (picked && hi_edge) atomicAdd(sel.n_edge + 1, 1ull);
+			}
+			return;
+		}
+	}
 	size_t lo = 0, hi = n_reads;                                   // first i with pm[i] >= rs
 	while (lo < hi) { const size_t mid = (lo + hi) >> 1; if (pm[mid] >= rs) hi = mid; else lo = mid + 1; }
 	const size_t first = lo;
@@ -318,30 +343,37 @@ void idl_sweep_free(idl_sweep_out *o)
 int idl_sweep(int device, const idl_sweep_in *in, int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out)
 {
 	if (!in || !out) return IDL_E_ARG;
-	return idl_sweep_impl(device, in, false, in->n_reads && in->cig_off ? (size_t)in->cig_off[in->n_reads] : 0, min_event_support, min_read_coverage, max_read_coverage, flags, out);
+	return idl_sweep_impl(device, in, false, in->n_reads && in->cig_off ? (size_t)in->cig_off[in->n_reads] : 0, 0, in->chrom_len, -1, nullptr, nullptr,
+	                      min_event_support, min_read_coverage, max_read_coverage, flags, out);
 }
 
 } // extern "C"
 
 // the body of idl_sweep; with dev_in the arrays of `in` already live on `device` (idl_bam_sweep: records parsed there by bamdev.cu)
-int idl_sweep_impl(int device, const idl_sweep_in *in, bool dev_in, size_t n_cig, int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage,
-                   uint32_t flags, idl_sweep_out **out)
+int idl_sweep_impl(int device, const idl_sweep_in *in, bool dev_in, size_t n_cig, int32_t zone_lo, int32_t zone_hi, long long n_iv, const int32_t *iv_beg,
+                   const int32_t *iv_end, int32_t min_event_support, int32_t min_read_coverage, int32_t max_read_coverage, uint32_t flags, idl_sweep_out **out)
 {
 	if (!in || !out || in->chrom_len < 0 || (in->n_reads && (!in->start || !in->stop || !in->flag || !in->cigar || !in->cig_off))) return IDL_E_ARG;
 	*out = nullptr;
 	if (min_read_coverage < 1 || max_read_coverage < min_read_coverage || min_event_support < 1 || min_event_support > 255) return IDL_E_ARG;
+	if (zone_lo < 0 || zone_hi < zone_lo || zone_hi > in->chrom_len) return IDL_E_ARG;
+	if (n_iv > 0 && (!iv_beg || !iv_end)) return IDL_E_ARG;
+	if (n_iv >= (1ll << 31)) return IDL_E_CAPACITY;
+	for (long long k = 0; k < n_iv; ++k)   // sorted and disjoint: the device finds a run's interval by one binary search
+		if (iv_beg[k] >= iv_end[k] || (k && iv_beg[k] < iv_end[k - 1])) return IDL_E_ARG;
 	int ndev = 0;
 	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return IDL_E_NO_DEVICE;
 	if (device < 0 || device >= ndev) return IDL_E_ARG;
 	if (in->n_reads >= (1ull << 31) || (size_t)in->chrom_len + 2 >= (1ull << 31)) return IDL_E_CAPACITY;
 	if (cudaSetDevice(device) != cudaSuccess) return IDL_E_CUDA;
-	const size_t n = in->n_reads, np = (size_t)in->chrom_len + 2;          // evidence positions 0 .. chrom_len, one more for the closing -1
+	const size_t n = in->n_reads, np = (size_t)(zone_hi - zone_lo) + 2;   // evidence positions zone_lo .. zone_hi (0 .. chrom_len), one more for the closing -1
 	const size_t npad = tiles(np) * SW_TILE, nrpad = std::max<size_t>(1, tiles(n)) * SW_TILE;
 	idl_sweep_out *o = (idl_sweep_out*)calloc(1, sizeof *o);
 	if (!o) return IDL_E_NOMEM;
 	cudaStream_t st = nullptr; cudaEvent_t ev[4] = {};
-	Dev d_start, d_stop, d_flag, d_cig, d_coff, d_diff, d_stopv, d_pm, d_cut, d_ev, d_tot, d_tot2, d_grand, d_rs, d_re, d_count, d_slot, d_roff, d_o1, d_o2, d_o3, d_o4, d_o5;
+	Dev d_start, d_stop, d_flag, d_cig, d_coff, d_diff, d_stopv, d_pm, d_cut, d_ev, d_tot, d_tot2, d_grand, d_rs, d_re, d_count, d_slot, d_roff, d_o1, d_o2, d_o3, d_o4, d_o5, d_iv, d_edge;
 	int rc = IDL_OK;
+	SwSelect sel = {-1, nullptr, nullptr, INT_MIN, INT_MAX, nullptr};
 #define SWCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { fprintf(stderr, "idl_sweep: %s: %s\n", #call, cudaGetErrorString(e_)); rc = IDL_E_CUDA; goto done; } } while (0)
 	{
 		SWCK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
@@ -354,6 +386,13 @@ int idl_sweep_impl(int device, const idl_sweep_in *in, bool dev_in, size_t n_cig
 		SWCK(d_diff.get(npad * 4, st)); SWCK(d_stopv.get(nrpad * 4, st)); SWCK(d_pm.get(nrpad * 4, st)); SWCK(d_cut.get(npad + 16, st)); SWCK(d_ev.get(npad + 16, st));
 		const size_t ntp = tiles(np), ntr = std::max<size_t>(1, tiles(n));
 		SWCK(d_tot.get(std::max(ntp, ntr) * 4, st)); SWCK(d_tot2.get(std::max(ntp, ntr) * 4, st)); SWCK(d_grand.get(16, st));
+		if (n_iv >= 0) {
+			SWCK(d_iv.get((size_t)n_iv * 8 + 16, st)); SWCK(d_edge.get(16, st));
+			sel.n_iv = (int)n_iv; sel.iv_beg = d_iv.as<int32_t>(); sel.iv_end = d_iv.as<int32_t>() + n_iv; sel.n_edge = d_edge.as<unsigned long long>();
+			sel.edge_lo = zone_lo > 0 ? zone_lo : INT_MIN; sel.edge_hi = zone_hi < in->chrom_len ? zone_hi : INT_MAX;
+			if (n_iv) { SWCK(cudaMemcpyAsync(d_iv.p, iv_beg, (size_t)n_iv * 4, cudaMemcpyHostToDevice, st)); SWCK(cudaMemcpyAsync(d_iv.as<int32_t>() + n_iv, iv_end, (size_t)n_iv * 4, cudaMemcpyHostToDevice, st)); }
+			SWCK(cudaMemsetAsync(d_edge.p, 0, 16, st));
+		}
 		SWCK(cudaEventRecord(ev[0], st));
 		if (n && !dev_in) {
 			SWCK(cudaMemcpyAsync(d_start.p, in->start, n * 4, cudaMemcpyHostToDevice, st)); SWCK(cudaMemcpyAsync(d_stop.p, in->stop, n * 4, cudaMemcpyHostToDevice, st));
@@ -369,11 +408,11 @@ int idl_sweep_impl(int device, const idl_sweep_in *in, bool dev_in, size_t n_cig
 		int n_runs = 0, n_runs_e = 0;
 		if (n) {
 			sw_mark_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, p_start, p_stop, p_flag, p_cig,
-			                                                           p_coff, in->chrom_len, d_diff.as<int>(), d_stopv.as<int32_t>());
+			                                                           p_coff, zone_lo, zone_hi, d_diff.as<int>(), d_stopv.as<int32_t>());
 			// (B) prefix maximum of the stops, cuts
 			sw_totals_kernel<true><<<(unsigned)ntr, SW_THREADS, 0, st>>>(d_stopv.as<int>(), n, d_tot.as<int>());
 			sw_scan_totals_kernel<true><<<1, SW_SCAN_THREADS, 0, st>>>(d_tot.as<int>(), ntr, nullptr);
-			sw_prefmax_apply_kernel<<<(unsigned)ntr, SW_THREADS, 0, st>>>(d_stopv.as<int32_t>(), p_start, n, d_tot.as<int>(), d_pm.as<int32_t>(), d_cut.as<uint8_t>(), in->chrom_len);
+			sw_prefmax_apply_kernel<<<(unsigned)ntr, SW_THREADS, 0, st>>>(d_stopv.as<int32_t>(), p_start, n, d_tot.as<int>(), d_pm.as<int32_t>(), d_cut.as<uint8_t>(), zone_lo, zone_hi);
 		}
 		// (C) evidence bytes
 		sw_totals_kernel<false><<<(unsigned)ntp, SW_THREADS, 0, st>>>(d_diff.as<int>(), np, d_tot.as<int>());
@@ -398,7 +437,7 @@ int idl_sweep_impl(int device, const idl_sweep_in *in, bool dev_in, size_t n_cig
 			                                                          d_rs.as<int32_t>(), d_re.as<int32_t>());
 			// (E) records of every run: count, accept, scan, write
 			const unsigned wb = (unsigned)(((size_t)n_runs * 32 + SW_THREADS - 1) / SW_THREADS);
-			sw_reads_kernel<false><<<wb, SW_THREADS, 0, st>>>(d_rs.as<int32_t>(), d_re.as<int32_t>(), n_runs, p_start, d_stopv.as<int32_t>(), d_pm.as<int32_t>(), n,
+			sw_reads_kernel<false><<<wb, SW_THREADS, 0, st>>>(d_rs.as<int32_t>(), d_re.as<int32_t>(), n_runs, zone_lo, sel, p_start, d_stopv.as<int32_t>(), d_pm.as<int32_t>(), n,
 			                                                 min_read_coverage, max_read_coverage, d_count.as<int>(), nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
 			sw_accept_kernel<<<(unsigned)((n_runs + 255) / 256), 256, 0, st>>>(d_count.as<int>(), n_runs, d_slot.as<int>(), d_roff.as<int>());
 			exclusive_sum(d_slot.as<int>(), (size_t)n_runs, d_tot.as<int>(), d_grand.as<int>() + 2, st);
@@ -411,7 +450,7 @@ int idl_sweep_impl(int device, const idl_sweep_in *in, bool dev_in, size_t n_cig
 			SWCK(d_o1.get((size_t)n_rois * 4 + 16, st)); SWCK(d_o2.get((size_t)n_rois * 4 + 16, st)); SWCK(d_o3.get((size_t)n_rois * 8 + 16, st)); SWCK(d_o4.get((size_t)n_rois * 4 + 16, st));
 			SWCK(d_o5.get((size_t)n_idx * 8 + 16, st));
 			if (n_rois)
-				sw_reads_kernel<true><<<wb, SW_THREADS, 0, st>>>(d_rs.as<int32_t>(), d_re.as<int32_t>(), n_runs, p_start, d_stopv.as<int32_t>(), d_pm.as<int32_t>(), n,
+				sw_reads_kernel<true><<<wb, SW_THREADS, 0, st>>>(d_rs.as<int32_t>(), d_re.as<int32_t>(), n_runs, zone_lo, sel, p_start, d_stopv.as<int32_t>(), d_pm.as<int32_t>(), n,
 				                                                min_read_coverage, max_read_coverage, d_count.as<int>(), d_slot.as<int>(), d_roff.as<int>(), d_o1.as<int32_t>(),
 				                                                d_o2.as<int32_t>(), d_o3.as<long long>(), d_o4.as<int32_t>(), d_o5.as<long long>());
 		}
@@ -435,6 +474,11 @@ int idl_sweep_impl(int device, const idl_sweep_in *in, bool dev_in, size_t n_cig
 		}
 		SWCK(cudaEventRecord(ev[3], st));
 		SWCK(cudaStreamSynchronize(st));
+		if (sel.n_edge) {
+			unsigned long long e2[2] = {0, 0};
+			SWCK(cudaMemcpy(e2, d_edge.p, 16, cudaMemcpyDeviceToHost));
+			o->n_edge[0] = (size_t)e2[0]; o->n_edge[1] = (size_t)e2[1];
+		}
 		cudaEventElapsedTime(&o->ms_h2d, ev[0], ev[1]); cudaEventElapsedTime(&o->ms_kernels, ev[1], ev[2]); cudaEventElapsedTime(&o->ms_d2h, ev[2], ev[3]);
 		// algorithmic bytes: every record once (start, stop, flag, CIGAR), every position's evidence byte written and read once, the results
 		o->algorithmic_bytes = (uint64_t)n * 10 + (uint64_t)n_cig * 4 + (uint64_t)np * 2 + (uint64_t)n_rois * 20 + (uint64_t)n_idx * 8;
@@ -444,7 +488,7 @@ int idl_sweep_impl(int device, const idl_sweep_in *in, bool dev_in, size_t n_cig
 	}
 done:
 	for (Dev *d : {&d_start, &d_stop, &d_flag, &d_cig, &d_coff, &d_diff, &d_stopv, &d_pm, &d_cut, &d_ev, &d_tot, &d_tot2, &d_grand, &d_rs, &d_re, &d_count, &d_slot, &d_roff,
-	               &d_o1, &d_o2, &d_o3, &d_o4, &d_o5})
+	               &d_o1, &d_o2, &d_o3, &d_o4, &d_o5, &d_iv, &d_edge})
 		if (d->p) { cudaFreeAsync(d->p, st); d->p = nullptr; }
 	for (auto &e : ev) if (e) cudaEventDestroy(e);
 	if (st) { cudaStreamSynchronize(st); cudaStreamDestroy(st); }

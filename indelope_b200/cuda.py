@@ -47,7 +47,7 @@ def lib():
 
 EXPORTS = ("idl_default_params idl_create idl_destroy idl_batch_alloc idl_batch_free idl_submit idl_upload idl_run_resident idl_wait "
            "idl_release idl_strerror idl_last_cuda_error idl_device_count idl_ksw2_batch idl_sweep idl_sweep_free "
-           "idl_bam_open idl_bam_get_info idl_bam_close idl_bam_sweep idl_bam_fetch idl_bam_reads_free idl_bam_set_reference idl_bam_submit idl_bam_pack idl_bam_open_slice idl_device_memory").split()
+           "idl_bam_open idl_bam_get_info idl_bam_close idl_bam_sweep idl_bam_fetch idl_bam_reads_free idl_bam_set_reference idl_bam_submit idl_bam_pack idl_bam_open_slice idl_device_memory idl_bam_sweep_window").split()
 
 
 class SweepIn(C.Structure):
@@ -59,7 +59,7 @@ class SweepOut(C.Structure):
     _fields_ = [("n_rois", C.c_size_t), ("roi_start", C.POINTER(C.c_int32)), ("roi_end", C.POINTER(C.c_int32)), ("roi_read_begin", C.POINTER(C.c_int64)),
                 ("roi_n_reads", C.POINTER(C.c_int32)), ("n_read_idx", C.c_size_t), ("read_idx", C.POINTER(C.c_int64)), ("n_runs", C.c_size_t),
                 ("n_evidence", C.c_size_t), ("evidence", u8p), ("ms_h2d", C.c_float), ("ms_kernels", C.c_float), ("ms_d2h", C.c_float),
-                ("algorithmic_bytes", C.c_uint64), ("streamed_bytes", C.c_uint64)]
+                ("algorithmic_bytes", C.c_uint64), ("streamed_bytes", C.c_uint64), ("n_edge", C.c_size_t * 2)]
 
 
 def sweep(chrom_len, start, stop, flag, cigar, cig_off, min_event_support=3, min_read_coverage=3, max_read_coverage=600, evidence=False, device=0):
@@ -85,7 +85,7 @@ def _sweep_out(L, out, evidence=False):
     r = dict(roi_start=arr(o.roi_start, o.n_rois, np.int32), roi_end=arr(o.roi_end, o.n_rois, np.int32), roi_read_begin=arr(o.roi_read_begin, o.n_rois, np.int64),
              roi_n_reads=arr(o.roi_n_reads, o.n_rois, np.int32), read_idx=arr(o.read_idx, o.n_read_idx, np.int64), n_runs=int(o.n_runs),
              evidence=arr(o.evidence, o.n_evidence, np.uint8) if evidence else None, ms_h2d=o.ms_h2d, ms_kernels=o.ms_kernels, ms_d2h=o.ms_d2h,
-             algorithmic_bytes=int(o.algorithmic_bytes), streamed_bytes=int(o.streamed_bytes))
+             algorithmic_bytes=int(o.algorithmic_bytes), streamed_bytes=int(o.streamed_bytes), n_edge=(int(o.n_edge[0]), int(o.n_edge[1])))
     L.idl_sweep_free(out)
     return r
 
@@ -154,6 +154,21 @@ class Bam:
         rc = L.idl_bam_sweep(self.h, target, min_event_support, min_read_coverage, max_read_coverage, 1 if evidence else 0, C.byref(out))
         if rc != 0:
             raise IdlError("idl_bam_sweep: %s" % L.idl_strerror(rc).decode())
+        return _sweep_out(L, out, evidence)
+
+    def sweep_window(self, target, zone_lo, zone_hi, iv_beg, iv_end, min_event_support=3, min_read_coverage=3, max_read_coverage=600, evidence=False):
+        """idl_bam_sweep_window: the regions of positions zone_lo .. zone_hi that overlap one of the sorted, disjoint intervals [iv_beg[k], iv_end[k]) and lie
+        strictly inside the zone's inner edges; n_edge = (selected runs touching zone_lo, touching zone_hi), left out"""
+        L = lib()
+        i32 = C.POINTER(C.c_int32)
+        L.idl_bam_sweep_window.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_size_t, i32, i32, C.c_int32, C.c_int32, C.c_int32, C.c_uint32,
+                                           C.POINTER(C.POINTER(SweepOut))]
+        b = np.ascontiguousarray(iv_beg, dtype=np.int32); e = np.ascontiguousarray(iv_end, dtype=np.int32)
+        out = C.POINTER(SweepOut)()
+        rc = L.idl_bam_sweep_window(self.h, target, int(zone_lo), int(zone_hi), len(b), b.ctypes.data_as(i32), e.ctypes.data_as(i32), min_event_support,
+                                    min_read_coverage, max_read_coverage, 1 if evidence else 0, C.byref(out))
+        if rc != 0:
+            raise IdlError("idl_bam_sweep_window: %s" % L.idl_strerror(rc).decode())
         return _sweep_out(L, out, evidence)
 
     def fetch(self, idx=None, what=BAM_SEQ | BAM_CIGAR):

@@ -385,6 +385,52 @@ def bai_target_span(bam, target):
     return dict(zip(("file_begin", "file_end", "first_record", "end_member", "end_offset"), (int(x.value) for x in v)))
 
 
+def bai_region_run(bam, target, w0, w1):
+    """idlh_bai_region_run: the records of `target` from the first record of 16 kb window w0 to the first record of window w1 + 1 (or to the target's end):
+    dict(file_begin, file_end, first_record, end_member, end_offset, zone_lo, to_end) with empty=True when the run holds no record"""
+    L = lib()
+    v = [C.c_uint64() for _ in range(5)]
+    zl, te = C.c_int64(), C.c_int32()
+    err = C.create_string_buffer(512)
+    L.idlh_bai_region_run.argtypes = [C.c_char_p, C.c_int32, C.c_int64, C.c_int64] + [C.POINTER(C.c_uint64)] * 5 + [C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.c_char_p, C.c_size_t]
+    rc = L.idlh_bai_region_run(str(bam).encode(), target, w0, w1, *[C.byref(x) for x in v], C.byref(zl), C.byref(te), err, 512)
+    if rc < 0:
+        raise IOError(err.value.decode())
+    out = dict(zip(("file_begin", "file_end", "first_record", "end_member", "end_offset"), (int(x.value) for x in v)))
+    out.update(zone_lo=int(zl.value), to_end=bool(te.value), empty=rc == 1)
+    return out
+
+
+def parse_regions(ref_names, ref_len, regions=(), bed=None):
+    """idlh_regions_parse: `-r` strings (chr[:beg[-end]], 1-based, inclusive) and a `-R` BED file (0-based, half open) -> one list of sorted, merged half-open
+    (beg, end) intervals per target of the header.  ValueError with the reason for a malformed string, a bad BED line or a target not in the header."""
+    L = lib()
+    L.idlh_regions_parse.restype = C.c_void_p
+    L.idlh_regions_parse.argtypes = [C.c_int32, C.POINTER(C.c_char_p), C.POINTER(C.c_int64), C.c_int32, C.POINTER(C.c_char_p), C.c_char_p, C.c_char_p, C.c_size_t]
+    L.idlh_regions_get.restype = C.c_int64
+    L.idlh_regions_get.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_int64]
+    L.idlh_regions_free.argtypes = [C.c_void_p]
+    n = len(ref_names)
+    names = (C.c_char_p * max(n, 1))(*[x.encode() for x in ref_names])
+    lens = (C.c_int64 * max(n, 1))(*[int(x) for x in ref_len])
+    regions = list(regions or [])
+    rv = (C.c_char_p * max(len(regions), 1))(*[str(x).encode() for x in regions])
+    err = C.create_string_buffer(512)
+    h = L.idlh_regions_parse(n, names, lens, len(regions), rv, str(bed).encode() if bed else None, err, 512)
+    if not h:
+        raise ValueError(err.value.decode())
+    try:
+        out = []
+        for c in range(n):
+            k = L.idlh_regions_get(h, c, None, None, 0)
+            b, e = (C.c_int64 * max(k, 1))(), (C.c_int64 * max(k, 1))()
+            L.idlh_regions_get(h, c, b, e, k)
+            out.append([(int(b[i]), int(e[i])) for i in range(k)])
+        return out
+    finally:
+        L.idlh_regions_free(h)
+
+
 def set_threads(n):
     """host threads of idlh_pack / idlh_pack_size (0 = $IDLH_THREADS, else every core up to 32)"""
     lib().idlh_set_threads(int(n))
