@@ -26,6 +26,7 @@
 // walked as ksw_backtrack (:47-79) through a 32 x 32 shared-memory tile, like the column-owned variant.
 #pragma once
 #include "ksw2.cuh"
+#include "ksw2_rows_sched.cuh"
 
 // reads of up to 32 W bases: W = 5 covers 160 bp and fits 80 registers (three CTAs per SM); 0 = not served by this variant
 // (W = 8 works -- the tests ran it -- but needs 128 registers; longer reads take the column-owned variant)
@@ -91,9 +92,8 @@ __device__ __forceinline__ void ksw_rows_word(const KswParams &P, uint32_t m, ui
 	x = xn; v = vn; u = un; y = yn;
 }
 
-// per-diagonal values shared by the slots of a thread.  onm / pm: bit s = slot s of this thread has a lane inside the target /
-// has lanes outside it as well; uon / upm: the same OR-ed over the warp (uniform: they steer the branches).
-struct KswRowsDiag { int lo0, tlen, gl, srcl, tsh; unsigned onm, uon, upm; uint32_t bconst, taddr; uint8_t *prow; };
+// per-diagonal values shared by the slots of a thread (lq: qlen, 0 for a group without a live alignment)
+struct KswRowsDiag { KswRowsAt at; int r, lq, tlen, gl, srcl, tsh; uint32_t bconst, taddr; uint8_t *prow; };
 
 // The slots of one diagonal, unrolled by template recursion: every index into the register arrays is a compile-time
 // constant from the start (a `#pragma unroll` loop around warp votes and shuffles is unrolled too late for the arrays to
@@ -103,26 +103,26 @@ struct KswRowsSlots {
 	static __device__ __forceinline__ void run(const KswParams &P, const KswRowsDiag &dg, const uint32_t (&C)[W], const uint32_t (&qw)[W], uint32_t (&x)[W], uint32_t (&v)[W],
 	                                           uint32_t (&u)[W], uint32_t (&y)[W], uint32_t (&gx)[W], uint32_t (&gy)[W], uint32_t &dm2, uint32_t &chk)
 	{
-		if (dg.uon & (1u << S)) {
-			const bool on = (dg.onm & (1u << S)) != 0u;
+		if (ksw_rows_live(dg.at, S)) {
 			uint32_t send = C[S];
 			if (S > 0 && dg.gl == 7) send = C[S > 0 ? S - 1 : 0];
 			uint32_t pc = __shfl_sync(FULL_MASK, send, dg.srcl);
 			if (S == 0 && dg.gl == 0) pc = dg.bconst;
-			if (dg.upm & (1u << S)) {
-				// the slot holds a word with lanes in front of t = 0 (the word of row r) or past t = tlen-1 (the word of row
-				// r - tlen): those lanes keep a fixed in-range state and stay out of the maximum
-				if (on) {
-					const int lo = dg.lo0 - 32 * S; // t of row 4w on this diagonal; lane c is row 4w + c at t = lo - c
-					uint32_t m = lo >= 3 ? 0xffffffffu : (lo < 0 ? 0u : (0xffffffffu >> (8 * (3 - lo)))); // a word wholly in front of t = 0 is parked as a whole
-					const int cf = lo - (dg.tlen - 1);
-					if (cf > 0) m = cf > 3 ? 0u : (m & (0xffffffffu << (8 * cf)));                            // ... and so is one wholly past the end
-					const uint32_t tw = __funnelshift_r(lds32(dg.taddr + 32 * S), lds32(dg.taddr + 32 * S + 4), dg.tsh); // target codes met by rows 4w .. 4w+3
-					ksw_rows_word<true, WILD>(P, m, pc, tw, qw[S], x[S], v[S], u[S], y[S], gx[S], gy[S], dm2, chk, (uint32_t*)(dg.prow + 32 * S));
-				}
-			} else if (on) {
-				const uint32_t tw = __funnelshift_r(lds32(dg.taddr + 32 * S), lds32(dg.taddr + 32 * S + 4), dg.tsh);
+			if (ksw_rows_interior(dg.at, S)) {
+				// every thread of the warp has all four lanes of the slot inside the target
+				const uint32_t tw = __funnelshift_r(lds32(dg.taddr + 32 * S), lds32(dg.taddr + 32 * S + 4), dg.tsh); // target codes met by rows 4w .. 4w+3
 				ksw_rows_word<false, WILD>(P, 0u, pc, tw, qw[S], x[S], v[S], u[S], y[S], gx[S], gy[S], dm2, chk, (uint32_t*)(dg.prow + 32 * S));
+			} else if (ksw_rows_lane_on(dg.r, dg.gl, S, dg.lq, dg.tlen)) {
+				// the ramps: the word may hold lanes in front of t = 0 (the word of row r) or past t = tlen-1 (the word of row
+				// r - tlen); those lanes keep a fixed in-range state and stay out of the maximum.  A word wholly inside the target
+				// gets m = all ones here, which makes the masked word the plain one: where groups of different shapes overlap it
+				// costs the few mask instructions, never a different result
+				const int lo = dg.r - 4 * dg.gl - 32 * S; // t of row 4w on this diagonal; lane c is row 4w + c at t = lo - c
+				uint32_t m = lo >= 3 ? 0xffffffffu : (lo < 0 ? 0u : (0xffffffffu >> (8 * (3 - lo)))); // a word wholly in front of t = 0 is parked as a whole
+				const int cf = lo - (dg.tlen - 1);
+				if (cf > 0) m = cf > 3 ? 0u : (m & (0xffffffffu << (8 * cf)));                            // ... and so is one wholly past the end
+				const uint32_t tw = __funnelshift_r(lds32(dg.taddr + 32 * S), lds32(dg.taddr + 32 * S + 4), dg.tsh);
+				ksw_rows_word<true, WILD>(P, m, pc, tw, qw[S], x[S], v[S], u[S], y[S], gx[S], gy[S], dm2, chk, (uint32_t*)(dg.prow + 32 * S));
 			}
 		}
 		KswRowsSlots<W, S + 1, WILD>::run(P, dg, C, qw, x, v, u, y, gx, gy, dm2, chk);
@@ -193,9 +193,21 @@ __device__ void ksw2_rows(bool valid, int qlen, const KswQuery query, int tlen, 
 	const bool wild_any = __any_sync(FULL_MASK, wild); // a code 4 anywhere in the four alignments: the scores take the wildcard mask
 	__syncwarp();
 
-	// slots that hold query rows: the same for every thread of the group -- in the last one some threads hold only padding rows (code 6: real
-	// cells of the query-extended problem that can only lose score), so that the eight threads always store a whole 32-byte sector
-	const int nsq = live ? (qlen + 31) >> 5 : 0;
+	// Which diagonals run which slot, and how (ksw2_rows_sched.cuh).  The slots that hold query rows are the same for every thread of a
+	// group -- in the last one some threads hold only padding rows (code 6: real cells of the query-extended problem that can only lose
+	// score), so that the eight threads always store a whole 32-byte sector.  Per slot and diagonal, three cases, all decided by values
+	// the same in every thread of the warp: outside the live window the slot is skipped; inside the interior window every thread runs
+	// its word without masks or tests; in between (the ramps) each thread tests its own word and masks the lanes outside the target.
+	// A group without a live alignment (valid == false, or an early KSW_ST_* status) counts as qlen = tlen = 0, which empties the
+	// interior window of the whole warp: its threads only ever see the ramp path, fail the lane test there (qlen = 0), and so never form
+	// a target address or a backtrack-matrix address, exactly as before.  At call-site B such a warp is mostly the last, partly filled one
+	// of a launch, or one holding tasks with qlen or tlen 0 (al_kernel clamps a negative tlen to 0): those have no diagonals and get the
+	// sort keys 0..15, below every task that has one, so they fill warps of their own, and at most one warp per launch mixes them with
+	// live alignments.
+	const int lq = live ? qlen : 0;
+	KswRowsWarp ws;
+	ws.qmin = __reduce_min_sync(FULL_MASK, lq); ws.qmax = __reduce_max_sync(FULL_MASK, lq);
+	ws.tmin = __reduce_min_sync(FULL_MASK, live ? tlen : 0); ws.tmax = __reduce_max_sync(FULL_MASK, live ? tlen : 0);
 	// score snapshots of this thread (taken when its best score rises): the last bytes of the group's region, 16 bytes per
 	// thread and vector, so that a group's store is one conflict-free 128-byte line; only the owner ever reads them back
 	constexpr int NSV = (2 * W + 3) / 4;
@@ -213,7 +225,6 @@ __device__ void ksw2_rows(bool valid, int qlen, const KswQuery query, int tlen, 
 	const int nr_all = (int)__reduce_max_sync(FULL_MASK, (unsigned)nr); // the warp runs until its longest alignment ends
 	for (int r = 0; r < nr_all; ++r, prow += PITCH) {
 		const bool act = r < nr;
-		const int lo0 = r - 4 * gl;                // t of row 4w on this diagonal is lo0 - 32 s
 		const int tbase = tb - r;
 		const uint32_t taddr = tw_sh + (uint32_t)(tbase & ~3);
 		const int tsh = 8 * (tbase & 3);
@@ -222,21 +233,9 @@ __device__ void ksw2_rows(bool valid, int qlen, const KswQuery query, int tlen, 
 		for (int s = 0; s < W; ++s) C[s] = prmt(u[s], y[s], 0x7300); // byte 2 = u of my top lane, byte 3 = y of it
 		const uint32_t bconst = r ? ((uint32_t)(P.q & 0xff) << 16) : 0u; // :212  u[r] = q (0 on diagonal 0), y[r] = 0
 		uint32_t dm2 = 0;
+		// only threads with a live word run a slot: whole sectors on the band's ramps cut DRAM fill reads but cost 1.2 ms (DESIGN.md 4.2c)
 		KswRowsDiag dg;
-		{
-			// my slots with a lane inside the target: t of the first row of slot s is lo0 - 32 s, wanted in [0, tlen + 2]
-			int s_hi = lo0 >> 5, s_lo = (lo0 - tlen + 29) >> 5;
-			s_hi = s_hi < nsq ? s_hi : nsq - 1; s_lo = s_lo > 0 ? s_lo : 0;
-			unsigned onm = 0, pm = 0;
-			if (act && s_hi >= s_lo) {
-				onm = ((2u << s_hi) - 1u) & ~((1u << s_lo) - 1u);
-				if (lo0 - 32 * s_hi < 3) pm = 1u << s_hi;          // the word of row r: lanes in front of t = 0
-				if (lo0 - 32 * s_lo > tlen - 1) pm |= 1u << s_lo;  // the word of row r - tlen: lanes past the target end
-			}
-			// only threads with a live word run a slot: whole sectors on the band's ramps cut DRAM fill reads but cost 1.2 ms (DESIGN.md 4.2c)
-			dg.onm = onm; dg.uon = __reduce_or_sync(FULL_MASK, onm); dg.upm = __reduce_or_sync(FULL_MASK, pm);
-		}
-		dg.lo0 = lo0; dg.tlen = tlen; dg.gl = gl; dg.srcl = srcl; dg.bconst = bconst; dg.taddr = taddr; dg.tsh = tsh; dg.prow = prow;
+		dg.at = ksw_rows_at(ws, r); dg.r = r; dg.lq = lq; dg.tlen = tlen; dg.gl = gl; dg.srcl = srcl; dg.bconst = bconst; dg.taddr = taddr; dg.tsh = tsh; dg.prow = prow;
 		if (wild_any) KswRowsSlots<W, 0, true>::run(P, dg, C, qw, x, v, u, y, gx, gy, dm2, chk);
 		else KswRowsSlots<W, 0, false>::run(P, dg, C, qw, x, v, u, y, gx, gy, dm2, chk);
 		const int goff = qe * (r + 1) + gbias;
