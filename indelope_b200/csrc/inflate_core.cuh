@@ -35,7 +35,7 @@ enum {
 	INF_OK = 0,
 	INF_E_BTYPE = 1,      // reserved block type
 	INF_E_STORED = 2,     // LEN / NLEN mismatch
-	INF_E_CODE = 3,       // over-subscribed or unusable Huffman code, bad repeat in the code lengths
+	INF_E_CODE = 3,       // over-subscribed or incomplete Huffman code, bad repeat in the code lengths
 	INF_E_SYMBOL = 4,     // a bit pattern no code word of the table matches, or length/distance symbol out of range
 	INF_E_DISTANCE = 5,   // distance beyond the start of the member (BGZF members carry no preset window)
 	INF_E_OUTPUT = 6,     // more (or fewer) bytes than ISIZE says
@@ -80,26 +80,42 @@ IDL_INF_FN uint32_t make_entry(int alphabet, int sym, int l)
 	return (uint32_t)K_BAD << 8 | (uint32_t)l;
 }
 
-// ---- bit reader over 32-bit little-endian words (the compressed buffer is padded: the reader looks up to 64 words ahead) ----
+// ---- bit reader over 32-bit little-endian words ----
 // On the device the next 32 words live one per lane (`win`), the 32 after them are already on their way (`win_next`): a refill is a
 // shuffle, and the latency of global memory is paid once per 128 bytes, a window ahead of where the decoder reads.
+// No load reaches past the last word that holds a byte of the stream (`wend`): the window loads behind it are not made, and the reader
+// takes zero words there.  A stream that needs those bits fails the block-end check (bits_overrun), the ISIZE bound or a symbol check; a
+// block without an end-of-block that ran off the member used to read on until its output reached ISIZE, up to ~120 KB behind the file.
+// IDL_INF_LOOKAHEAD (tests only): the one-lane build keeps the same 2 x 32-word window and makes the device's loads, so that a checked
+// build sees exactly the addresses the warp touches.
+#ifndef IDL_INF_LOOKAHEAD
+#define IDL_INF_LOOKAHEAD 0
+#endif
 struct Bits {
 	const uint32_t *w;      // word 0 = the aligned word that holds the first byte of the stream
 	uint32_t wi;            // next word to take
 	uint64_t bb; int bc;    // bit buffer: bc valid bits, the next bit of the stream is bit 0
 	uint32_t skip, len_byte;   // bytes of word 0 in front of the stream, length of the stream
+	uint32_t wend;          // words w[0 .. wend) hold the stream; nothing behind them is loaded
 #ifdef __CUDACC__
 	uint32_t win, win_next; // win = w[(wi & ~31) + lane], win_next = the 32 words after those
+#elif IDL_INF_LOOKAHEAD
+	uint32_t win[32], win_next[32];
 #endif
 };
+IDL_INF_FN uint32_t bits_load(const Bits &B, uint32_t i) { return i < B.wend ? B.w[i] : 0u; }
 IDL_INF_FN uint32_t bits_next_word(Bits &B)
 {
 #ifdef __CUDACC__
 	const uint32_t v = __shfl_sync(0xffffffffu, B.win, (int)(B.wi & 31u));
-	if ((++B.wi & 31u) == 0) { B.win = B.win_next; B.win_next = B.w[B.wi + 32u + (threadIdx.x & 31u)]; }
+	if ((++B.wi & 31u) == 0) { B.win = B.win_next; B.win_next = bits_load(B, B.wi + 32u + (threadIdx.x & 31u)); }
+	return v;
+#elif IDL_INF_LOOKAHEAD
+	const uint32_t v = B.win[B.wi & 31u];
+	if ((++B.wi & 31u) == 0) for (uint32_t l = 0; l < 32; ++l) { B.win[l] = B.win_next[l]; B.win_next[l] = bits_load(B, B.wi + 32u + l); }
 	return v;
 #else
-	return B.w[B.wi++];
+	return bits_load(B, B.wi++);
 #endif
 }
 IDL_INF_FN void bits_open(Bits &B, const uint8_t *base, size_t off, size_t len)
@@ -107,8 +123,11 @@ IDL_INF_FN void bits_open(Bits &B, const uint8_t *base, size_t off, size_t len)
 	const size_t a = off + ((uintptr_t)base & 3);
 	B.w = (const uint32_t*)(base - ((uintptr_t)base & 3)) + (a >> 2);
 	B.wi = 0; B.skip = (uint32_t)(a & 3); B.len_byte = (uint32_t)len;
+	B.wend = (uint32_t)((B.skip + len + 3) >> 2);
 #ifdef __CUDACC__
-	B.win = B.w[threadIdx.x & 31u]; B.win_next = B.w[32u + (threadIdx.x & 31u)];
+	B.win = bits_load(B, threadIdx.x & 31u); B.win_next = bits_load(B, 32u + (threadIdx.x & 31u));
+#elif IDL_INF_LOOKAHEAD
+	for (uint32_t l = 0; l < 32; ++l) { B.win[l] = bits_load(B, l); B.win_next[l] = bits_load(B, 32u + l); }
 #endif
 	B.bb = (uint64_t)(bits_next_word(B) >> (B.skip * 8)); B.bc = 32 - (int)B.skip * 8;
 }
@@ -147,6 +166,9 @@ IDL_INF_FN int build_code(int lane, int alphabet, const uint8_t *lens, int n, ui
 			next[l] = code; offs[l] = o; o += count[l];
 		}
 	}
+	// incomplete: as in zlib and libdeflate, only a literal/length or distance code that is empty or is one 1-bit code word (a bit pattern
+	// outside the code then decodes to no symbol); never the code-length code
+	if (left > 0 && (alphabet == A_CL || (left != 1 << 15 && !(left == 1 << 14 && count[1] == 1)))) return INF_E_CODE;
 	for (int s = 0; s < n; ++s) {
 		const int l = lens[s];
 		if (!l) continue;
@@ -209,10 +231,10 @@ IDL_INF_FN int inflate_member(int lane, Tables &T, const uint8_t *base, size_t i
 		} else if (btype == 1 || btype == 2) {
 			if (btype == 1) {
 				for (int i = lane; i < 288; i += IDL_INF_LANES) T.lens[i] = (uint8_t)(i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : 8);
-				for (int i = lane; i < 30; i += IDL_INF_LANES) T.lens[288 + i] = 5;
+				for (int i = lane; i < 32; i += IDL_INF_LANES) T.lens[288 + i] = 5;   // all 32 five-bit words (a complete code); 30 and 31 decode to K_BAD
 				IDL_INF_SYNC();
 				if (build_code(lane, A_LIT, T.lens, 288, T.lit_fast, LIT_BITS, T.lit_sym, T.lit_count)) return INF_E_CODE;
-				if (build_code(lane, A_DIST, T.lens + 288, 30, T.dist_fast, DIST_BITS, T.dist_sym, T.dist_count)) return INF_E_CODE;
+				if (build_code(lane, A_DIST, T.lens + 288, 32, T.dist_fast, DIST_BITS, T.dist_sym, T.dist_count)) return INF_E_CODE;
 			} else {
 				const int hlit = (int)bits_take(B, 5) + 257, hdist = (int)bits_take(B, 5) + 1, hclen = (int)bits_take(B, 4) + 4;
 				if (hlit > 286 || hdist > 30) return INF_E_CODE;
