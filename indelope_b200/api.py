@@ -114,11 +114,11 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
     """`indelope --gpu-decode [options] <fasta> <bam>` in process: the VCF (header + records) with everything in front of callsemble on the
     device as well -- BGZF inflate and record parse (idl_bam_open), gen_roi per target (idl_bam_sweep, src/indelope.nim:515-545,601-602), the
     batches built from the resident records (idl_bam_submit).  The host reads the two files and writes the VCF text.
-    by_target: the file is not decoded as a whole but target by target, each from the run of BGZF members <bam>.bai points to
-    (idl_bam_open_slice) -- for files that do not fit in device memory; needs the index.
     regions (list of `chr[:beg[-end]]`, 1-based, inclusive) and / or bed (a BED file, 0-based, half open): `indelope -r ... -R ...` -- only the regions of
-    interest of the whole-file run that overlap them, from just the BGZF members that hold them (idl_bam_sweep_window; needs the index).  `timings` then
-    also receives one dict per target with slices, retries and bytes read and decoded.  ValueError for a bad region or BED line."""
+    interest of the whole-file run that overlap them, from just the BGZF members that hold them (idl_bam_open_slice, idl_bam_sweep_window; needs the
+    index).  `timings` then also receives one dict per target with slices, retries and bytes read and decoded.  ValueError for a bad region or BED line.
+    by_target: the file is not decoded as a whole but target by target, through the same loop with every target whole as its interval -- for files
+    that do not fit in device memory; needs the index."""
     if regions or bed:
         by_target = True
     if by_target:
@@ -135,9 +135,8 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
         ref.set_targets(whole.ref_names, whole.ref_len)
         names, seqs = ref.sequences()
         keep = (ref,)
-    selected = None
-    if regions or bed:
-        selected = host.parse_regions(names, ref_len, regions, bed)
+    if by_target:
+        selected = host.parse_regions(names, ref_len, regions, bed) if regions or bed else [[(0, n)] for n in ref_len]
         if names:
             host.bai_target_span(bam, 0)      # IOError without the index, before anything runs
     caller = Caller(device, min_reads=min_reads, min_ctg_len=min_ctg_len, min_event_len=min_event_len, **kw)
@@ -147,13 +146,7 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
     done = [0]
     sweep_args = dict(min_event_support=max(3, min_reads - 2), min_read_coverage=min_reads, max_read_coverage=600)
 
-    def slice_of(sp):
-        with open(bam, "rb") as f:
-            f.seek(sp["file_begin"]); run = f.read(sp["file_end"] - sp["file_begin"])
-        return cuda.Bam(run, device=device, slice=dict(ref_names=names, ref_len=ref_len, first_record=sp["first_record"], end_member=sp["end_member"],
-                                                       end_offset=sp["end_offset"])), len(run)
-
-    def call_swept(b, c, r, first=0):
+    def call_resident(b, c, r, first=0):
         """regions [first, n) of one sweep of b through idl_bam_submit, records appended to out"""
         n = len(r["roi_start"]) - first
         if n <= 0:
@@ -182,7 +175,7 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
         done[0] += n
 
     def call_target_regions(c, ivs):
-        """the slices of one target's intervals, grown until no selected region touches an inner zone edge (indelope_main.cpp main_regions)"""
+        """the slices of one target's intervals, grown until no selected region touches an inner zone edge (indelope_main.cpp run_sliced)"""
         stats = dict(target=c, intervals=len(ivs), slices=0, retries=0, bytes_read=0, bytes_decoded=0, regions=0)
         todo = []
         for b0, e0 in ivs:
@@ -204,9 +197,12 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
                     stats["retries"] += 1
                     todo.insert(0, [w0, w1 + 1, iv, host.bai_region_run(bam, c, w0, w1 + 1)])
                 continue
-            b, nbytes = slice_of(run)
+            with open(bam, "rb") as f:
+                f.seek(run["file_begin"]); data = f.read(run["file_end"] - run["file_begin"])
+            b = cuda.Bam(data, device=device, slice=dict(ref_names=names, ref_len=ref_len, first_record=run["first_record"], end_member=run["end_member"],
+                                                         end_offset=run["end_offset"]))
             try:
-                stats["slices"] += 1; stats["bytes_read"] += nbytes; stats["bytes_decoded"] += b.info["inflated_bytes"]
+                stats["slices"] += 1; stats["bytes_read"] += len(data); stats["bytes_decoded"] += b.info["inflated_bytes"]
                 zone_hi = ref_len[c] if run["to_end"] else int(b.fetch([b.n_records - 1], what=0)["start"][0]) - 1
                 if zone_hi < run["zone_lo"] or zone_hi < iv[-1][1] - 1:
                     stats["retries"] += 1
@@ -219,7 +215,7 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
                     todo.insert(0, [w0, w1, iv, host.bai_region_run(bam, c, w0, w1)])
                     continue
                 first = int(np.searchsorted(r["roi_start"], last_end, side="right"))   # regions an earlier slice (before this one grew left) called
-                call_swept(b, c, r, first)
+                call_resident(b, c, r, first)
                 stats["regions"] += len(r["roi_start"]) - first
                 if len(r["roi_start"]) > first:
                     last_end = int(r["roi_end"][-1])
@@ -232,22 +228,10 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
         for c, name in enumerate(names):
             if name == "hs37d5" or name.startswith("GL"):   # skippable targets, src/indelope.nim:41-42
                 continue
-            if selected is not None:
-                if selected[c]:
-                    call_target_regions(c, selected[c])
-                continue
-            if by_target:
-                sp = host.bai_target_span(bam, c)
-                if sp is None:
-                    continue
-                b, _ = slice_of(sp)
-            else:
-                b = whole
-            try:
-                call_swept(b, c, b.sweep(c, **sweep_args))
-            finally:
-                if by_target:
-                    b.close()
+            if not by_target:
+                call_resident(whole, c, whole.sweep(c, **sweep_args))
+            elif selected[c]:
+                call_target_regions(c, selected[c])
         caller.status_counts = writer.status_counts()
     finally:
         caller.close()

@@ -3,6 +3,7 @@ back must give the same reads, the same regions of interest and the same oracle 
 specification says (checked here with Python's gzip on the BGZF members, independent of the C++ reader)."""
 import gzip
 import os
+import shutil
 import struct
 import subprocess
 
@@ -157,8 +158,19 @@ def test_cli_help_and_no_cpu_path(files):
     assert out.returncode == 0 and "--min-event-len" in out.stdout and "--min-reads" in out.stdout and "--threads" in out.stdout
     assert subprocess.run([exe, fa], capture_output=True).returncode == 1
     if not util.has_gpu():
-        r = subprocess.run([exe, "--min-event-len", "5", "--min-reads", "5", fa, bam], capture_output=True, text=True)
-        assert r.returncode == 1 and "no CPU path" in r.stderr and r.stdout == ""  # fails loudly, prints nothing
+        # every front end fails loudly and prints nothing: streamed, the whole file on the device, target by target, regions
+        for args, env in (([], {}), (["-g"], {}), (["-g"], {"INDELOPE_BY_TARGET": "1"}), (["-r", "chrS1"], {})):
+            r = subprocess.run([exe, "--min-event-len", "5", "--min-reads", "5"] + args + [fa, bam], capture_output=True, text=True, env=dict(os.environ, **env))
+            assert r.returncode == 1 and "no CPU path" in r.stderr and r.stdout == "", (args, env, r.stderr)
+
+
+def test_cli_by_target_without_index_fails_before_any_output(files, tmp_path):
+    """target-by-target decoding needs <bam>.bai: without it the run stops before the header (and before looking for a device)"""
+    ds, fa, bam = files
+    nobai = tmp_path / "nobai.bam"
+    shutil.copy(bam, nobai)
+    r = subprocess.run([build.build_cli(), "-g", fa, str(nobai)], capture_output=True, text=True, env=dict(os.environ, INDELOPE_BY_TARGET="1"))
+    assert r.returncode == 1 and "no index" in r.stderr and r.stdout == "", r.stderr
 
 
 @pytest.mark.gpu

@@ -227,6 +227,21 @@ def test_errors_leave_stdout_empty(files, tmp_path):
         api.call_bam(fa, bam, regions=["chrQ:1-5"])
     with pytest.raises(IOError, match="no index"):
         api.call_bam(fa, str(nobai), regions=["chrS1:1-5"])
+    with pytest.raises(IOError, match="no index"):
+        api.call_bam(fa, str(nobai), by_target=True)
+
+
+def test_by_target_is_the_regions_loop_over_whole_targets(files):
+    """target-by-target decoding goes through the sliced loop with one interval per target: a whole target is one slice, swept once"""
+    ds, fa, bam, rois, arrays, d = files
+    want = api.call_bam(fa, bam, **CALL)
+    t = []
+    assert api.call_bam(fa, bam, by_target=True, timings=t, **CALL) == want
+    stats = [x for x in t if "slices" in x]
+    assert [x["target"] for x in stats] == [0, 1] and all(x["slices"] == 1 and x["retries"] == 0 for x in stats), stats
+    r = run_cli(fa, bam, ["-g"], env={"INDELOPE_BY_TARGET": "1"})
+    assert r.returncode == 0 and r.stdout == want, r.stderr
+    assert timing(r.stderr, "slices") == 2 and timing(r.stderr, "retries") == 0
 
 
 # ---- a directed fixture: long evidence runs, slices that must grow, a deep region across a zone edge ---------------------------------------------------
