@@ -395,6 +395,39 @@ int idl_bam_submit(idl_ctx *ctx, idl_bam *bam, size_t n_regions, const int32_t *
 int idl_bam_pack(idl_ctx *ctx, idl_bam *bam, size_t n_regions, const int32_t *roi_chrom, const int32_t *roi_start, const int32_t *roi_end,
                  const int32_t *roi_n_reads, const int64_t *read_idx, uint32_t ordinal_base, idl_batch *out);
 
+/* ---------------------------------------------------------------------------------------------------------------
+ * A bgzip-compressed reference (ref.fa.gz, what htslib's fai_load opens for the reference's open_fai, src/indelope.nim:593) inflated and parsed
+ * on the device.  idl_fasta_open takes the file's bytes: the BGZF members are inflated as idl_bam_open inflates them (one warp per member, CRC
+ * checked), then byte-parallel passes over the text split it into records by the rules of the host loader (libindelope_host's load_fasta):
+ * lines end at '\n'; a line whose first byte is '>' starts a record whose name is the rest of the line up to the first ' ', '\t' or '\r'; every
+ * other line belongs to the latest record, its bytes kept verbatim except for the trailing run of '\r' and ' '.  A non-empty text whose first
+ * byte is not '>' is IDL_E_FORMAT; an empty text has no records.  Only BGZF is taken: plain gzip (members without the BC subfield) is
+ * IDL_E_FORMAT with a message that says to recompress with bgzip; a corrupt member is reported with its number and the decoder's error.  The
+ * sequences stay on the device (about the size of the text; the compressed and inflated bytes are freed before the call returns).
+ * --------------------------------------------------------------------------------------------------------------- */
+typedef struct idl_fasta idl_fasta;
+
+typedef struct idl_fasta_info {
+	uint64_t file_bytes, inflated_bytes;   /* compressed input, inflated text */
+	uint64_t sequence_bytes;               /* the records' sequences together (the parse's output) */
+	uint32_t n_members, n_chunks;          /* BGZF members (the EOF marker included), upload chunks */
+	int64_t n_records;
+	const char *const *name;               /* library-owned, valid until idl_fasta_close */
+	const int64_t *len;                    /* sequence lengths */
+	float ms_h2d, ms_inflate, ms_parse;    /* CUDA events on the call's stream, phases as in idl_bam_info; ms_parse includes the names' copy to the host */
+	uint64_t parse_algorithmic_bytes;      /* the text read once + the sequences written once + the per-record arrays */
+	uint64_t parse_streamed_bytes;         /* what the parse passes move through HBM (the text read three times, ...) */
+} idl_fasta_info;
+
+int idl_fasta_open(int device, const uint8_t *file, size_t file_len, idl_fasta **fa, char *err, size_t errlen);
+const idl_fasta_info *idl_fasta_get_info(const idl_fasta *fa);
+/* the sequence of one record into dst (dst_len >= its length) */
+int idl_fasta_copy(const idl_fasta *fa, int64_t record, uint8_t *dst, size_t dst_len);
+void idl_fasta_close(idl_fasta *fa);
+/* idl_bam_set_reference from a record of a FASTA on the same device (a device-to-device copy): IDL_E_ARG for a length that is not the target's, or a
+ * FASTA on another device */
+int idl_bam_set_reference_fasta(idl_bam *bam, int32_t target, const idl_fasta *fa, int64_t record);
+
 #ifdef __cplusplus
 }
 #endif

@@ -128,6 +128,9 @@ const char *idlh_dataset_chrom_name(const idlh_dataset *d, int32_t chrom);
 /* the device reads the BAM (idl_bam_open of indelope_cuda.h); the host keeps the reference sequences and turns what idl_bam_sweep / idl_bam_fetch
  * return into the idlh_rois that idlh_pack and idlh_vcf_records take */
 idlh_dataset *idlh_load_fasta(const char *fasta_path, char *err, size_t errlen);
+/* a reference (no reads) from n names and sequences found elsewhere -- idl_fasta_open of a bgzipped FASTA on the device; everything is copied.  Every
+ * loader here takes <fasta_path> plain or compressed with bgzip (BGZF members inflated on idlh_set_threads' host threads); plain gzip is refused. */
+idlh_dataset *idlh_dataset_from_sequences(int32_t n, const char *const *names, const uint8_t *const *seqs, const int64_t *lens);
 /* the FASTA's sequences in the order of the BAM header's targets; of the BAM only the header is read */
 idlh_dataset *idlh_load_targets(const char *fasta_path, const char *bam_path, char *err, size_t errlen);
 /* where one target's records lie in the file, from <bam>.bai: the run of whole BGZF members [*file_begin, *file_end) and the start / end of the record
@@ -149,6 +152,8 @@ idlh_regions *idlh_regions_parse(int32_t n_ref, const char *const *ref_name, con
 int64_t idlh_regions_get(const idlh_regions *r, int32_t target, int64_t *beg, int64_t *end, int64_t cap);   /* intervals of a target (up to cap copied); returns their number */
 void idlh_regions_free(idlh_regions *r);
 int idlh_dataset_set_targets(idlh_dataset *d, int32_t n_ref, const char *const *ref_name, const int64_t *ref_len, char *err, size_t errlen);
+/* the same with the targets of a BAM file's header (only the members that hold the header are read): what idlh_load_targets does after loading the FASTA */
+int idlh_dataset_set_bam_targets(idlh_dataset *d, const char *bam_path, char *err, size_t errlen);
 idlh_rois *idlh_rois_from_arrays(const idlh_dataset *d, int64_t n_reads, const int32_t *start, const int32_t *stop, const int32_t *len, const uint8_t *mapq, const uint16_t *flag,
                                  const int64_t *seq_off, const uint8_t *bases, const uint8_t *quals, int64_t n_rois, const int32_t *roi_chrom, const int32_t *roi_start,
                                  const int32_t *roi_stop, const int32_t *roi_n_reads, const int64_t *read_idx);

@@ -118,23 +118,42 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
     interest of the whole-file run that overlap them, from just the BGZF members that hold them (idl_bam_open_slice, idl_bam_sweep_window; needs the
     index).  `timings` then also receives one dict per target with slices, retries and bytes read and decoded.  ValueError for a bad region or BED line.
     by_target: the file is not decoded as a whole but target by target, through the same loop with every target whole as its interval -- for files
-    that do not fit in device memory; needs the index."""
+    that do not fit in device memory; needs the index.
+    A FASTA compressed with bgzip is inflated and parsed on the device (cuda.Fasta); the batches take the targets' sequences from there."""
     if regions or bed:
         by_target = True
+    fa_dev, record_of = None, None
+    with open(fasta, "rb") as f:
+        if f.read(2) == b"\x1f\x8b":
+            f.seek(0)
+            fa_dev = cuda.Fasta(f.read(), device=device)
+    if fa_dev is not None:
+        ref = host.Dataset.from_sequences(fa_dev.names, [fa_dev.sequence(r) for r in range(fa_dev.n_records)])
     if by_target:
-        st = host.Stream(fasta, bam)          # parses the BAM header and orders the FASTA's sequences after it; no record is read through it
-        tg = st.targets()
-        ta = tg.arrays()
-        names, seqs = ta["chrom_names"], ta["chrom_seqs"]
+        if fa_dev is not None:
+            ref.set_bam_targets(bam)
+            names, seqs = ref.sequences()
+            keep = (ref, fa_dev)
+        else:
+            st = host.Stream(fasta, bam)      # parses the BAM header and orders the FASTA's sequences after it; no record is read through it
+            tg = st.targets()
+            ta = tg.arrays()
+            names, seqs = ta["chrom_names"], ta["chrom_seqs"]
+            keep = (st, tg)
         ref_len = [len(x) for x in seqs]
-        keep = (st, tg)
     else:
-        ref = host.Dataset.load_fasta(fasta)
+        if fa_dev is None:
+            ref = host.Dataset.load_fasta(fasta)
         data = open(bam, "rb").read()
         whole = cuda.Bam(data, device=device)
         ref.set_targets(whole.ref_names, whole.ref_len)
         names, seqs = ref.sequences()
-        keep = (ref,)
+        keep = (ref, fa_dev)
+    if fa_dev is not None:   # each target's record: the first of its name, as set_targets takes it
+        first = {}
+        for r, nm in enumerate(fa_dev.names):
+            first.setdefault(nm, r)
+        record_of = [first[nm] for nm in names]
     if by_target:
         selected = host.parse_regions(names, ref_len, regions, bed) if regions or bed else [[(0, n)] for n in ref_len]
         if names:
@@ -156,7 +175,10 @@ def call_bam(fasta, bam, device=0, min_reads=3, min_ctg_len=73, min_event_len=4,
         idx = r["read_idx"][int(r["roi_read_begin"][first]):]
         begin = np.concatenate([[0], np.cumsum(nr)]).astype(np.int64)
         rois = host.Rois(arrays=dict(empty, roi_chrom=chrom, roi_start=rs, roi_stop=re, roi_read_begin=begin[:-1], roi_n_reads=nr, read_idx=idx, chrom_names=names, chrom_seqs=seqs))
-        b.set_reference(c, seqs[c])
+        if fa_dev is not None:
+            b.set_reference_fasta(c, fa_dev, record_of[c])
+        else:
+            b.set_reference(c, seqs[c])
         inflight = []
 
         def drain():

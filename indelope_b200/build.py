@@ -19,7 +19,7 @@ CUDA_LIB = os.path.join(HERE, "libindelope_cuda.so")
 HOST_LIB = os.path.join(HERE, "libindelope_host.so")
 CLI_BIN = os.path.join(HERE, "indelope")
 
-CUDA_SRCS = ["pipeline.cu", "sweep.cu", "bamdev.cu"]
+CUDA_SRCS = ["pipeline.cu", "sweep.cu", "bamdev.cu", "fastadev.cu"]
 HOST_SRCS = ["host/synth_sweep.cpp", "host/pack_vcf.cpp", "host/bamio.cpp"]
 CLI_SRCS = ["host/indelope_main.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--use_fast_math",

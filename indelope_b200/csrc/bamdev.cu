@@ -50,7 +50,7 @@ constexpr int INF_CTAS_PER_SM = INF_CTAS_PER_SM_;
 constexpr unsigned SEG_BYTES = 1u << 16;     // segment of the inflated stream one warp chains
 constexpr int SCAN_THREADS = 256, SCAN_ITEMS = 8, SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
 
-struct Member { unsigned long long in_off; unsigned long long out_off; uint32_t in_len, out_len, crc, pad; };
+using Member = BgzfMember;
 
 // ---- stage 2 ----
 __global__ void __launch_bounds__(INF_WARPS * 32, INF_CTAS_PER_SM)
@@ -489,6 +489,84 @@ const char *inf_error_text(int rc)
 
 } // namespace
 
+// ---- the BGZF inflate stage (bamdev.h) ----
+bool bgzf_walk(const uint8_t *file, size_t file_len, std::vector<BgzfMember> &members, std::vector<size_t> &member_at, size_t &total, std::string &why)
+{
+	total = 0;
+	for (size_t at = 0; at < file_len;) {
+		if (file_len - at < 18) { why = "truncated BGZF header"; return false; }
+		const uint8_t *h = file + at;
+		if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4)) { why = "not a BGZF file (is it BAM? CRAM is not supported)"; return false; }
+		const unsigned xlen = h16(h + 10);
+		if (file_len - at < 12 + (size_t)xlen) { why = "truncated BGZF extra field"; return false; }
+		int bsize = -1;
+		for (unsigned x = 0; x + 4 <= xlen;) {
+			const uint8_t *e = h + 12 + x; const unsigned slen = h16(e + 2);
+			if (e[0] == 'B' && e[1] == 'C' && slen == 2) bsize = h16(e + 4);
+			x += 4 + slen;
+		}
+		if (bsize < 0) { why = "BGZF block without BC subfield"; return false; }
+		const size_t csize = (size_t)bsize + 1;
+		if (csize < 12 + (size_t)xlen + 8 || file_len - at < csize) { why = "truncated BGZF block"; return false; }
+		const uint32_t usize = h32(h + csize - 4);
+		if (usize > 65536) { why = "BGZF block larger than 64 KiB"; return false; }
+		BgzfMember M; M.in_off = at + 12 + xlen; M.in_len = (uint32_t)(csize - 12 - xlen - 8); M.out_off = total; M.out_len = usize; M.crc = h32(h + csize - 8); M.pad = 0;
+		members.push_back(M); member_at.push_back(at);
+		total += usize; at += csize;
+	}
+	return true;
+}
+
+cudaError_t bgzf_inflate_chunks(cudaStream_t st, int n_sm, const uint8_t *file, size_t file_len, const std::vector<BgzfMember> &members, uint8_t *d_comp,
+                                const BgzfMember *d_members, uint8_t *d_out, unsigned long long *d_err, unsigned *d_next, uint32_t *n_chunks)
+{
+	// The file goes up in chunks of whole members and every chunk's members are inflated as soon as they have arrived, on one of four
+	// streams: the copy of chunk k+1 (a staged copy when the caller's buffer is pageable) overlaps the kernels of chunks k, k-1, ...
+	// One member is a serial chain of ~9 ms whatever the chunk's size, so consecutive chunks' kernels have to share the SMs.
+	constexpr int NS = 4; constexpr size_t CHUNK = 32u << 20;
+	cudaStream_t ks[NS] = {}; cudaEvent_t ce[64] = {}, ke[NS] = {};
+	cudaError_t e_ = cudaSuccess;
+	for (int k = 0; k < NS && e_ == cudaSuccess; ++k) { e_ = cudaStreamCreateWithFlags(&ks[k], cudaStreamNonBlocking); if (e_ == cudaSuccess) e_ = cudaEventCreateWithFlags(&ke[k], cudaEventDisableTiming); }
+	if (e_ == cudaSuccess) e_ = cudaEventCreateWithFlags(&ce[0], cudaEventDisableTiming);
+	if (e_ == cudaSuccess) e_ = cudaEventRecord(ce[0], st);   // the member table, the cleared counters
+	size_t m0 = 0, byte0 = 0; int chunk = 0;
+	while (m0 < members.size() && e_ == cudaSuccess) {
+		size_t m1 = m0, byte1 = byte0;
+		while (m1 < members.size() && (m1 == m0 || members[m1].in_off + members[m1].in_len + 8 - byte0 <= CHUNK)) { byte1 = (size_t)(members[m1].in_off + members[m1].in_len + 8); ++m1; }
+		if (chunk >= 62) { m1 = members.size(); byte1 = file_len; }   // (a file of more than 2 GB: the rest as one chunk)
+		const int c = chunk + 1;
+		e_ = cudaMemcpyAsync(d_comp + byte0, file + byte0, byte1 - byte0, cudaMemcpyHostToDevice, st);
+		if (e_ == cudaSuccess) e_ = cudaEventCreateWithFlags(&ce[c], cudaEventDisableTiming);
+		if (e_ == cudaSuccess) e_ = cudaEventRecord(ce[c], st);
+		cudaStream_t k_st = ks[chunk % NS];
+		if (e_ == cudaSuccess) e_ = cudaStreamWaitEvent(k_st, ce[c], 0);
+		if (e_ == cudaSuccess && chunk < NS) e_ = cudaStreamWaitEvent(k_st, ce[0], 0);
+		if (e_ == cudaSuccess) {
+			const size_t nm = m1 - m0;
+			const unsigned ctas = (unsigned)std::min<size_t>((size_t)n_sm * INF_CTAS_PER_SM, (nm + INF_WARPS - 1) / INF_WARPS);
+			bgzf_inflate_kernel<<<ctas, INF_WARPS * 32, 0, k_st>>>(d_comp, d_members, (uint32_t)m0, (uint32_t)m1, d_out, d_err, d_next + c);
+			e_ = cudaGetLastError();
+		}
+		m0 = m1; byte0 = byte1; ++chunk;
+	}
+	// the call's stream continues when every chunk's kernel is done (the padding behind the file was cleared before the first of them started)
+	for (int k = 0; k < NS && e_ == cudaSuccess; ++k) { e_ = cudaEventRecord(ke[k], ks[k]); if (e_ == cudaSuccess) e_ = cudaStreamWaitEvent(st, ke[k], 0); }
+	const cudaError_t e_sync = cudaStreamSynchronize(st);
+	for (auto &e : ce) if (e) cudaEventDestroy(e);
+	for (int k = 0; k < NS; ++k) { if (ke[k]) cudaEventDestroy(ke[k]); if (ks[k]) cudaStreamDestroy(ks[k]); }
+	if (e_ != cudaSuccess) return e_;
+	if (e_sync != cudaSuccess) return e_sync;
+	*n_chunks = (uint32_t)chunk;
+	return cudaSuccess;
+}
+
+std::string bgzf_error_text(unsigned long long first_error)
+{
+	char msg[160];
+	snprintf(msg, sizeof msg, "BGZF block %llu failed to inflate (corrupt data or CRC mismatch: %s)", first_error >> 8, inf_error_text((int)(first_error & 0xff)));
+	return msg;
+}
+
 struct idl_bam {
 	int device = 0;
 	cudaStream_t st = nullptr;
@@ -553,27 +631,7 @@ static int bam_open_impl(int device, const uint8_t *file, size_t file_len, const
 	if (device < 0 || device >= ndev) return IDL_E_ARG;
 	// 1. members
 	std::vector<Member> members; std::vector<size_t> member_at; size_t total = 0;
-	for (size_t at = 0; at < file_len;) {
-		if (file_len - at < 18) { set_err(err, errlen, "truncated BGZF header"); return IDL_E_FORMAT; }
-		const uint8_t *h = file + at;
-		if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4)) { set_err(err, errlen, "not a BGZF file (is it BAM? CRAM is not supported)"); return IDL_E_FORMAT; }
-		const unsigned xlen = h16(h + 10);
-		if (file_len - at < 12 + (size_t)xlen) { set_err(err, errlen, "truncated BGZF extra field"); return IDL_E_FORMAT; }
-		int bsize = -1;
-		for (unsigned x = 0; x + 4 <= xlen;) {
-			const uint8_t *e = h + 12 + x; const unsigned slen = h16(e + 2);
-			if (e[0] == 'B' && e[1] == 'C' && slen == 2) bsize = h16(e + 4);
-			x += 4 + slen;
-		}
-		if (bsize < 0) { set_err(err, errlen, "BGZF block without BC subfield"); return IDL_E_FORMAT; }
-		const size_t csize = (size_t)bsize + 1;
-		if (csize < 12 + (size_t)xlen + 8 || file_len - at < csize) { set_err(err, errlen, "truncated BGZF block"); return IDL_E_FORMAT; }
-		const uint32_t usize = h32(h + csize - 4);
-		if (usize > 65536) { set_err(err, errlen, "BGZF block larger than 64 KiB"); return IDL_E_FORMAT; }
-		Member M; M.in_off = at + 12 + xlen; M.in_len = (uint32_t)(csize - 12 - xlen - 8); M.out_off = total; M.out_len = usize; M.crc = h32(h + csize - 8); M.pad = 0;
-		members.push_back(M); member_at.push_back(at);
-		total += usize; at += csize;
-	}
+	{ std::string why; if (!bgzf_walk(file, file_len, members, member_at, total, why)) { set_err(err, errlen, why); return IDL_E_FORMAT; } }
 	if (members.empty() || (!slice && total < 12)) { set_err(err, errlen, "not a BAM file"); return IDL_E_FORMAT; }
 	if (members.size() >= (1ull << 32)) return IDL_E_CAPACITY;
 	// IDL_BAM_TIMING=1: wall-clock phases of the call on stderr (context creation and allocations are not inside the CUDA events)
@@ -611,42 +669,8 @@ static int bam_open_impl(int device, const uint8_t *file, size_t file_len, const
 		BCK(cudaMemsetAsync(d_err, 0xff, 64, st)); BCK(cudaMemsetAsync(d_next, 0, 4 * 64, st)); BCK(cudaMemsetAsync(b->d_out + total, 0, 64, st));
 		BCK(cudaEventRecord(ev[1], st));
 		{
-			// The file goes up in chunks of whole members and every chunk's members are inflated as soon as they have arrived, on one of four
-			// streams: the copy of chunk k+1 (a staged copy when the caller's buffer is pageable) overlaps the kernels of chunks k, k-1, ...
-			// One member is a serial chain of ~9 ms whatever the chunk's size, so consecutive chunks' kernels have to share the SMs.
-			constexpr int NS = 4; constexpr size_t CHUNK = 32u << 20;
-			cudaStream_t ks[NS] = {}; cudaEvent_t ce[64] = {}, ke[NS] = {};
-			cudaError_t e_ = cudaSuccess;
-			for (int k = 0; k < NS && e_ == cudaSuccess; ++k) { e_ = cudaStreamCreateWithFlags(&ks[k], cudaStreamNonBlocking); if (e_ == cudaSuccess) e_ = cudaEventCreateWithFlags(&ke[k], cudaEventDisableTiming); }
-			if (e_ == cudaSuccess) e_ = cudaEventCreateWithFlags(&ce[0], cudaEventDisableTiming);
-			if (e_ == cudaSuccess) e_ = cudaEventRecord(ce[0], st);   // the member table, the cleared counters
-			size_t m0 = 0, byte0 = 0; int chunk = 0;
-			while (m0 < members.size() && e_ == cudaSuccess) {
-				size_t m1 = m0, byte1 = byte0;
-				while (m1 < members.size() && (m1 == m0 || members[m1].in_off + members[m1].in_len + 8 - byte0 <= CHUNK)) { byte1 = (size_t)(members[m1].in_off + members[m1].in_len + 8); ++m1; }
-				if (chunk >= 62) { m1 = members.size(); byte1 = file_len; }   // (a file of more than 2 GB: the rest as one chunk)
-				const int c = chunk + 1;
-				e_ = cudaMemcpyAsync(b->d_comp + byte0, file + byte0, byte1 - byte0, cudaMemcpyHostToDevice, st);
-				if (e_ == cudaSuccess) e_ = cudaEventCreateWithFlags(&ce[c], cudaEventDisableTiming);
-				if (e_ == cudaSuccess) e_ = cudaEventRecord(ce[c], st);
-				cudaStream_t k_st = ks[chunk % NS];
-				if (e_ == cudaSuccess) e_ = cudaStreamWaitEvent(k_st, ce[c], 0);
-				if (e_ == cudaSuccess && chunk < NS) e_ = cudaStreamWaitEvent(k_st, ce[0], 0);
-				if (e_ == cudaSuccess) {
-					const size_t nm = m1 - m0;
-					const unsigned ctas = (unsigned)std::min<size_t>((size_t)n_sm * INF_CTAS_PER_SM, (nm + INF_WARPS - 1) / INF_WARPS);
-					bgzf_inflate_kernel<<<ctas, INF_WARPS * 32, 0, k_st>>>(b->d_comp, d_members, (uint32_t)m0, (uint32_t)m1, b->d_out, d_err, d_next + c);
-					e_ = cudaGetLastError();
-				}
-				m0 = m1; byte0 = byte1; ++chunk;
-			}
-			// the call's stream continues when every chunk's kernel is done (the padding behind the file was cleared before the first of them started)
-			for (int k = 0; k < NS && e_ == cudaSuccess; ++k) { e_ = cudaEventRecord(ke[k], ks[k]); if (e_ == cudaSuccess) e_ = cudaStreamWaitEvent(st, ke[k], 0); }
-			const cudaError_t e_sync = cudaStreamSynchronize(st);
-			for (auto &e : ce) if (e) cudaEventDestroy(e);
-			for (int k = 0; k < NS; ++k) { if (ke[k]) cudaEventDestroy(ke[k]); if (ks[k]) cudaStreamDestroy(ks[k]); }
-			if (e_ != cudaSuccess || e_sync != cudaSuccess) { why = std::string("inflate: ") + cudaGetErrorString(e_ != cudaSuccess ? e_ : e_sync); rc = IDL_E_CUDA; goto done; }
-			b->info.n_chunks = (uint32_t)chunk;
+			const cudaError_t e_ = bgzf_inflate_chunks(st, n_sm, file, file_len, members, b->d_comp, d_members, b->d_out, d_err, d_next, &b->info.n_chunks);
+			if (e_ != cudaSuccess) { why = std::string("inflate: ") + cudaGetErrorString(e_); rc = IDL_E_CUDA; goto done; }
 		}
 		BCK(cudaEventRecord(ev[2], st));
 		unsigned long long herr[8];
@@ -656,11 +680,7 @@ static int bam_open_impl(int device, const uint8_t *file, size_t file_len, const
 		BCK(cudaMemcpyAsync(head.data(), b->d_out, head.size(), cudaMemcpyDeviceToHost, st));
 		BCK(cudaStreamSynchronize(st));
 		tw[3] = now();
-		if (herr[0] != ~0ULL) {
-			char msg[160];
-			snprintf(msg, sizeof msg, "BGZF block %llu failed to inflate (corrupt data or CRC mismatch: %s)", herr[0] >> 8, inf_error_text((int)(herr[0] & 0xff)));
-			BFAIL(msg);
-		}
+		if (herr[0] != ~0ULL) BFAIL(bgzf_error_text(herr[0]));
 		uint32_t n_ref = 0; std::vector<int32_t> ref_len32; size_t begin = 0, rec_total = total;
 		if (!slice) {
 			if (memcmp(head.data(), "BAM\1", 4) != 0) BFAIL("not a BAM file");
@@ -972,7 +992,8 @@ template <class T> cudaError_t scratch_get(idl_bam::ScratchSet &S, int slot, siz
 	*out = (T*)S.p[slot];
 	return cudaSuccess;
 }
-// exclusive 64-bit scan of n uint32 values into out[0..n] (out[n] = total); tot = scratch for the tile totals
+} // namespace
+
 cudaError_t scan_u32(const uint32_t *in, size_t n, unsigned long long *out, unsigned long long *tot, cudaStream_t st)
 {
 	const size_t nt = std::max<size_t>(1, (n + 1 + SCAN_TILE - 1) / SCAN_TILE);
@@ -981,7 +1002,6 @@ cudaError_t scan_u32(const uint32_t *in, size_t n, unsigned long long *out, unsi
 	scan_apply_kernel<<<(unsigned)nt, SCAN_THREADS, 0, st>>>(in, n, tot, out);
 	return cudaGetLastError();
 }
-} // namespace
 
 int bam_device_of(const idl_bam *b) { return b ? b->device : -1; }
 
@@ -1060,6 +1080,21 @@ extern "C" int idl_bam_set_reference(idl_bam *b, int32_t target, const uint8_t *
 	uint8_t *d = nullptr;
 	if (cudaMalloc((void**)&d, (size_t)len + 64) != cudaSuccess) return IDL_E_NOMEM;
 	if (cudaMemcpyAsync(d, seq, (size_t)len, cudaMemcpyHostToDevice, b->st) != cudaSuccess || cudaMemsetAsync(d + len, 0, 64, b->st) != cudaSuccess ||
+	    cudaMemcpyAsync(b->d_ref_seq + target, &d, 8, cudaMemcpyHostToDevice, b->st) != cudaSuccess || cudaStreamSynchronize(b->st) != cudaSuccess) { cudaFree(d); return IDL_E_CUDA; }
+	b->ref_seq[(size_t)target] = d;
+	return IDL_OK;
+}
+
+extern "C" int idl_bam_set_reference_fasta(idl_bam *b, int32_t target, const idl_fasta *fa, int64_t record)
+{
+	const uint8_t *src = nullptr; int64_t len = 0; int dev = -1;
+	if (!b || target < 0 || target >= b->info.n_ref || fasta_record_on_device(fa, record, &src, &len, &dev) != IDL_OK) return IDL_E_ARG;
+	if (dev != b->device || len != b->ref_len[(size_t)target]) return IDL_E_ARG;
+	if (cudaSetDevice(b->device) != cudaSuccess) return IDL_E_CUDA;
+	if (b->ref_seq[(size_t)target]) return IDL_OK;
+	uint8_t *d = nullptr;
+	if (cudaMalloc((void**)&d, (size_t)len + 64) != cudaSuccess) return IDL_E_NOMEM;
+	if (cudaMemcpyAsync(d, src, (size_t)len, cudaMemcpyDeviceToDevice, b->st) != cudaSuccess || cudaMemsetAsync(d + len, 0, 64, b->st) != cudaSuccess ||
 	    cudaMemcpyAsync(b->d_ref_seq + target, &d, 8, cudaMemcpyHostToDevice, b->st) != cudaSuccess || cudaStreamSynchronize(b->st) != cudaSuccess) { cudaFree(d); return IDL_E_CUDA; }
 	b->ref_seq[(size_t)target] = d;
 	return IDL_OK;

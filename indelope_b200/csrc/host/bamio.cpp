@@ -99,10 +99,9 @@ bool bgzf_inflate_block(const std::vector<uint8_t> &file, const BgzfBlock &b, ui
 	return (uint32_t)crc32(crc32(0L, Z_NULL, 0), dst, (uInt)b.usize) == le32(h + b.csize - 8);
 }
 
-bool bgzf_read_all(const char *path, int threads, std::vector<uint8_t> &out, std::string &why)
+// every member of a BGZF file's bytes inflated (and CRC-checked) by `threads` workers
+bool bgzf_inflate_all(const std::vector<uint8_t> &file, int threads, std::vector<uint8_t> &out, std::string &why)
 {
-	std::vector<uint8_t> file;
-	if (!read_file(path, file, why)) return false;
 	std::vector<BgzfBlock> blocks; size_t total = 0;
 	if (!bgzf_index(file, blocks, total, why)) return false;
 	out.resize(total);
@@ -122,6 +121,13 @@ bool bgzf_read_all(const char *path, int threads, std::vector<uint8_t> &out, std
 	for (auto &t : pool) t.join();
 	if (!ok.load()) { why = "BGZF block failed to inflate (corrupt data or CRC mismatch)"; return false; }
 	return true;
+}
+
+bool bgzf_read_all(const char *path, int threads, std::vector<uint8_t> &out, std::string &why)
+{
+	std::vector<uint8_t> file;
+	if (!read_file(path, file, why)) return false;
+	return bgzf_inflate_all(file, threads, out, why);
 }
 
 struct BgzfWriter {
@@ -237,10 +243,22 @@ inline uint8_t code16(uint8_t c)
 // ---------------------------------------------------------------------------------------------------------------
 // FASTA
 // ---------------------------------------------------------------------------------------------------------------
+// A FASTA file, plain or compressed with bgzip (ref.fa.gz: what htslib's fai_load opens for the reference's open_fai, src/indelope.nim:593); the
+// BGZF members are inflated on pack_threads() threads.  Plain gzip is refused, as fai_load refuses it.
 bool load_fasta(const char *path, idlh_dataset &D, std::string &why)
 {
 	std::vector<uint8_t> file;
 	if (!read_file(path, file, why)) return false;
+	if (file.size() >= 2 && file[0] == 0x1f && file[1] == 0x8b) {
+		std::vector<uint8_t> text;
+		if (!bgzf_inflate_all(file, pack_threads(), text, why)) {
+			if (why.compare(0, 15, "not a BGZF file") == 0 || why == "BGZF block without BC subfield")
+				why = "gzip member without the BGZF BC subfield (plain gzip)";
+			why = std::string(path) + ": " + why + "; a compressed FASTA must be compressed with bgzip (recompress it with bgzip)";
+			return false;
+		}
+		file.swap(text);
+	}
 	size_t i = 0; const size_t n = file.size();
 	while (i < n) {
 		if (file[i] != '>') { why = std::string("FASTA record does not start with '>' in ") + path; return false; }
@@ -583,8 +601,16 @@ idlh_dataset *idlh_load_targets(const char *fasta_path, const char *bam_path, ch
 	idlh_dataset *D = new idlh_dataset();
 	memset(&D->P, 0, sizeof D->P);
 	std::string why;
-	auto fail = [&](const std::string &m) -> idlh_dataset* { set_err(err, errlen, m); delete D; return nullptr; };
-	if (!load_fasta(fasta_path, *D, why)) return fail(why);
+	if (!load_fasta(fasta_path, *D, why)) { set_err(err, errlen, why); delete D; return nullptr; }
+	if (idlh_dataset_set_bam_targets(D, bam_path, err, errlen) != 0) { delete D; return nullptr; }
+	return D;
+}
+
+/* idlh_dataset_set_targets with the targets of <bam_path>'s header: only the first members of the file are read and inflated, as far as the header
+ * reaches.  Same checks and messages as idlh_load.  0 = ok. */
+int idlh_dataset_set_bam_targets(idlh_dataset *D, const char *bam_path, char *err, size_t errlen)
+{
+	auto fail = [&](const std::string &m) -> int { set_err(err, errlen, m); return 1; };
 	FILE *f = fopen(bam_path, "rb");
 	if (!f) return fail(std::string("cannot open ") + bam_path);
 	std::vector<uint8_t> file, u; size_t cpos = 0; bool eof = false;
@@ -609,7 +635,7 @@ idlh_dataset *idlh_load_targets(const char *fasta_path, const char *bam_path, ch
 		}
 		return true;
 	};
-	auto done = [&](idlh_dataset *r) { fclose(f); return r; };
+	auto done = [&](int r) { fclose(f); return r; };
 	if (!need(12) || memcmp(u.data(), "BAM\1", 4) != 0) return done(fail(std::string(bam_path) + ": not a BAM file"));
 	size_t at = 4;
 	const uint32_t l_text = le32(u.data() + at); at += 4;
@@ -630,7 +656,7 @@ idlh_dataset *idlh_load_targets(const char *fasta_path, const char *bam_path, ch
 		names.push_back(name); chroms.push_back(D->chroms[k]);
 	}
 	D->names.swap(names); D->chroms.swap(chroms);
-	return done(D);
+	return done(0);
 }
 
 /* the reference sequences alone (the device reads the BAM: idl_bam_open) */
@@ -640,6 +666,15 @@ idlh_dataset *idlh_load_fasta(const char *fasta_path, char *err, size_t errlen)
 	memset(&D->P, 0, sizeof D->P);
 	std::string why;
 	if (!load_fasta(fasta_path, *D, why)) { set_err(err, errlen, why); delete D; return nullptr; }
+	return D;
+}
+
+/* a reference from names and sequences found elsewhere (idl_fasta_open: a bgzipped FASTA parsed on the device); everything is copied */
+idlh_dataset *idlh_dataset_from_sequences(int32_t n, const char *const *names, const uint8_t *const *seqs, const int64_t *lens)
+{
+	idlh_dataset *D = new idlh_dataset();
+	memset(&D->P, 0, sizeof D->P);
+	for (int32_t k = 0; k < n; ++k) { D->names.emplace_back(names[k]); D->chroms.emplace_back(seqs[k], seqs[k] + lens[k]); }
 	return D;
 }
 

@@ -33,6 +33,9 @@ struct idlh_rois {
 	idlh_roiset view;
 };
 
+// host threads of idlh_pack and of the bgzipped FASTA's inflate (idlh_set_threads; 0 = $IDLH_THREADS, else every core up to 32) (pack_vcf.cpp)
+int pack_threads();
+
 // skippable (src/indelope.nim:40-47): the two decoy-contig name tests and the flag tests
 inline bool idlh_skippable_chrom(const std::string &name) { return name == "hs37d5" || name.compare(0, 2, "GL") == 0; }
 inline bool idlh_skippable_flag(uint16_t f) { return (f & 0x400) || (f & 0x200) || (f & 0x4) || (f & 0x800) || (f & 0x100); }

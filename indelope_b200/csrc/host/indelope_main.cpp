@@ -14,6 +14,7 @@
 #include <cstring>
 #include <algorithm>
 #include <deque>
+#include <map>
 #include <string>
 #include <chrono>
 #include <thread>
@@ -28,7 +29,7 @@ static const char USAGE[] =
 	"\n"
 	"Arguments:\n"
 	"\n"
-	"  <reference>     reference fasta file.\n"
+	"  <reference>     reference fasta file, plain or compressed with bgzip (with -g, -r or -R it is then inflated and parsed on the GPU).\n"
 	"  <BAM>           call variants in this file (coordinate sorted).\n"
 	"\n"
 	"Options:\n"
@@ -102,6 +103,8 @@ struct Calls {
 	int create_rc = IDL_OK;
 	idlh_dataset *ref = nullptr;
 	idlh_rois *targets = nullptr;          // ref without regions
+	idl_fasta *fa = nullptr;               // a bgzipped reference parsed on the device (open_reference): the batches take its sequences from there
+	std::vector<int64_t> fa_record;        // per target of ref: its record in fa
 	idlh_vcf *writer = idlh_vcf_new();
 	std::vector<Lane> lanes;               // pinned batches of submit_packed, one per stream
 	std::deque<Flight> inflight;
@@ -179,9 +182,12 @@ struct Calls {
 	{
 		const idlh_roiset *all = idlh_rois_view(targets);
 		double t0 = now_s();
-		for (size_t k = 0; k < n && !status; ++k)
-			if ((k == 0 || chrom[k] != chrom[k - 1]) && idl_bam_set_reference(bam, chrom[k], all->chrom_seq[chrom[k]], all->chrom_len[chrom[k]]) != IDL_OK)
-				status = die("idl_bam_set_reference", "could not place the reference on the device");
+		for (size_t k = 0; k < n && !status; ++k) {
+			if (k > 0 && chrom[k] == chrom[k - 1]) continue;
+			const int r = fa ? idl_bam_set_reference_fasta(bam, chrom[k], fa, fa_record[(size_t)chrom[k]])
+			                 : idl_bam_set_reference(bam, chrom[k], all->chrom_seq[chrom[k]], all->chrom_len[chrom[k]]);
+			if (r != IDL_OK) status = die("idl_bam_set_reference", "could not place the reference on the device");
+		}
 		t_ref += now_s() - t0;
 		size_t at_idx = 0;
 		for (size_t lo = 0; lo < n && !status; ) {
@@ -216,8 +222,68 @@ struct Calls {
 		targets = nullptr;
 		if (ref) idlh_dataset_free(ref);
 		ref = nullptr;
+		if (fa) idl_fasta_close(fa);
+		fa = nullptr;
+	}
+
+	// after ref has been ordered as the BAM header lists its targets: each target's record in fa (the first of its name, as idlh_dataset_set_targets
+	// takes it)
+	void map_fasta_records()
+	{
+		if (!fa) return;
+		const idl_fasta_info *fi = idl_fasta_get_info(fa);
+		std::map<std::string, int64_t> first;
+		for (int64_t r = fi->n_records - 1; r >= 0; --r) first[fi->name[r]] = r;
+		fa_record.clear();
+		for (int32_t c = 0; c < idlh_dataset_n_chroms(ref); ++c) fa_record.push_back(first[idlh_dataset_chrom_name(ref, c)]);
 	}
 };
+
+static bool is_gzip(const std::string &path)
+{
+	FILE *f = fopen(path.c_str(), "rb");
+	if (!f) return false;
+	unsigned char m[2] = {0, 0};
+	const bool gz = fread(m, 1, 2, f) == 2 && m[0] == 0x1f && m[1] == 0x8b;
+	fclose(f);
+	return gz;
+}
+
+// The reference of the front ends that decode on the device, into calls.ref (the FASTA's records in file order).  A bgzipped FASTA is read here and
+// inflated and parsed on the device (idl_fasta_open), where it stays for idl_bam_set_reference_fasta; the host keeps copies of the sequences for the
+// VCF writer.  A plain FASTA is loaded on the host as before.  0, or the exit status after the message.
+static int open_reference(const Options &o, Calls &calls)
+{
+	char err[512] = {0};
+	if (!is_gzip(o.fa)) {
+		calls.ref = idlh_load_fasta(o.fa.c_str(), err, sizeof err);
+		return calls.ref ? 0 : die("input", err);
+	}
+	const double t0 = now_s();
+	const int64_t size = file_size(o.fa);
+	std::vector<uint8_t> file;
+	const std::string why = size < 0 ? "cannot open " + o.fa : read_range(o.fa, 0, (uint64_t)size, file);
+	if (!why.empty()) return die("input", why);
+	const double t_read = now_s() - t0, t1 = now_s();
+	const int rc = idl_fasta_open(o.device, file.data(), file.size(), &calls.fa, err, sizeof err);
+	if (rc == IDL_E_NO_DEVICE) return no_device(rc);
+	if (rc != IDL_OK) return die("input", o.fa + ": " + (err[0] ? err : idl_strerror(rc)));
+	const double t_open = now_s() - t1, t2 = now_s();
+	const idl_fasta_info *fi = idl_fasta_get_info(calls.fa);
+	std::vector<std::vector<uint8_t>> seqs((size_t)fi->n_records);
+	std::vector<const uint8_t*> sp; std::vector<const char*> np;
+	for (int64_t r = 0; r < fi->n_records; ++r) {
+		seqs[(size_t)r].resize((size_t)fi->len[r]);
+		if (idl_fasta_copy(calls.fa, r, seqs[(size_t)r].data(), seqs[(size_t)r].size()) != IDL_OK) return die("idl_fasta_copy", "cannot copy the reference back from the device");
+		sp.push_back(seqs[(size_t)r].data()); np.push_back(fi->name[r]);
+	}
+	calls.ref = idlh_dataset_from_sequences((int32_t)fi->n_records, np.data(), sp.data(), fi->len);
+	if (timing)
+		fprintf(stderr, "indelope timing (reference on the device): read %.3f s, idl_fasta_open %.3f s (h2d %.1f ms, inflate %.1f ms, parse %.1f ms; %.1f MB -> %.1f MB -> "
+		        "%.1f MB of sequence, %lld records), copy back %.3f s\n", t_read, t_open, fi->ms_h2d, fi->ms_inflate, fi->ms_parse, fi->file_bytes / 1e6,
+		        fi->inflated_bytes / 1e6, fi->sequence_bytes / 1e6, (long long)fi->n_records, now_s() - t2);
+	return 0;
+}
 
 // The host reads and sweeps the BAM, a group of regions at a time, in bounded memory (idlh_stream_*); while the GPU works on a batch the host reads and
 // sweeps the next stretch of the file.
@@ -291,16 +357,17 @@ static int run_whole_file(const Options &o)
 		if (open_rc == IDL_OK) calls.create(o.device);
 	});
 	double t1 = now_s();
-	calls.ref = idlh_load_fasta(o.fa.c_str(), err, sizeof err);
+	const int ref_status = open_reference(o, calls);
 	const double t_fasta = now_s() - t1;
 	opener.join();
 	std::vector<uint8_t>().swap(file);
-	if (!calls.ref) status = die("input", err);
+	if (ref_status) status = ref_status;
 	else if (open_rc == IDL_E_NO_DEVICE) status = no_device(open_rc);
 	else if (open_rc != IDL_OK) status = die("input", o.bam + ": " + (bam_err[0] ? bam_err : idl_strerror(open_rc)));
 	else if (calls.create_rc != IDL_OK) status = no_device(calls.create_rc);
 	const idl_bam_info *info = bam ? idl_bam_get_info(bam) : nullptr;
 	if (!status && idlh_dataset_set_targets(calls.ref, info->n_ref, info->ref_name, info->ref_len, err, sizeof err) != 0) status = die("input", err);
+	if (!status) calls.map_fasta_records();
 	double t_sweep = 0;
 	if (!status) {
 		// gen_roi per target, in header order (:599-602)
@@ -359,8 +426,9 @@ static int run_sliced(const Options &o)
 	// the intervals, targets in header order, and the first slice of each: the window holding the position in front of it to the window behind its last
 	// base.  Every error of these comes before a missing device's, and before anything is printed.
 	auto plan = [&]() {
-		calls.ref = idlh_load_targets(o.fa.c_str(), o.bam.c_str(), err, sizeof err);
-		if (!calls.ref) { status = die("input", err); return; }
+		if ((status = open_reference(o, calls))) return;
+		if (idlh_dataset_set_bam_targets(calls.ref, o.bam.c_str(), err, sizeof err) != 0) { status = die("input", err); return; }
+		calls.map_fasta_records();
 		calls.targets = no_regions(calls.ref);
 		const idlh_roiset *all = idlh_rois_view(calls.targets);
 		for (int32_t c = 0; c < all->n_chroms; ++c) { names.push_back(all->chrom_name[c]); lens.push_back(all->chrom_len[c]); }

@@ -135,6 +135,8 @@ Win region_window(const idlh_roiset *rs, int64_t k, const idl_params *p, F &&per
 // ---- a small fork-join helper: packing a step of the chr1 workload is ~400 Mbases; one core cannot feed the GPU ----
 std::atomic<int> g_threads{0};
 
+} // namespace
+
 int pack_threads()
 {
 	int n = g_threads.load();
@@ -142,6 +144,8 @@ int pack_threads()
 	if (n <= 0) { n = (int)std::thread::hardware_concurrency(); if (n > 32) n = 32; }
 	return n < 1 ? 1 : n;
 }
+
+namespace {
 
 // f(begin, end, thread) over [0, n) in blocks handed out dynamically
 template <class F>

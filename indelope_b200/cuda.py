@@ -47,7 +47,8 @@ def lib():
 
 EXPORTS = ("idl_default_params idl_create idl_destroy idl_batch_alloc idl_batch_free idl_submit idl_upload idl_run_resident idl_wait "
            "idl_release idl_strerror idl_last_cuda_error idl_device_count idl_ksw2_batch idl_sweep idl_sweep_free "
-           "idl_bam_open idl_bam_get_info idl_bam_close idl_bam_sweep idl_bam_fetch idl_bam_reads_free idl_bam_set_reference idl_bam_submit idl_bam_pack idl_bam_open_slice idl_device_memory idl_bam_sweep_window").split()
+           "idl_bam_open idl_bam_get_info idl_bam_close idl_bam_sweep idl_bam_fetch idl_bam_reads_free idl_bam_set_reference idl_bam_submit idl_bam_pack idl_bam_open_slice idl_device_memory idl_bam_sweep_window "
+           "idl_fasta_open idl_fasta_get_info idl_fasta_copy idl_fasta_close idl_bam_set_reference_fasta").split()
 
 
 class SweepIn(C.Structure):
@@ -197,6 +198,14 @@ class Bam:
         L.idl_bam_reads_free(out)
         return r
 
+    def set_reference_fasta(self, target, fasta, record):
+        """the sequence of one target from record `record` of a Fasta on the same device (a device-to-device copy)"""
+        L = lib()
+        L.idl_bam_set_reference_fasta.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int64]
+        rc = L.idl_bam_set_reference_fasta(self.h, target, fasta.h, record)
+        if rc != 0:
+            raise IdlError("idl_bam_set_reference_fasta: %s" % L.idl_strerror(rc).decode())
+
     def set_reference(self, target, seq):
         """the sequence of one target (ASCII bytes / uint8 array, as in the FASTA) for the batches built on the device"""
         a = np.ascontiguousarray(seq, dtype=np.uint8)
@@ -209,6 +218,51 @@ class Bam:
     def close(self):
         if self.h:
             lib().idl_bam_close(self.h); self.h = None
+
+    def __del__(self):
+        self.close()
+
+
+class FastaInfo(C.Structure):
+    _fields_ = [("file_bytes", C.c_uint64), ("inflated_bytes", C.c_uint64), ("sequence_bytes", C.c_uint64), ("n_members", C.c_uint32), ("n_chunks", C.c_uint32),
+                ("n_records", C.c_int64), ("name", C.POINTER(C.c_char_p)), ("len", C.POINTER(C.c_int64)), ("ms_h2d", C.c_float), ("ms_inflate", C.c_float),
+                ("ms_parse", C.c_float), ("parse_algorithmic_bytes", C.c_uint64), ("parse_streamed_bytes", C.c_uint64)]
+
+
+class Fasta:
+    """idl_fasta_*: a bgzip-compressed FASTA (`data` = the file's bytes) inflated and parsed on the GPU; the sequences stay there.  IdlError for plain
+    gzip, a corrupt member or a text that does not start with '>'."""
+
+    def __init__(self, data, device=0):
+        L = lib()
+        L.idl_fasta_open.argtypes = [C.c_int, C.c_char_p, C.c_size_t, C.POINTER(C.c_void_p), C.c_char_p, C.c_size_t]
+        L.idl_fasta_get_info.argtypes = [C.c_void_p]; L.idl_fasta_get_info.restype = C.POINTER(FastaInfo)
+        L.idl_fasta_copy.argtypes = [C.c_void_p, C.c_int64, u8p, C.c_size_t]
+        L.idl_fasta_close.argtypes = [C.c_void_p]
+        self.h = C.c_void_p()
+        err = C.create_string_buffer(512)
+        rc = L.idl_fasta_open(device, data, len(data), C.byref(self.h), err, 512)
+        if rc != 0:
+            self.h = None
+            raise IdlError("idl_fasta_open: %s: %s" % (L.idl_strerror(rc).decode(), err.value.decode()))
+        i = L.idl_fasta_get_info(self.h).contents
+        self.n_records = int(i.n_records)
+        self.names = [i.name[k].decode("latin-1") for k in range(self.n_records)]
+        self.lengths = [int(i.len[k]) for k in range(self.n_records)]
+        self.info = {k: getattr(i, k) for k in ("file_bytes", "inflated_bytes", "sequence_bytes", "n_members", "n_chunks", "ms_h2d", "ms_inflate", "ms_parse",
+                                                 "parse_algorithmic_bytes", "parse_streamed_bytes")}
+
+    def sequence(self, record):
+        """one record's sequence copied to the host (uint8 array)"""
+        out = np.empty(self.lengths[record], dtype=np.uint8)
+        rc = lib().idl_fasta_copy(self.h, record, out.ctypes.data_as(u8p), len(out))
+        if rc != 0:
+            raise IdlError("idl_fasta_copy: %s" % lib().idl_strerror(rc).decode())
+        return out
+
+    def close(self):
+        if self.h:
+            lib().idl_fasta_close(self.h); self.h = None
 
     def __del__(self):
         self.close()

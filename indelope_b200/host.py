@@ -60,6 +60,9 @@ def lib():
         L.idlh_load_fasta.restype = C.c_void_p
         L.idlh_load_fasta.argtypes = [C.c_char_p, C.c_char_p, C.c_size_t]
         L.idlh_dataset_set_targets.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_char_p), i64p, C.c_char_p, C.c_size_t]
+        L.idlh_dataset_set_bam_targets.argtypes = [C.c_void_p, C.c_char_p, C.c_char_p, C.c_size_t]
+        L.idlh_dataset_from_sequences.restype = C.c_void_p
+        L.idlh_dataset_from_sequences.argtypes = [C.c_int32, C.POINTER(C.c_char_p), C.POINTER(u8p), i64p]
         L.idlh_load_region.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.c_int64, C.c_int64, C.c_char_p, C.c_size_t]
         L.idlh_write_fasta.argtypes = [C.c_void_p, C.c_char_p]
         L.idlh_write_bam.argtypes = [C.c_void_p, C.c_char_p, C.c_int]
@@ -181,12 +184,31 @@ class Dataset:
 
     @classmethod
     def load_fasta(cls, fasta):
-        """the reference sequences alone (the BAM is decoded on the device: cuda.Bam)"""
+        """the reference sequences alone (the BAM is decoded on the device: cuda.Bam); the FASTA plain or compressed with bgzip"""
         err = C.create_string_buffer(512)
         h = lib().idlh_load_fasta(str(fasta).encode(), err, 512)
         if not h:
             raise IOError(err.value.decode())
         return cls(_handle=h)
+
+    @classmethod
+    def from_sequences(cls, names, seqs):
+        """a reference without reads from names and sequences (bytes / uint8 arrays), e.g. those of a cuda.Fasta; everything is copied"""
+        a = [np.ascontiguousarray(np.frombuffer(x, np.uint8) if isinstance(x, (bytes, bytearray)) else x, dtype=np.uint8) for x in seqs]
+        n = len(a)
+        nm = (C.c_char_p * max(n, 1))(*[x.encode("latin-1") for x in names])
+        sp = (u8p * max(n, 1))(*[x.ctypes.data_as(u8p) for x in a])
+        lens = np.array([len(x) for x in a] or [0], dtype=np.int64)
+        return cls(_handle=lib().idlh_dataset_from_sequences(n, nm, sp, lens.ctypes.data_as(i64p)))
+
+    def set_bam_targets(self, bam):
+        """set_targets with the targets of a BAM file's header (only the header's members are read)"""
+        err = C.create_string_buffer(512)
+        if lib().idlh_dataset_set_bam_targets(self.h, str(bam).encode(), err, 512) != 0:
+            raise IOError(err.value.decode())
+        c = (C.c_int64 * 4)()
+        lib().idlh_dataset_counts(self.h, c)
+        self.n_reads, self.n_bases, self.n_events, self.n_chroms = list(c)
 
     def set_targets(self, names, lengths):
         """order the sequences as a BAM header lists its targets (same checks and messages as Dataset.load)"""

@@ -123,6 +123,17 @@ type
     ms_h2d*, ms_inflate*, ms_parse*: cfloat
     n_chunks*: uint32
 
+  IdlFasta* = pointer                      ## a bgzipped FASTA parsed into device memory (idl_fasta_open)
+
+  IdlFastaInfo* {.bycopy.} = object        ## idl_fasta_info
+    file_bytes*, inflated_bytes*, sequence_bytes*: uint64
+    n_members*, n_chunks*: uint32
+    n_records*: int64
+    name*: cstringArray
+    len*: ptr UncheckedArray[int64]
+    ms_h2d*, ms_inflate*, ms_parse*: cfloat
+    parse_algorithmic_bytes*, parse_streamed_bytes*: uint64
+
   IdlBamSlice* {.bycopy.} = object         ## idl_bam_slice: a run of BGZF members holding one target's records (found through the .bai)
     n_ref*: int32
     ref_name*: cstringArray
@@ -185,6 +196,12 @@ proc idl_bam_submit*(ctx: IdlCtx, bam: IdlBam, n_regions: csize_t, roi_chrom, ro
                      ordinal_base: uint32, ticket: ptr uint64): cint {.importc.}
 proc idl_bam_pack*(ctx: IdlCtx, bam: IdlBam, n_regions: csize_t, roi_chrom, roi_start, roi_end, roi_n_reads: ptr int32, read_idx: ptr int64,
                    ordinal_base: uint32, b: ptr IdlBatch): cint {.importc.}
+# a bgzip-compressed reference on the device (ref.fa.gz, what open_fai reads through htslib, src/indelope.nim:593)
+proc idl_fasta_open*(device: cint, file: ptr uint8, file_len: csize_t, fa: ptr IdlFasta, err: cstring, errlen: csize_t): cint {.importc.}
+proc idl_fasta_get_info*(fa: IdlFasta): ptr IdlFastaInfo {.importc.}
+proc idl_fasta_copy*(fa: IdlFasta, record: int64, dst: ptr uint8, dst_len: csize_t): cint {.importc.}
+proc idl_fasta_close*(fa: IdlFasta) {.importc.}
+proc idl_bam_set_reference_fasta*(bam: IdlBam, target: int32, fa: IdlFasta, record: int64): cint {.importc.}
 {.pop.}
 
 when isMainModule:
